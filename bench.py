@@ -168,6 +168,22 @@ def emit_line(line):
     out.flush()
 
 
+# --dump-outputs: every array of one run together stays under 64 MB (np.save adds a header of about 128 bytes per file)
+DUMP_LIMIT_BYTES = 60 << 20
+
+
+def dump_outputs(out_dir, arrays, seed):
+    """Write out_dir/<name>.npy (float64) for each (batch, ...) array of `arrays`.  When all instances do not fit in
+    DUMP_LIMIT_BYTES, every file holds the same instances: a sample drawn with `seed`, in ascending instance order."""
+    os.makedirs(out_dir, exist_ok=True)
+    batch = len(next(iter(arrays.values())))
+    per_instance = sum(a[0].nbytes for a in arrays.values())
+    n = min(batch, DUMP_LIMIT_BYTES // per_instance)
+    idx = np.sort(np.random.default_rng(seed).choice(batch, n, replace=False)) if n < batch else np.arange(batch)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a[idx], dtype=np.float64))
+
+
 def splitmix_uniform(seed, index):
     """Counter-based splitmix64 -> double in [0,1); vectorised twin of oracle_splitmix_uniform."""
     idx = np.asarray(index, dtype=np.uint64)
@@ -491,6 +507,9 @@ def run_anymal(args, rank, local_rank, world):
     launches = solver.launchCount() - launches0
     profile = solver.getProfile()
     solver.setProfiling(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {n: np.stack(solver.getSolution(n), axis=1) for n in ("q", "v", "a", "u", "f")},
+                     ANYMAL_SEED[args.workload])
     # end-to-end: host states in, first control input out, through the public API
     for _ in range(3):
         solver.updateSolution(0.0, q0, v0, ls)
@@ -643,6 +662,8 @@ def run_iiwa(args, rank, local_rank, world):
     launches = solver.launchCount() - launches0
     profile = solver.getProfile()
     solver.setProfiling(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {n: solver.getSolution(n) for n in ("q", "v", "a", "u", "lmd", "gmm", "beta")}, w["seed"])
 
     # ---- end-to-end arm: host buffers through the public API ----------------------------------
     q_host = q_pin.numpy()
@@ -772,7 +793,12 @@ def main():
     ap.add_argument("--workload", default="iiwa14_unocp", choices=list(IIWA_WORKLOADS) + ["anymal_trotting", "anymal_running"],
                     help="iiwa14_unocp = BASELINE configs[2] (the headline); iiwa14_unocp_config / iiwa14_unparnmpc_task = "
                          "configs[0] / configs[1]; anymal_* = configs[3] / configs[4]")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the solution of the last one (rank 0's instances) as DIR/<field>.npy, "
+                         "float64; beyond 64 MB in all, a fixed seeded sample of the instances")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU solver computed; it needs --impl b200")
     claim_stdout()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -13,7 +13,10 @@ Here the URDF itself is parsed again, with different code and different mathemat
     pinocchio::urdf::buildModel sees: urdfdom keeps joints in a std::map<std::string, ...> and fills
     Link::child_joints in that (alphabetical) order.
 
-Needs the reference's URDF files; skipped (loudly) where /root/reference does not exist, e.g. on the GPU box."""
+Needs the reference's URDF files, stored as tests/golden/iiwa14.urdf (idocp's examples/iiwa14/iiwa_description/urdf/iiwa14.urdf)
+and tests/golden/anymal.urdf (examples/anymal/anymal_b_simple_description/urdf/anymal.urdf); skipped (loudly) while they are
+absent.  include/idocp_b200/idocp_b200.hpp holds the content hashes of both files (kUrdfHashIiwa14, kUrdfHashAnymalExamples);
+tests/test_cpp_host.py checks a stored iiwa14.urdf against its hash."""
 import math
 import os
 import xml.etree.ElementTree as ET
@@ -21,12 +24,15 @@ import xml.etree.ElementTree as ET
 import numpy as np
 import pytest
 
-IIWA_URDF = "/root/reference/examples/iiwa14/iiwa_description/urdf/iiwa14.urdf"
-ANYMAL_URDF = "/root/reference/examples/anymal/anymal_b_simple_description/urdf/anymal.urdf"
+from conftest import GOLDEN
+
+IIWA_URDF = os.path.join(GOLDEN, "iiwa14.urdf")
+ANYMAL_URDF = os.path.join(GOLDEN, "anymal.urdf")
 G = 9.81
 
-pytestmark = pytest.mark.skipif(not os.path.exists(IIWA_URDF),
-                                reason="URDF files of the reference not present (/root/reference): independent model check NOT run")
+pytestmark = pytest.mark.skipif(not (os.path.exists(IIWA_URDF) and os.path.exists(ANYMAL_URDF)),
+                                reason="tests/golden/iiwa14.urdf and anymal.urdf (idocp's URDF files) not present: "
+                                       "independent model check NOT run")
 
 
 def _floats(s, n):
