@@ -118,7 +118,7 @@ EXPORTS = [
     "idocp_b200_fb_get_profile", "idocp_b200_fb_record_bytes", "idocp_b200_fb_problem_default",
     "idocp_b200_fb_total_weight", "idocp_b200_fb_contact_frame_positions", "idocp_b200_fb_clear_line_search_filter",
     "idocp_b200_fb_set_strict_discretization",
-    "idocp_b200_fb_create_sharded", "idocp_b200_fb_sharded_destroy", "idocp_b200_fb_sharded_num_shards",
+    "idocp_b200_fb_create_sharded", "idocp_b200_fb_sharded_destroy", "idocp_b200_fb_sharded_num_shards", "idocp_b200_fb_sharded_shard",
     "idocp_b200_fb_sharded_set_solution", "idocp_b200_fb_sharded_set_cost_reference", "idocp_b200_fb_sharded_discretize",
     "idocp_b200_fb_sharded_init_constraints", "idocp_b200_fb_sharded_set_strict_discretization",
     "idocp_b200_fb_sharded_update_solution", "idocp_b200_fb_sharded_compute_kkt_residual", "idocp_b200_fb_sharded_kkt_error",
@@ -213,34 +213,33 @@ class Library:
                      "launch_count"):
             getattr(L, "idocp_b200_fb_sharded_" + name).argtypes = getattr(L, "idocp_b200_fb_" + name).argtypes
         L.idocp_b200_fb_create_sharded.argtypes = [C.POINTER(FbProblem), C.c_void_p, C.c_int, _ip, C.c_int, C.POINTER(C.c_void_p)]
-        L.idocp_b200_fb_sharded_destroy.argtypes = [C.c_void_p]
-        L.idocp_b200_fb_sharded_num_shards.argtypes = [C.c_void_p, _ip, _ip]
         L.idocp_b200_fb_problem_default.argtypes = [C.POINTER(FbProblem)]
         L.idocp_b200_fb_total_weight.restype = C.c_double
         L.idocp_b200_fb_contact_frame_positions.argtypes = [_dp, _dp]
         L.idocp_b200_create_sharded.argtypes = [C.POINTER(Problem), C.c_int, C.c_int, _ip, C.c_int, C.POINTER(C.c_void_p)]
-        L.idocp_b200_sharded_destroy.argtypes = [C.c_void_p]
-        L.idocp_b200_sharded_num_shards.argtypes = [C.c_void_p, _ip, _ip]
-        L.idocp_b200_sharded_shard.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]
-        L.idocp_b200_sharded_set_solution.argtypes = [C.c_void_p, C.c_char_p, _dp, C.c_int]
-        L.idocp_b200_sharded_init_constraints.argtypes = [C.c_void_p]
-        L.idocp_b200_sharded_init_backward_correction.argtypes = [C.c_void_p, C.c_double]
-        L.idocp_b200_sharded_set_task_reference.argtypes = [C.c_void_p, _dp]
-        L.idocp_b200_sharded_update_solution.argtypes = [C.c_void_p, C.c_double, _dp, _dp, C.c_int]
-        L.idocp_b200_sharded_compute_kkt_residual.argtypes = [C.c_void_p, C.c_double, _dp, _dp]
-        L.idocp_b200_sharded_kkt_error.argtypes = [C.c_void_p, _dp]
-        L.idocp_b200_sharded_get_solution.argtypes = [C.c_void_p, C.c_char_p, _dp]
-        L.idocp_b200_sharded_get_stage_solution.argtypes = [C.c_void_p, C.c_char_p, C.c_int, _dp]
-        L.idocp_b200_sharded_get_step_sizes.argtypes = [C.c_void_p, _dp, _dp]
-        L.idocp_b200_sharded_get_status.argtypes = [C.c_void_p, _ip]
-        L.idocp_b200_sharded_clear_line_search_filter.argtypes = [C.c_void_p]
-        L.idocp_b200_sharded_sync.argtypes = [C.c_void_p]
+        for name in ("set_solution", "init_constraints", "init_backward_correction", "set_task_reference", "update_solution",
+                     "compute_kkt_residual", "kkt_error", "get_solution", "get_stage_solution", "get_step_sizes", "get_status",
+                     "clear_line_search_filter", "sync"):
+            getattr(L, "idocp_b200_sharded_" + name).argtypes = getattr(L, "idocp_b200_" + name).argtypes
+        for family in ("", "fb_"):
+            getattr(L, "idocp_b200_%ssharded_destroy" % family).argtypes = [C.c_void_p]
+            getattr(L, "idocp_b200_%ssharded_num_shards" % family).argtypes = [C.c_void_p, _ip, _ip]
+            getattr(L, "idocp_b200_%ssharded_shard" % family).argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]
         self.L = L
 
     def check(self, rc):
         if rc < 0:
             raise Idocp_b200Error("idocp_b200 error %d: %s" % (rc, self.L.idocp_b200_last_error().decode()))
         return rc
+
+    def entry(self, family, name, sharded):
+        """The entry point idocp_b200_<family><name> of a solver handle, or its sharded twin idocp_b200_<family>sharded_<name>
+        (same arguments); raises for an entry point that has no sharded twin."""
+        full = "idocp_b200_%s%s%s" % (family, "sharded_" if sharded else "", name)
+        try:
+            return getattr(self.L, full)
+        except AttributeError:
+            raise Idocp_b200Error("%s does not exist: a sharded solver has one single-device solver per device" % full) from None
 
     def version(self):
         return self.L.idocp_b200_version().decode()

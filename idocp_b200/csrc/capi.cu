@@ -62,8 +62,11 @@ static const char* kKernelClassNames[KC_NUM] = {"linearize", "riccati", "expand"
                                                 "fb_riccati_backward", "fb_riccati_forward", "fb_expand", "fb_update", "fb_kkt",
                                                 "update_linearize", "step_min"};
 
-// launch bookkeeping shared by every solver handle: stream, launch counter, per-kernel-class event timing
-struct LaunchProfiler {
+// What every solver handle of both families owns: its device and stream, the device allocations, the CUDA events, the
+// launch counter and the per-kernel-class event timing.  open() / release() are the one lifecycle of a handle; the
+// *_sync / *_launch_count / *_stream / *_set_profiling / *_get_profile entry points of both families forward here.
+struct DeviceHandle {
+  int device = 0;
   cudaStream_t stream = nullptr;
   long long launches = 0;
   // profiling: 0 off, 1 = CUDA events recorded around every launch on the launching stream and
@@ -129,11 +132,75 @@ struct LaunchProfiler {
     *p = static_cast<T*>(q);
     return 0;
   }
+
+  // device count and index checks, then the handle's non-blocking stream on `device`
+  int open(int device) {
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0)
+      return fail(IDOCP_B200_NO_DEVICE, "no CUDA device available (there is no CPU fallback)");
+    if (device < 0 || device >= ndev) return fail(IDOCP_B200_INVALID_ARGUMENT, "invalid device index");
+    CUDA_OK(cudaSetDevice(device));
+    this->device = device;
+    if (cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking) != cudaSuccess)
+      return fail(IDOCP_B200_CUDA_ERROR, "cudaStreamCreate failed");
+    return IDOCP_B200_OK;
+  }
+  // waits for the stream, then frees everything open() and the handle's calls created
+  void release() {
+    cudaSetDevice(device);
+    if (stream) cudaStreamSynchronize(stream);
+    resolve_profile();
+    for (cudaEvent_t e : event_pool) cudaEventDestroy(e);
+    if (copies_done) cudaEventDestroy(copies_done);
+    for (void* p : allocs) cudaFree(p);
+    if (stream) cudaStreamDestroy(stream);
+  }
+
+  int sync() {
+    CUDA_OK(cudaSetDevice(device));
+    CUDA_OK(cudaStreamSynchronize(stream));
+    return IDOCP_B200_OK;
+  }
+  int launch_count(long long* out) const {
+    *out = launches;
+    return IDOCP_B200_OK;
+  }
+  int get_stream(void** out) const {
+    *out = reinterpret_cast<void*>(stream);
+    return IDOCP_B200_OK;
+  }
+  int set_profiling(int enabled) {
+    resolve_profile();
+    profiling = enabled != 0;
+    for (int k = 0; k < KC_NUM; ++k) { prof_ms[k] = 0; prof_calls[k] = 0; }
+    return IDOCP_B200_OK;
+  }
+  int get_profile(int cap, const char** names, double* ms, long long* calls) {
+    resolve_profile();
+    int n = 0;
+    for (int k = 0; k < KC_NUM && n < cap; ++k) {
+      if (prof_calls[k] == 0) continue;
+      names[n] = kKernelClassNames[k];
+      ms[n] = prof_ms[k];
+      calls[n] = prof_calls[k];
+      ++n;
+    }
+    return n;
+  }
 };
 
-struct idocp_b200_solver : LaunchProfiler {
+template <typename H>
+static int destroy_handle(H* h) {
+  if (h) {
+    h->release();
+    delete h;
+  }
+  return IDOCP_B200_OK;
+}
+
+struct idocp_b200_solver : DeviceHandle {
   idocp_b200_problem prob;
-  int kind = 0, device = 0;
+  int kind = 0;
   int B = 0, Bp = 0, N = 0;
   DevProblem* d_prob = nullptr;
   DevProblem h_prob;
@@ -264,22 +331,17 @@ extern "C" int idocp_b200_create(const idocp_b200_problem* p, int solver_kind, i
     return fail(IDOCP_B200_INVALID_ARGUMENT, "invalid value: barrier / fraction_rate");
   if (solver_kind != IDOCP_B200_SOLVER_UNOCP && solver_kind != IDOCP_B200_SOLVER_UNPARNMPC)
     return fail(IDOCP_B200_INVALID_ARGUMENT, "unknown solver kind");
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0)
-    return fail(IDOCP_B200_NO_DEVICE, "no CUDA device available (there is no CPU fallback)");
-  if (device < 0 || device >= ndev) return fail(IDOCP_B200_INVALID_ARGUMENT, "invalid device index");
-  CUDA_OK(cudaSetDevice(device));
   idocp_b200_solver* h = new idocp_b200_solver();
+  const int orc = h->open(device);
+  if (orc != IDOCP_B200_OK) {
+    delete h;
+    return orc;
+  }
   h->prob = *p;
   h->kind = solver_kind;
-  h->device = device;
   h->B = batch;
   h->Bp = (batch + 3) / 4 * 4;
   h->N = p->N;
-  if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess) {
-    delete h;
-    return fail(IDOCP_B200_CUDA_ERROR, "cudaStreamCreate failed");
-  }
   fill_dev_problem(*p, h->h_prob);
   const size_t N = h->N, Bp = h->Bp, G = Bp / 4;
   const bool par = solver_kind == IDOCP_B200_SOLVER_UNPARNMPC;
@@ -361,18 +423,7 @@ extern "C" int idocp_b200_create(const idocp_b200_problem* p, int solver_kind, i
   return IDOCP_B200_OK;
 }
 
-extern "C" int idocp_b200_destroy(idocp_b200_solver* h) {
-  if (!h) return IDOCP_B200_OK;
-  cudaSetDevice(h->device);
-  if (h->stream) cudaStreamSynchronize(h->stream);
-  h->resolve_profile();
-  for (cudaEvent_t e : h->event_pool) cudaEventDestroy(e);
-  if (h->copies_done) cudaEventDestroy(h->copies_done);
-  for (void* p : h->allocs) cudaFree(p);
-  if (h->stream) cudaStreamDestroy(h->stream);
-  delete h;
-  return IDOCP_B200_OK;
-}
+extern "C" int idocp_b200_destroy(idocp_b200_solver* h) { return destroy_handle(h); }
 
 static int field_index(const char* name) {
   if (!name) return -1;
@@ -898,48 +949,23 @@ extern "C" int idocp_b200_set_pipelining(idocp_b200_solver* h, int enabled) {
 }
 
 extern "C" int idocp_b200_sync(idocp_b200_solver* h) {
-  if (!h) return fail(IDOCP_B200_INVALID_ARGUMENT, "null handle");
-  CUDA_OK(cudaSetDevice(h->device));
-  CUDA_OK(cudaStreamSynchronize(h->stream));
-  return IDOCP_B200_OK;
+  return h ? h->sync() : fail(IDOCP_B200_INVALID_ARGUMENT, "null handle");
 }
-
 extern "C" int idocp_b200_launch_count(idocp_b200_solver* h, long long* out) {
-  if (!h || !out) return fail(IDOCP_B200_INVALID_ARGUMENT, "launch_count: null pointer");
-  *out = h->launches;
-  return IDOCP_B200_OK;
+  return h && out ? h->launch_count(out) : fail(IDOCP_B200_INVALID_ARGUMENT, "launch_count: null pointer");
 }
-
 extern "C" int idocp_b200_stream(idocp_b200_solver* h, void** out) {
-  if (!h || !out) return fail(IDOCP_B200_INVALID_ARGUMENT, "stream: null pointer");
-  *out = reinterpret_cast<void*>(h->stream);
-  return IDOCP_B200_OK;
+  return h && out ? h->get_stream(out) : fail(IDOCP_B200_INVALID_ARGUMENT, "stream: null pointer");
 }
-
 extern "C" int idocp_b200_set_profiling(idocp_b200_solver* h, int enabled) {
-  if (!h) return fail(IDOCP_B200_INVALID_ARGUMENT, "null handle");
-  h->resolve_profile();
-  h->profiling = enabled != 0;
-  for (int k = 0; k < KC_NUM; ++k) { h->prof_ms[k] = 0; h->prof_calls[k] = 0; }
-  return IDOCP_B200_OK;
+  return h ? h->set_profiling(enabled) : fail(IDOCP_B200_INVALID_ARGUMENT, "null handle");
 }
-
 extern "C" int idocp_b200_get_profile(idocp_b200_solver* h, int cap, const char** names, double* ms, long long* calls) {
-  if (!h || !names || !ms || !calls) return fail(IDOCP_B200_INVALID_ARGUMENT, "get_profile: null pointer");
-  h->resolve_profile();
-  int n = 0;
-  for (int k = 0; k < KC_NUM && n < cap; ++k) {
-    if (h->prof_calls[k] == 0) continue;
-    names[n] = kKernelClassNames[k];
-    ms[n] = h->prof_ms[k];
-    calls[n] = h->prof_calls[k];
-    ++n;
-  }
-  return n;
+  return h && names && ms && calls ? h->get_profile(cap, names, ms, calls)
+                                   : fail(IDOCP_B200_INVALID_ARGUMENT, "get_profile: null pointer");
 }
 
 #include "derivative_checker.inc"
-#include "sharded_capi.inc"
 #include "hybrid_capi.inc"
 #include "fb_capi.inc"
-#include "fb_sharded_capi.inc"
+#include "sharded_capi.inc"

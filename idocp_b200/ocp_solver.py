@@ -47,11 +47,11 @@ class OCPSolver:
 
     def _f(self, name):
         """The C-ABI entry point `name` of this solver: idocp_b200_fb_<name> or its sharded twin (same arguments)."""
-        return getattr(self.lib.L, ("idocp_b200_fb_sharded_" if self._sharded else "idocp_b200_fb_") + name)
+        return self.lib.entry("fb_", name, self._sharded)
 
     def __del__(self):
         if getattr(self, "_h", None):
-            (self.lib.L.idocp_b200_fb_sharded_destroy if self._sharded else self.lib.L.idocp_b200_fb_destroy)(self._h)
+            self._f("destroy")(self._h)
             self._h = None
 
     # ---- contact schedule (ocp_solver.cpp:173-194) ----
@@ -124,10 +124,8 @@ class OCPSolver:
         self.lib.check(self._f("update_solution")(self._h, float(t), None, None, int(line_search)))
 
     def stream(self):
-        if self._sharded:
-            raise capi.Idocp_b200Error("stream(): a sharded solver has one stream per device")
         p = C.c_void_p()
-        self.lib.check(self.lib.L.idocp_b200_fb_stream(self._h, C.byref(p)))
+        self.lib.check(self._f("stream")(self._h, C.byref(p)))
         return p.value or 0
 
     def computeKKTResidual(self, t, q, v):
@@ -189,14 +187,12 @@ class OCPSolver:
         return n.value
 
     def setProfiling(self, enabled):
-        if self._sharded:
-            raise capi.Idocp_b200Error("profiling is per single-device solver")
-        self.lib.check(self.lib.L.idocp_b200_fb_set_profiling(self._h, int(enabled)))
+        self.lib.check(self._f("set_profiling")(self._h, int(enabled)))
 
     def getProfile(self):
         cap = 32
         names = (C.c_char_p * cap)()
         ms = np.zeros(cap)
         calls = (C.c_longlong * cap)()
-        n = self.lib.check(self.lib.L.idocp_b200_fb_get_profile(self._h, cap, names, capi.dptr(ms), calls))
+        n = self.lib.check(self._f("get_profile")(self._h, cap, names, capi.dptr(ms), calls))
         return {names[i].decode(): dict(ms=float(ms[i]), calls=int(calls[i])) for i in range(n)}

@@ -96,18 +96,33 @@ def task_space_circle_ref(t):
 class _BatchSolver:
     kind = None
 
-    def __init__(self, problem, batch, device=0, lib=None):
+    def __init__(self, problem, batch, device=0, lib=None, devices=None):
+        """devices = [d0, d1, ...]: the batch sharded over several GPUs of this node by ONE solver object
+        (idocp_b200_create_sharded: contiguous split, one device + stream per shard, no collective); `first` then holds the
+        first instance of every shard.  Entry points without a sharded twin raise on such a solver."""
         self.lib = lib or capi.default_library()
         self.batch = int(batch)
         self.N = int(problem.N)
         self.problem = problem
         self._h = C.c_void_p()
-        self.lib.check(self.lib.L.idocp_b200_create(C.byref(problem), self.kind, self.batch, device,
-                                                    C.byref(self._h)))
+        self._sharded = devices is not None
+        if self._sharded:
+            devs = (C.c_int * len(devices))(*[int(d) for d in devices])
+            self.lib.check(self.lib.L.idocp_b200_create_sharded(C.byref(problem), self.kind, self.batch, devs, len(devices),
+                                                                C.byref(self._h)))
+            first = (C.c_int * (len(devices) + 1))()
+            self.lib.check(self._f("num_shards")(self._h, C.byref(C.c_int()), first))
+            self.first = list(first)
+        else:
+            self.lib.check(self.lib.L.idocp_b200_create(C.byref(problem), self.kind, self.batch, device, C.byref(self._h)))
+
+    def _f(self, name):
+        """The C-ABI entry point `name` of this solver: idocp_b200_<name> or its sharded twin."""
+        return self.lib.entry("", name, self._sharded)
 
     def close(self):
         if getattr(self, "_h", None):
-            self.lib.L.idocp_b200_destroy(self._h)
+            self._f("destroy")(self._h)
             self._h = None
 
     def __del__(self):
@@ -135,10 +150,10 @@ class _BatchSolver:
             bc = 0
         else:
             raise ValueError("setSolution: bad shape %s" % (value.shape,))
-        self.lib.check(self.lib.L.idocp_b200_set_solution(self._h, name.encode(), dptr(value), bc))
+        self.lib.check(self._f("set_solution")(self._h, name.encode(), dptr(value), bc))
 
     def initConstraints(self):
-        self.lib.check(self.lib.L.idocp_b200_init_constraints(self._h))
+        self.lib.check(self._f("init_constraints")(self._h))
 
     def stageTimes(self, t):
         """Time at which every stage index is linearised (unocp_solver.cpp:80-93 / unbackward_correction.cpp:73-95)."""
@@ -154,28 +169,27 @@ class _BatchSolver:
         table = np.ascontiguousarray(table, dtype=np.float64)
         if table.shape != (self.N + 1, 12):
             raise ValueError("task reference table must have shape (%d, 12)" % (self.N + 1))
-        self.lib.check(self.lib.L.idocp_b200_set_task_reference(self._h, dptr(table)))
+        self.lib.check(self._f("set_task_reference")(self._h, dptr(table)))
 
     def updateSolution(self, t, q, v, line_search=False):
         q, v = self._x(q), self._x(v)
-        self.lib.check(self.lib.L.idocp_b200_update_solution(self._h, float(t), dptr(q), dptr(v), int(line_search)))
+        self.lib.check(self._f("update_solution")(self._h, float(t), dptr(q), dptr(v), int(line_search)))
 
     def updateSolutionDevice(self, t, q_ptr, v_ptr, line_search=False):
         """q_ptr / v_ptr: device addresses (e.g. torch.Tensor.data_ptr()) of (batch, dimv) float64."""
-        self.lib.check(self.lib.L.idocp_b200_update_solution_device(self._h, float(t), C.c_void_p(q_ptr),
-                                                                    C.c_void_p(v_ptr), int(line_search)))
+        self.lib.check(self._f("update_solution_device")(self._h, float(t), C.c_void_p(q_ptr), C.c_void_p(v_ptr),
+                                                         int(line_search)))
 
     def computeKKTResidual(self, t, q, v):
         q, v = self._x(q), self._x(v)
-        self.lib.check(self.lib.L.idocp_b200_compute_kkt_residual(self._h, float(t), dptr(q), dptr(v)))
+        self.lib.check(self._f("compute_kkt_residual")(self._h, float(t), dptr(q), dptr(v)))
 
     def computeKKTResidualDevice(self, t, q_ptr, v_ptr):
-        self.lib.check(self.lib.L.idocp_b200_compute_kkt_residual_device(self._h, float(t), C.c_void_p(q_ptr),
-                                                                         C.c_void_p(v_ptr)))
+        self.lib.check(self._f("compute_kkt_residual_device")(self._h, float(t), C.c_void_p(q_ptr), C.c_void_p(v_ptr)))
 
     def KKTError(self):
         out = np.zeros(self.batch)
-        self.lib.check(self.lib.L.idocp_b200_kkt_error(self._h, dptr(out)))
+        self.lib.check(self._f("kkt_error")(self._h, dptr(out)))
         return out
 
     def _nstages(self, name, full_names):
@@ -183,14 +197,14 @@ class _BatchSolver:
 
     def getSolution(self, name):
         out = np.zeros((self.batch, self._nstages(name, ("q", "v", "lmd", "gmm")), DIMV))
-        self.lib.check(self.lib.L.idocp_b200_get_solution(self._h, name.encode(), dptr(out)))
+        self.lib.check(self._f("get_solution")(self._h, name.encode(), dptr(out)))
         return out
 
     def getStageSolution(self, name, stage, out=None):
         """UnOCPSolver::getSolution(int stage), one field: (batch, dimv)."""
         if out is None:
             out = np.zeros((self.batch, DIMV))
-        self.lib.check(self.lib.L.idocp_b200_get_stage_solution(self._h, name.encode(), int(stage), dptr(out)))
+        self.lib.check(self._f("get_stage_solution")(self._h, name.encode(), int(stage), dptr(out)))
         return out
 
     def saveSolution(self, path_to_file, name, instance=0):
@@ -202,67 +216,67 @@ class _BatchSolver:
                     f.write("".join("%g " % x for x in row) + "\n")
 
     def clearLineSearchFilter(self):
-        self.lib.check(self.lib.L.idocp_b200_clear_line_search_filter(self._h))
+        self.lib.check(self._f("clear_line_search_filter")(self._h))
 
     def isCurrentSolutionFeasible(self):
         out = np.zeros(self.batch, dtype=np.int32)
-        self.lib.check(self.lib.L.idocp_b200_is_feasible(self._h, out.ctypes.data_as(C.POINTER(C.c_int))))
+        self.lib.check(self._f("is_feasible")(self._h, out.ctypes.data_as(C.POINTER(C.c_int))))
         return out.astype(bool)
 
     # -- additions for parity tests / measurement ----------------------------------------------
     def getDirection(self, name):
         out = np.zeros((self.batch, self._nstages(name, ("dq", "dv", "dlmd", "dgmm")), DIMV))
-        self.lib.check(self.lib.L.idocp_b200_get_direction(self._h, name.encode(), dptr(out)))
+        self.lib.check(self._f("get_direction")(self._h, name.encode(), dptr(out)))
         return out
 
     def getConstraintData(self, name):
         # "slack" / "dual": the six joint-limit components; "acc_slack" / "acc_dual": the two acceleration limits
         out = np.zeros((self.batch, self.N, 2 if name.startswith("acc_") else NUM_CONSTRAINTS, DIMV))
-        self.lib.check(self.lib.L.idocp_b200_get_constraint_data(self._h, name.encode(), dptr(out)))
+        self.lib.check(self._f("get_constraint_data")(self._h, name.encode(), dptr(out)))
         return out
 
     def getStepSizes(self):
         p, d = np.zeros(self.batch), np.zeros(self.batch)
-        self.lib.check(self.lib.L.idocp_b200_get_step_sizes(self._h, dptr(p), dptr(d)))
+        self.lib.check(self._f("get_step_sizes")(self._h, dptr(p), dptr(d)))
         return p, d
 
     def setPipelining(self, enabled):
         """UnOCPSolver: fuse the update with the linearisation of the new iterate (default on; idocp_b200_set_pipelining)."""
-        self.lib.check(self.lib.L.idocp_b200_set_pipelining(self._h, int(bool(enabled))))
+        self.lib.check(self._f("set_pipelining")(self._h, int(bool(enabled))))
 
     def getUnKKT(self, stage):
         Q = np.zeros((self.batch, 21, 21))
         res = np.zeros((self.batch, 35))
-        self.lib.check(self.lib.L.idocp_b200_get_unkkt(self._h, int(stage), dptr(Q), dptr(res)))
+        self.lib.check(self._f("get_unkkt")(self._h, int(stage), dptr(Q), dptr(res)))
         return np.ascontiguousarray(Q.transpose(0, 2, 1)), res   # column-major -> [row, col]
 
     def getStatus(self):
         out = np.zeros(self.batch, dtype=np.int32)
-        self.lib.check(self.lib.L.idocp_b200_get_status(self._h, out.ctypes.data_as(C.POINTER(C.c_int))))
+        self.lib.check(self._f("get_status")(self._h, out.ctypes.data_as(C.POINTER(C.c_int))))
         return out
 
     def sync(self):
-        self.lib.check(self.lib.L.idocp_b200_sync(self._h))
+        self.lib.check(self._f("sync")(self._h))
 
     def launchCount(self):
         n = C.c_longlong(0)
-        self.lib.check(self.lib.L.idocp_b200_launch_count(self._h, C.byref(n)))
+        self.lib.check(self._f("launch_count")(self._h, C.byref(n)))
         return n.value
 
     def stream(self):
         s = C.c_void_p()
-        self.lib.check(self.lib.L.idocp_b200_stream(self._h, C.byref(s)))
+        self.lib.check(self._f("stream")(self._h, C.byref(s)))
         return s.value or 0
 
     def setProfiling(self, enabled):
-        self.lib.check(self.lib.L.idocp_b200_set_profiling(self._h, int(enabled)))
+        self.lib.check(self._f("set_profiling")(self._h, int(enabled)))
 
     def getProfile(self):
         cap = 16
         names = (C.c_char_p * cap)()
         ms = np.zeros(cap)
         calls = (C.c_longlong * cap)()
-        n = self.lib.check(self.lib.L.idocp_b200_get_profile(self._h, cap, names, dptr(ms), calls))
+        n = self.lib.check(self._f("get_profile")(self._h, cap, names, dptr(ms), calls))
         return {names[i].decode(): (ms[i], calls[i]) for i in range(n)}
 
 
@@ -349,96 +363,16 @@ class UnParNMPCSolver(_BatchSolver):
     kind = SOLVER_UNPARNMPC
 
     def initBackwardCorrection(self, t):
-        self.lib.check(self.lib.L.idocp_b200_init_backward_correction(self._h, float(t)))
+        self.lib.check(self._f("init_backward_correction")(self._h, float(t)))
 
 
-class ShardedSolver:
-    """One UnOCPSolver / UnParNMPCSolver over several GPUs of one node (idocp_b200_create_sharded): the batch is split into
-    contiguous shards, one device + stream per shard, no collective.  Same method names as the single-device classes for
-    the reference API; arrays are (batch, ...) over the WHOLE batch."""
+class ShardedSolver(_BatchSolver):
+    """One UnOCPSolver / UnParNMPCSolver (`kind`) over several GPUs of one node: the batch is split into contiguous shards,
+    one device + stream per shard, no collective.  Same methods and argument shapes as the single-device classes; arrays
+    are (batch, ...) over the WHOLE batch."""
 
     def __init__(self, problem, batch, devices, kind=SOLVER_UNOCP, lib=None):
-        self.lib = lib or capi.default_library()
-        self.batch, self.N, self.kind, self.problem = int(batch), int(problem.N), kind, problem
-        self._h = C.c_void_p()
-        devs = (C.c_int * len(devices))(*[int(d) for d in devices])
-        self.lib.check(self.lib.L.idocp_b200_create_sharded(C.byref(problem), kind, self.batch, devs, len(devices),
-                                                            C.byref(self._h)))
-        n = C.c_int(0)
-        first = (C.c_int * (len(devices) + 1))()
-        self.lib.check(self.lib.L.idocp_b200_sharded_num_shards(self._h, C.byref(n), first))
-        self.first = list(first)
+        self.kind = kind
+        super().__init__(problem, batch, lib=lib, devices=devices)
 
-    def close(self):
-        if getattr(self, "_h", None):
-            self.lib.L.idocp_b200_sharded_destroy(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def _x(self, a):
-        a = np.ascontiguousarray(np.asarray(a, dtype=np.float64))
-        if a.shape != (self.batch, DIMV):
-            raise ValueError("expected an array of shape (%d, %d)" % (self.batch, DIMV))
-        return a
-
-    def setSolution(self, name, value):
-        value = np.ascontiguousarray(np.asarray(value, dtype=np.float64))
-        if value.shape not in ((DIMV,), (self.batch, DIMV)):
-            raise ValueError("setSolution: bad shape %s" % (value.shape,))
-        self.lib.check(self.lib.L.idocp_b200_sharded_set_solution(self._h, name.encode(), dptr(value), int(value.ndim == 1)))
-
-    def initConstraints(self):
-        self.lib.check(self.lib.L.idocp_b200_sharded_init_constraints(self._h))
-
-    def initBackwardCorrection(self, t):
-        self.lib.check(self.lib.L.idocp_b200_sharded_init_backward_correction(self._h, float(t)))
-
-    def setTaskReference(self, table):
-        table = np.ascontiguousarray(table, dtype=np.float64)
-        self.lib.check(self.lib.L.idocp_b200_sharded_set_task_reference(self._h, dptr(table)))
-
-    def updateSolution(self, t, q, v, line_search=False):
-        q, v = self._x(q), self._x(v)
-        self.lib.check(self.lib.L.idocp_b200_sharded_update_solution(self._h, float(t), dptr(q), dptr(v), int(line_search)))
-
-    def computeKKTResidual(self, t, q, v):
-        q, v = self._x(q), self._x(v)
-        self.lib.check(self.lib.L.idocp_b200_sharded_compute_kkt_residual(self._h, float(t), dptr(q), dptr(v)))
-
-    def KKTError(self):
-        out = np.zeros(self.batch)
-        self.lib.check(self.lib.L.idocp_b200_sharded_kkt_error(self._h, dptr(out)))
-        return out
-
-    def getSolution(self, name):
-        nst = self.N + 1 if (name in ("q", "v", "lmd", "gmm") and self.kind == SOLVER_UNOCP) else self.N
-        out = np.zeros((self.batch, nst, DIMV))
-        self.lib.check(self.lib.L.idocp_b200_sharded_get_solution(self._h, name.encode(), dptr(out)))
-        return out
-
-    def getStageSolution(self, name, stage, out=None):
-        if out is None:
-            out = np.zeros((self.batch, DIMV))
-        self.lib.check(self.lib.L.idocp_b200_sharded_get_stage_solution(self._h, name.encode(), int(stage), dptr(out)))
-        return out
-
-    def getStepSizes(self):
-        p, d = np.zeros(self.batch), np.zeros(self.batch)
-        self.lib.check(self.lib.L.idocp_b200_sharded_get_step_sizes(self._h, dptr(p), dptr(d)))
-        return p, d
-
-    def getStatus(self):
-        out = np.zeros(self.batch, dtype=np.int32)
-        self.lib.check(self.lib.L.idocp_b200_sharded_get_status(self._h, out.ctypes.data_as(C.POINTER(C.c_int))))
-        return out
-
-    def clearLineSearchFilter(self):
-        self.lib.check(self.lib.L.idocp_b200_sharded_clear_line_search_filter(self._h))
-
-    def sync(self):
-        self.lib.check(self.lib.L.idocp_b200_sharded_sync(self._h))
+    initBackwardCorrection = UnParNMPCSolver.initBackwardCorrection

@@ -378,6 +378,8 @@ int idocp_b200_fb_create_sharded(const idocp_b200_fb_problem* problem, const ido
                                  const int* devices, int n_devices, idocp_b200_fb_sharded** out);
 int idocp_b200_fb_sharded_destroy(idocp_b200_fb_sharded* s);
 int idocp_b200_fb_sharded_num_shards(const idocp_b200_fb_sharded* s, int* n, int* first);
+/* the single-device solver behind shard `index` (borrowed), as idocp_b200_sharded_shard */
+int idocp_b200_fb_sharded_shard(idocp_b200_fb_sharded* s, int index, idocp_b200_fb_solver** out);
 int idocp_b200_fb_sharded_set_solution(idocp_b200_fb_sharded* s, const char* name, const double* value, int per_instance);
 int idocp_b200_fb_sharded_set_cost_reference(idocp_b200_fb_sharded* s, int kind, int index, const double* q_ref, const double* v_ref);
 int idocp_b200_fb_sharded_discretize(idocp_b200_fb_sharded* s, double t, int cap, int* kind, int* index, double* stage_t, double* dt,

@@ -277,12 +277,12 @@ class OCPSolver {
   OCPSolver(const Robot& robot, const std::shared_ptr<CostFunction>& cost,
             const std::shared_ptr<Constraints>& constraints, const double T, const int N, const int max_num_impulse = 0,
             const int nthreads = 1, const int batch = 1, const int device = 0)
-      : OCPSolver(robot, cost, constraints, T, N, max_num_impulse, nthreads, batch, std::vector<int>{device}, false) {}
+      : OCPSolver(robot, cost, constraints, T, N, max_num_impulse, nthreads, batch, std::vector<int>{device}) {}
   // the batch sharded over several GPUs of this node by ONE solver object (idocp_b200_fb_create_sharded): the GPU counterpart
-  // of the reference's nthreads
+  // of the reference's nthreads.  One device is one shard.
   OCPSolver(const Robot& robot, const std::shared_ptr<CostFunction>& cost,
             const std::shared_ptr<Constraints>& constraints, const double T, const int N, const int max_num_impulse,
-            const int nthreads, const int batch, const std::vector<int>& devices, const bool sharded = true)
+            const int nthreads, const int batch, const std::vector<int>& devices)
       : cost_(cost), batch_(batch) {
     if (T <= 0) detail::die("invalid value: T must be positive!");
     if (N <= 0) detail::die("invalid value: N must be positive!");
@@ -294,8 +294,7 @@ class OCPSolver {
       // UnconstrainedDynamics; exact eliminations of one KKT system, so the iterates agree up to rounding (stated, not
       // checkable here: the reference cannot be built).  Forwarded to the specialised GPU solver.
       if (max_num_impulse != 0) detail::die("idocp_b200: a fixed-base robot has no contacts: max_num_impulse must be 0");
-      un_ = sharded ? std::make_shared<UnOCPSolver>(robot, cost, constraints, T, N, nthreads, batch, devices)
-                    : std::make_shared<UnOCPSolver>(robot, cost, constraints, T, N, nthreads, batch, devices[0]);
+      un_ = std::make_shared<UnOCPSolver>(robot, cost, constraints, T, N, nthreads, batch, devices);
       return;
     }
     if (!cost || !constraints) detail::die("idocp_b200: cost and constraints must not be null");
@@ -328,15 +327,9 @@ class OCPSolver {
     detail::check(idocp_b200_contact_sequence_create(4, 2 * max_num_impulse + 2, &cs));
     cs_.reset(cs, [](idocp_b200_contact_sequence* x) { idocp_b200_contact_sequence_destroy(x); });
     if (devices.empty()) detail::die("idocp_b200: OCPSolver needs at least one device");
-    if (sharded) {
-      idocp_b200_fb_sharded* sh = nullptr;
-      detail::check(idocp_b200_fb_create_sharded(&p, cs, batch, devices.data(), static_cast<int>(devices.size()), &sh));
-      sh_.reset(sh, [](idocp_b200_fb_sharded* x) { idocp_b200_fb_sharded_destroy(x); });
-    } else {
-      idocp_b200_fb_solver* h = nullptr;
-      detail::check(idocp_b200_fb_create(&p, cs, batch, devices[0], &h));
-      h_.reset(h, [](idocp_b200_fb_solver* x) { idocp_b200_fb_destroy(x); });
-    }
+    idocp_b200_fb_sharded* sh = nullptr;
+    detail::check(idocp_b200_fb_create_sharded(&p, cs, batch, devices.data(), static_cast<int>(devices.size()), &sh));
+    sh_.reset(sh, [](idocp_b200_fb_sharded* x) { idocp_b200_fb_sharded_destroy(x); });
     prob_ = p;
   }
   int batch() const { return batch_; }
@@ -362,18 +355,18 @@ class OCPSolver {
   // setSolution(name, value): broadcast to every instance and stage ("f": one 3-vector for every contact)
   void setSolution(const std::string& name, const VectorXd& value) {
     if (un_) { un_->setSolution(name, value); return; }
-    detail::check(fb_set_solution(name.c_str(), value.data(), 0));
+    detail::check(idocp_b200_fb_sharded_set_solution(sh_.get(), name.c_str(), value.data(), 0));
   }
   void setSolution(const std::string& name, const Vector3d& value) {
-    detail::check(fb_set_solution(name.c_str(), value.d, 0));
+    detail::check(idocp_b200_fb_sharded_set_solution(sh_.get(), name.c_str(), value.d, 0));
   }
   void setSolution(const std::string& name, const double* value_per_instance) {
-    detail::check(fb_set_solution(name.c_str(), value_per_instance, 1));
+    detail::check(idocp_b200_fb_sharded_set_solution(sh_.get(), name.c_str(), value_per_instance, 1));
   }
   void initConstraints(const double t) {
     if (un_) { un_->initConstraints(); return; }
     sampleReference(t);
-    detail::check(fb_init_constraints(t));
+    detail::check(idocp_b200_fb_sharded_init_constraints(sh_.get(), t));
   }
   void updateSolution(const double t, const VectorXd& q, const VectorXd& v, const bool line_search = false) {
     if (un_) { un_->updateSolution(t, q, v, line_search); return; }
@@ -383,7 +376,7 @@ class OCPSolver {
   void updateSolution(const double t, const double* q, const double* v, const bool line_search = false) {
     if (un_) { un_->updateSolution(t, q, v, line_search); return; }
     sampleReference(t);
-    detail::check(fb_update_solution(t, q, v, line_search ? 1 : 0));
+    detail::check(idocp_b200_fb_sharded_update_solution(sh_.get(), t, q, v, line_search ? 1 : 0));
   }
   void computeKKTResidual(const double t, const VectorXd& q, const VectorXd& v) {
     if (un_) { un_->computeKKTResidual(t, q, v); return; }
@@ -393,19 +386,19 @@ class OCPSolver {
   void computeKKTResidual(const double t, const double* q, const double* v) {
     if (un_) { un_->computeKKTResidual(t, q, v); return; }
     sampleReference(t);
-    detail::check(fb_compute_kkt_residual(t, q, v));
+    detail::check(idocp_b200_fb_sharded_compute_kkt_residual(sh_.get(), t, q, v));
   }
   void clearLineSearchFilter() {
     if (un_) { un_->clearLineSearchFilter(); return; }
-    detail::check(fb_clear_line_search_filter());
+    detail::check(idocp_b200_fb_sharded_clear_line_search_filter(sh_.get()));
   }
   // assert(isWellDefined()) of OCPDiscretizer::discretizeOCP as a run-time error (default) or ignored like a Release build
-  void setStrictDiscretization(bool strict) { detail::check(fb_set_strict_discretization(strict ? 1 : 0)); }
+  void setStrictDiscretization(bool strict) { detail::check(idocp_b200_fb_sharded_set_strict_discretization(sh_.get(), strict ? 1 : 0)); }
   double KKTError() { return KKTErrors()[0]; }
   std::vector<double> KKTErrors() {
     if (un_) return un_->KKTErrors();
     std::vector<double> out(batch_);
-    detail::check(fb_kkt_error(out.data()));
+    detail::check(idocp_b200_fb_sharded_kkt_error(sh_.get(), out.data()));
     return out;
   }
   // getSolution(name): the grid stages 0..N (q, v) or 0..N-1 (a, f, u) of one instance (ocp_solver.cpp:244-280)
@@ -417,7 +410,7 @@ class OCPSolver {
     for (int e = 0; e < n; ++e) {
       const bool grid = kind_[e] == 0, terminal = kind_[e] == 4;
       if (!(grid || (terminal && (name == "q" || name == "v")))) continue;
-      const int dim = fb_get(e, name.c_str(), buf.data());
+      const int dim = idocp_b200_fb_sharded_get(sh_.get(), e, name.c_str(), buf.data());
       detail::check(dim);
       VectorXd x(name == "f" ? dimf_[e] : dim);
       if (name == "f") {   // f_stack(): the active contacts only
@@ -438,7 +431,7 @@ class OCPSolver {
     for (int e = 0; e < n; ++e) {
       if (kind_[e] != 0 || index_[e] != time_stage) continue;
       std::vector<double> buf(static_cast<size_t>(batch_) * 12 * 36);
-      detail::check(fb_get(e, "K", buf.data()));
+      detail::check(idocp_b200_fb_sharded_get(sh_.get(), e, "K", buf.data()));
       Kq.assign(12 * 18, 0.0);
       Kv.assign(12 * 18, 0.0);
       for (int r = 0; r < 12; ++r)
@@ -452,9 +445,14 @@ class OCPSolver {
   }
   void sync() {
     if (un_) { un_->sync(); return; }
-    detail::check(fb_sync());
+    detail::check(idocp_b200_fb_sharded_sync(sh_.get()));
   }
-  idocp_b200_fb_solver* handle() { return h_.get(); }
+  // the single-device solver of shard `shard` (the whole batch when the solver was built on one device)
+  idocp_b200_fb_solver* handle(int shard = 0) {
+    idocp_b200_fb_solver* h = nullptr;
+    detail::check(idocp_b200_fb_sharded_shard(sh_.get(), shard, &h));
+    return h;
+  }
   // time of the first scheduled discrete event (impulse or lift); false when the schedule has none
   bool firstEventTime(double& time) const {
     int phases = 0, impulses = 0, lifts = 0;
@@ -474,7 +472,7 @@ class OCPSolver {
     return any;
   }
   // first control input of every instance: out [batch][12]
-  void getFirstControlInput(double* out) { detail::check(fb_get(0, "u", out)); }
+  void getFirstControlInput(double* out) { detail::check(idocp_b200_fb_sharded_get(sh_.get(), 0, "u", out)); }
 
  private:
   static void pack(const ContactStatus& s, std::vector<int>& a, std::vector<double>& pts) {
@@ -488,8 +486,8 @@ class OCPSolver {
     const int cap = IDOCP_B200_MAX_GRID + 1 + 3 * IDOCP_B200_MAX_EVENTS;
     kind_.assign(cap, 0); index_.assign(cap, 0); t_.assign(cap, 0.0); dimf_.assign(cap, 0);
     std::vector<int> act(static_cast<size_t>(cap) * 4, 0);
-    const int n = fb_discretize(t_last_, cap, kind_.data(), index_.data(), t_.data(), nullptr, dimf_.data(), nullptr,
-                                           act.data());
+    const int n = idocp_b200_fb_sharded_discretize(sh_.get(), t_last_, cap, kind_.data(), index_.data(), t_.data(), nullptr,
+                                                   dimf_.data(), nullptr, act.data());
     detail::check(n);
     active_.assign(n, {0, 0, 0, 0});
     for (int e = 0; e < n; ++e)
@@ -506,7 +504,7 @@ class OCPSolver {
       cost_->fbConfig()->update_q_ref(t_[e], q_ref);
       const int kind = kind_[e] == 4 ? 0 : kind_[e];
       const VectorXd v_ref = cost_->fbConfig()->v_ref(t_[e]);
-      detail::check(fb_set_cost_reference(kind, index_[e], q_ref.data(), v_ref.data()));
+      detail::check(idocp_b200_fb_sharded_set_cost_reference(sh_.get(), kind, index_[e], q_ref.data(), v_ref.data()));
     }
   }
   void replicate(const VectorXd& q, const VectorXd& v) {
@@ -521,20 +519,8 @@ class OCPSolver {
   }
   std::shared_ptr<CostFunction> cost_;
   std::shared_ptr<idocp_b200_contact_sequence> cs_;
-  std::shared_ptr<idocp_b200_fb_solver> h_;
-  std::shared_ptr<idocp_b200_fb_sharded> sh_;   // set instead of h_ by the device-list constructor
+  std::shared_ptr<idocp_b200_fb_sharded> sh_;
   std::shared_ptr<UnOCPSolver> un_;             // fixed-base robot without contacts: the specialised solver does the work
-  // the C-ABI entry points of this solver: single-device or sharded (same arguments behind the handle)
-#define IDOCP_B200_FB_FWD(name)                                                                       \
-  template <typename... Args>                                                                         \
-  int fb_##name(Args... args) {                                                                       \
-    return sh_ ? idocp_b200_fb_sharded_##name(sh_.get(), args...) : idocp_b200_fb_##name(h_.get(), args...); \
-  }
-  IDOCP_B200_FB_FWD(set_solution) IDOCP_B200_FB_FWD(init_constraints) IDOCP_B200_FB_FWD(update_solution)
-  IDOCP_B200_FB_FWD(compute_kkt_residual) IDOCP_B200_FB_FWD(clear_line_search_filter) IDOCP_B200_FB_FWD(set_strict_discretization)
-  IDOCP_B200_FB_FWD(kkt_error) IDOCP_B200_FB_FWD(get) IDOCP_B200_FB_FWD(sync) IDOCP_B200_FB_FWD(discretize)
-  IDOCP_B200_FB_FWD(set_cost_reference)
-#undef IDOCP_B200_FB_FWD
   idocp_b200_fb_problem prob_;
   int batch_ = 1;
   double t_last_ = 0.0;

@@ -4,6 +4,7 @@
 namespace emu {
 Block* g_block = nullptr;
 uint3_emu threadIdx_, blockIdx_, blockDim_, gridDim_;
+long long g_event_serial = 0, g_live_events = 0;
 static const size_t kStack = 256 * 1024;
 
 static void switch_to(int next) {
@@ -110,3 +111,6 @@ void launch(dim3 grid, dim3 block, size_t smem_bytes, const std::function<void()
   g_block = nullptr;
 }
 }  // namespace emu
+
+// emulator build only (not part of include/idocp_b200.h): lets the tests check that destroying a handle releases its events
+extern "C" int idocp_b200_emu_live_events(void) { return static_cast<int>(emu::g_live_events); }

@@ -58,6 +58,8 @@ struct Block {
 };
 extern Block* g_block;
 extern thread_local int t_dummy;
+// cudaEventCreate hands out distinct non-null tokens; events created and not yet destroyed (idocp_b200_emu_live_events)
+extern long long g_event_serial, g_live_events;
 void yield();
 void warp_barrier();
 void block_barrier();
@@ -185,8 +187,15 @@ inline cudaError_t cudaDeviceSynchronize() { return 0; }
 inline cudaError_t cudaGetLastError() { return 0; }
 inline cudaError_t cudaPeekAtLastError() { return 0; }
 inline const char* cudaGetErrorString(cudaError_t) { return "emu"; }
-inline cudaError_t cudaEventCreate(cudaEvent_t* e) { *e = nullptr; return 0; }
-inline cudaError_t cudaEventDestroy(cudaEvent_t) { return 0; }
+inline cudaError_t cudaEventCreate(cudaEvent_t* e) {
+  *e = reinterpret_cast<cudaEvent_t>(++emu::g_event_serial);
+  ++emu::g_live_events;
+  return 0;
+}
+inline cudaError_t cudaEventDestroy(cudaEvent_t e) {
+  if (e) --emu::g_live_events;
+  return 0;
+}
 inline cudaError_t cudaEventRecord(cudaEvent_t, cudaStream_t = nullptr) { return 0; }
 inline cudaError_t cudaEventSynchronize(cudaEvent_t) { return 0; }
 inline cudaError_t cudaEventElapsedTime(float* ms, cudaEvent_t, cudaEvent_t) { *ms = 0.f; return 0; }
