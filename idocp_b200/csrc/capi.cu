@@ -575,7 +575,7 @@ static int unocp_update(idocp_b200_solver* h, const double* d_q, const double* d
     // two swap roles
     IDOCP_LAUNCH(h, KC_STEP_MIN, k_step_min, (h->Bp + 127) / 128, 128, 0, h->L, override_alpha);
     const long ul_tasks = static_cast<long>(h->N + 1) * h->L.G;
-    const int ul_grid = static_cast<int>(std::min<long>((ul_tasks + UL_WARPS - 1) / UL_WARPS, static_cast<long>(IDOCP_UL_CTAS_PER_SM) * h->sm_count));
+    const int ul_grid = static_cast<int>(std::min<long>((ul_tasks + UL_WARPS - 1) / UL_WARPS, static_cast<long>(UL_CTAS_PER_SM) * h->sm_count));
     if (task && h->kkt_tracking)
       IDOCP_LAUNCH(h, KC_UPDATE_LINEARIZE, (k_update_linearize<true, true>), ul_grid, UL_THREADS, kUlSmem, h->d_prob, h->L);
     else if (task)

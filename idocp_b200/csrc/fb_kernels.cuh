@@ -129,20 +129,11 @@ enum { FBM_SET = 0, FBM_ADD = 1, FBM_SUB = 2 };
 // unchanged, so the bits do not depend on the tiling.  FBM_SET starts a chain with the plain product a_0 b_0;
 // FBM_ADD / FBM_SUB start it from init(i, j); store(i, j, value) receives the finished element.
 // The caller separates dependent calls with __syncthreads().
-// `rot` (optional): independent products issued back to back without a barrier start their tile -> thread assignment
-// where the previous one stopped (*rot is advanced by the tile count), so that e.g. four 81-tile products keep all
-// 128 threads busy (3 rounds) instead of using threads 0..80 four times.
 template <int MODE, class Init, class Store>
 __device__ __forceinline__ void fb_mm_simt_f(int m, int n, int k, const double* __restrict__ A, int ars, int acs, const double* __restrict__ B,
-                                        int brs, int bcs, Init init, Store store, int* rot = nullptr) {
+                                        int brs, int bcs, Init init, Store store) {
   const int tm = (m + 1) >> 1, tn = (n + 1) >> 1, total = tm * tn;
-  int first = threadIdx.x;
-  if (rot) {
-    first = (int)threadIdx.x - *rot;
-    if (first < 0) first += blockDim.x;
-    *rot = (*rot + total) % (int)blockDim.x;
-  }
-  for (int t = first; t < total; t += blockDim.x) {
+  for (int t = threadIdx.x; t < total; t += blockDim.x) {
     const int i0 = t / tn, j0 = t - i0 * tn;
     const int i1 = i0 + tm, j1 = j0 + tn;
     const bool hi = i1 < m, hj = j1 < n;
@@ -187,6 +178,8 @@ __device__ __forceinline__ void fb_mm_simt_f(int m, int n, int k, const double* 
 // from two operand loads, i.e. 5 x fewer shared-memory wavefronts and 8 x fewer FP64 instructions for the same chain.
 // A warp owns an 8 x 16 strip of C (two tiles sharing the A fragment: two independent accumulator chains).
 // Fragment layout (PTX ISA, m8n8k4 .f64): a = A[g][t], b = B[t][g], c / d = C[g][2 t + {0, 1}] with g = lane / 4, t = lane % 4.
+// `rot` (optional): independent products issued back to back without a barrier start their strip -> warp assignment where
+// the previous one stopped (*rot is advanced by the strip count), so that the warps share out the strips of all of them.
 // ---------------------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void fb_dmma(double& d0, double& d1, double a, double b) {
 #ifndef IDOCP_B200_EMU
@@ -198,9 +191,6 @@ __device__ __forceinline__ void fb_dmma(double& d0, double& d1, double a, double
 template <int MODE, class Init, class Store>
 __device__ __forceinline__ void fb_mm_f(int m, int n, int k, const double* __restrict__ A, int ars, int acs, const double* __restrict__ B,
                                         int brs, int bcs, Init init, Store store, int* rot = nullptr) {
-#ifdef IDOCP_FB_MM_SIMT
-  fb_mm_simt_f<MODE>(m, n, k, A, ars, acs, B, brs, bcs, init, store, rot);
-#else
   const int nw = blockDim.x >> 5, warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
   const int tm = (m + 7) >> 3, tn = (n + 15) >> 4, total = tm * tn;
   int first = warp;
@@ -239,7 +229,6 @@ __device__ __forceinline__ void fb_mm_f(int m, int n, int k, const double* __res
       if (cb + 1 < n) store(row, cb + 1, c11);
     }
   }
-#endif
 }
 template <int MODE>
 __device__ __forceinline__ void fb_mm(int m, int n, int k, const double* __restrict__ A, int ars, int acs, const double* __restrict__ B,
@@ -635,35 +624,6 @@ struct FbLin {
   double cdJ[FB_NC * FB_NV], cdw[FB_NC];   // ContactDistance: J2 rows and dt dual / slack (written and read only while it is active)
 };
 
-// Optional per-phase cycle counters of the three heavy kernels (tools/fb_phase_clocks.py builds a variant library with
-// -DFB_PHASE_CLOCKS; the product library carries none of this).
-#ifdef FB_PHASE_CLOCKS
-__device__ unsigned long long g_fb_phase[3][32];
-#define FB_PHASE_BEGIN() long long fb_t_prev = clock64()
-#define FB_PHASE(kernel, i)                                                               \
-  do {                                                                                    \
-    __syncthreads();                                                                      \
-    if (threadIdx.x == 0) {                                                               \
-      const long long t = clock64();                                                      \
-      atomicAdd(&g_fb_phase[kernel][i], (unsigned long long)(t - fb_t_prev));             \
-      fb_t_prev = t;                                                                      \
-    }                                                                                     \
-  } while (0)
-#define FBW_PHASE(kernel, i)                                                              \
-  do {                                                                                    \
-    __syncwarp();                                                                         \
-    if ((threadIdx.x & 31) == 0) {                                                        \
-      const long long t = clock64();                                                      \
-      atomicAdd(&g_fb_phase[kernel][i], (unsigned long long)(t - fb_t_prev));             \
-      fb_t_prev = t;                                                                      \
-    }                                                                                     \
-  } while (0)
-#else
-#define FB_PHASE_BEGIN()
-#define FB_PHASE(kernel, i)
-#define FBW_PHASE(kernel, i)
-#endif
-
 struct FbRobotWork {
   // inputs (same order as FbSol)
   double lmd[FB_NV], gmm[FB_NV], q[FB_NQ], v[FB_NV], a[FB_NV], u[FB_NU], beta[FB_NV], nu_passive[FB_NPASS], f[FB_MAXF], mu[FB_MAXF],
@@ -951,13 +911,9 @@ __device__ __noinline__ void fbw_dminus(const double* R, const double* p, const 
     }
 }
 
-#ifndef FB_ROBOT_WARPS
-#define FB_ROBOT_WARPS 6   // x 2 CTAs per SM: 12 warps (18.6 KB of shared memory and 168 registers each)
-#endif
-#ifndef FB_ROBOT_MINB
-#define FB_ROBOT_MINB 2
-#endif
-#define FB_LS_WARPS 5      // k_fb_ls_eval (FbLsWork, 23 KB per warp)
+constexpr int FB_ROBOT_WARPS = 6;   // x 2 CTAs per SM: 12 warps (18.6 KB of shared memory and 168 registers each)
+constexpr int FB_ROBOT_MINB = 2;
+constexpr int FB_LS_WARPS = 5;      // k_fb_ls_eval (FbLsWork, 23 KB per warp)
 
 template <bool RESIDUAL_ONLY>
 __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot(FbArrays A, FbLin* lin) {
@@ -979,7 +935,6 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
   FbDir& Dr = A.dir[rec];
   FbLin& L = lin[rec];
 
-  FB_PHASE_BEGIN();
   // ---- load ----
   // every load of the lane is issued before its first store (a copy loop through generic pointers keeps load -> store order:
   // one DRAM round trip per element)
@@ -1006,7 +961,6 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
     if (lane < FB_NQ) w.qprev[lane] = p0;
   }
   __syncwarp();
-  FBW_PHASE(2, 0);
   if (lane < FB_MAXF) {   // forces of inactive contacts are zero for the dynamics; stacks of the active ones
     const int i = lane / 3;
     w.fm[lane] = (!terminal && el.active[i]) ? w.f[lane] : 0.0;
@@ -1032,7 +986,6 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
     if (lane == 2) fbw_dminus(w.relR[2], w.relp[2], w.relJ[2], w.Fqq_prev6);
   }
   __syncwarp();
-  FBW_PHASE(2, 1);
   const double* J6c = w.relJ[0];
   const double* Fqq6 = w.relJ[1];
 
@@ -1139,7 +1092,6 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
     }
     return;
   }
-  FBW_PHASE(2, 2);
   // augmentDualResidual: joint limits on the lq / lv / lu tails, friction cones on lf
   if (lane >= 6 && lane < FB_NV) {
     const int j = lane - 6;
@@ -1214,14 +1166,11 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
   }
   __syncwarp();
 
-  FBW_PHASE(2, 3);
   // ---- contact dynamics: kinematics, RNEA + derivatives, contact rows ----
   const double baumgarte = pr.T / pr.N;
   if (!impulse) {
     fbw_forward_kinematics(w, lane, w.q, w.v, w.a);
-    FBW_PHASE(2, 4);
     fbw_rnea_derivatives(w, lane, ANYMAL_GRAVITY, true, L, true);
-    FBW_PHASE(2, 5);
     if (lane < FB_NU) L.IDC[6 + lane] -= w.u[lane];
   } else {
     fbw_forward_kinematics(w, lane, w.q, nullptr, w.a);
@@ -1230,7 +1179,6 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
     __syncwarp();
     fbw_forward_kinematics(w, lane, w.q, w.t18, nullptr);
   }
-  FBW_PHASE(2, 6);
   // rows of every active contact, one after the other; lane = dof
   {
     int k = 0;
@@ -1312,7 +1260,6 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
     }
   }
   __syncwarp();
-  FBW_PHASE(2, 7);
   // augment: lq += dt dIDdq^T beta, lv += dt dIDdv^T beta, la += dt M^T beta, lf -= dt dCda beta, lu ...
   {
     const double* dIDdq = L.dIDCdqv;
@@ -1371,7 +1318,6 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
     __syncwarp();
   }
 
-  FBW_PHASE(2, 8);
   if (!RESIDUAL_ONLY) {
     // ---- cost Hessian (sparse part of Qxx, Qaa, Qff) and condenseSlackAndDual ----
     FBW_FOR(x, 36) {
@@ -1460,7 +1406,6 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
     }
   }
 
-  FBW_PHASE(2, 9);
   // ---- ForwardSwitchingConstraint::linearizeSwitchingConstraint (:27-68) ----
   if (dimi > 0) {
     const double c1 = el.dt + el.dt_next, c2 = el.dt * el.dt_next;
@@ -1515,7 +1460,6 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
       for (int l = 0; l < dimi; ++l) la = fma(L.Phia[l * FB_NV + j], w.xi[l], la);
     }
   }
-  FBW_PHASE(2, 10);
   // ---- store the stage vectors ----
   if (lane < FB_NV) { L.lq[lane] = lq; L.lv[lane] = lv; L.la[lane] = la; L.Fq[lane] = Fq; L.Fv[lane] = Fv; }
   if (lane < FB_MAXF) L.lf[lane] = lane < dimf ? lf : 0.0;
@@ -1611,11 +1555,9 @@ struct FbDenseWork {
 // 36 KB: six CTAs share the 228 KB of an SM (43.8 KB, five CTAs, with Qafqv and M^-1 / J M^-1 in storage of their own)
 static_assert(6 * (sizeof(FbDenseWork) + 1024) <= 228 * 1024, "six CTAs of k_fb_condense per SM");
 
-#ifndef IDOCP_FB_DENSE_MINB
-#define IDOCP_FB_DENSE_MINB 6
-#endif
+constexpr int FB_DENSE_MINB = 6;
 static_assert(FB_MAXF * FB_NV + FB_MAXF * FB_MAXF >= FB_NV * (FB_NV + 1), "the JMi / Sm scratch holds the 18 x 19 trailing matrix of LLT(M)");
-__global__ void __launch_bounds__(128, IDOCP_FB_DENSE_MINB) k_fb_condense(FbArrays A, const FbLin* lin) {
+__global__ void __launch_bounds__(128, FB_DENSE_MINB) k_fb_condense(FbArrays A, const FbLin* lin) {
   IDOCP_DYN_SMEM(FbDenseWork, wp);
   FbDenseWork& w = *wp;
   const int tid = threadIdx.x;
@@ -1644,13 +1586,11 @@ __global__ void __launch_bounds__(128, IDOCP_FB_DENSE_MINB) k_fb_condense(FbArra
   const int dimf = el.dimf, nvf = NV + dimf, dimi = el.sw ? el.dimi : 0;
   FbExp& Ex = A.exp[rec];
   FbDir& Dr = A.dir[rec];
-  FB_PHASE_BEGIN();
   fb_load<FB_NVF + FB_NVF * FB_NX>(w.IDC, L.IDC);
   fb_load<FB_NV * FB_NV>(w.Mm, L.Mm);
   fb_load<(offsetof(FbLin, Phix) - offsetof(FbLin, dCda)) / sizeof(double)>(w.dCda, L.dCda);
   if (tid == 0) w.info = 0;
   __syncthreads();
-  FB_PHASE(0, 0);
   // ---- MJtJinv = [[M, J^T], [J, 0]]^-1 by dense Cholesky ----
   {
     const int n = NV, ld = NVF;
@@ -1660,19 +1600,15 @@ __global__ void __launch_bounds__(128, IDOCP_FB_DENSE_MINB) k_fb_condense(FbArra
     // leaves the SM with five active warps
     // (the dense owner-per-element sweep fb_llt_factor_solve_cta<2, 3> took 36 barrier steps: 28 k of the 74 k cycles per stage)
     fb_minv_tree_cta(w.Mm, w.s.f.L, w.s.f.rd, w.Minv, w.s.f.fail, &w.info, 0);
-    FB_PHASE(0, 1);
-    FB_PHASE(0, 2);
     fb_mm<FBM_SET>(dimf, n, n, w.dCda, n, 1, w.Minv, n, 1, w.JMi, n);
     __syncthreads();
     fb_mm<FBM_SET>(dimf, dimf, n, w.JMi, n, 1, w.dCda, 1, n, w.Sm, dimf);
     __syncthreads();
-    FB_PHASE(0, 3);
     if (dimf > 0) {
       FB_FOR(x, dimf * dimf) { const int r = x / dimf; w.s.f.Si[x] = (x - r * dimf == r) ? 1.0 : 0.0; }
       __syncthreads();
       fb_llt_factor_solve_cta<1, 2>(w.Sm, dimf, dimf, w.s.f.Ls, dimf, w.s.f.rds, w.s.f.Si, dimf, dimf, &w.info, 100);
     }
-    FB_PHASE(0, 4);
     FB_FOR(x, dimf * dimf) { const int r = x / dimf, c = x - r * dimf; w.MJtJinv[(n + r) * ld + n + c] = -w.s.f.Si[x]; }
     fb_mm<FBM_SET>(n, dimf, dimf, w.JMi, 1, n, w.s.f.Si, dimf, 1, w.MJtJinv + n, ld);     // TR = (J Minv)^T S^-1
     __syncthreads();
@@ -1685,12 +1621,10 @@ __global__ void __launch_bounds__(128, IDOCP_FB_DENSE_MINB) k_fb_condense(FbArra
     FB_FOR(x, dimf * n) { const int r = x / n, c = x - r * n; w.MJtJinv[(n + r) * ld + c] = w.MJtJinv[c * ld + n + r]; }   // BL = TR^T
     __syncthreads();
   }
-  FB_PHASE(0, 5);
   // ---- condensing ----
   fb_mm<FBM_SET>(nvf, NX, nvf, w.MJtJinv, NVF, 1, w.dIDCdqv, NX, 1, w.MJ_dIDC, NX);
   fb_mv<FBM_SET>(nvf, nvf, w.MJtJinv, NVF, 1, w.IDC, w.MJ_IDC);
   __syncthreads();
-  FB_PHASE(0, 6);
   double* Qafqv = w.Qafqv;
   double* Qafu = w.s.Qafu;
   FB_FOR(x, NV * NX) { const int r = x / NX; Qafqv[x] = -w.Qaa[r] * w.MJ_dIDC[x]; }
@@ -1705,7 +1639,6 @@ __global__ void __launch_bounds__(128, IDOCP_FB_DENSE_MINB) k_fb_condense(FbArra
   FB_FOR(x, dimf * NX) Qafqv[NV * NX + x] = -Qafqv[NV * NX + x];
   fb_mv<FBM_SUB>(dimf, dimf, w.Qff, MAXF, 1, w.MJ_IDC + NV, w.laf + NV);
   __syncthreads();
-  FB_PHASE(0, 7);
   // Qxx -= MJ_dIDC^T Qafqv, starting from the sparse cost / constraint Hessian; the Qvq block is never read
   // (the Riccati sweep rebuilds it from Qqv, backward_riccati_recursion_factorizer.hxx:93) and is left untouched
   int rot = 0;   // tile rotation across the independent products below (fb_mm_f)
@@ -1777,7 +1710,6 @@ __global__ void __launch_bounds__(128, IDOCP_FB_DENSE_MINB) k_fb_condense(FbArra
       Kt.P[tid] = acc;
     }
   }
-  FB_PHASE(0, 8);
   // ---- expansion record ----
   fb_copy(Ex.MJtJinv, w.MJtJinv, NVF * NVF + NVF * NX + NVF);   // MJtJinv, MJ_dIDC, MJ_IDC
   fb_copy(Ex.Qafqv, Qafqv, NVF * NX);
@@ -1797,7 +1729,6 @@ __global__ void __launch_bounds__(128, IDOCP_FB_DENSE_MINB) k_fb_condense(FbArra
       Kt.Qxx[r * NX + c] = v;
     }
   }
-  FB_PHASE(0, 9);
 }
 
 
@@ -1837,10 +1768,8 @@ struct FbRicWork {
 
 static_assert(offsetof(FbRicWork, L) % 16 == 0, "warp_llt.cuh reads the factor two doubles at a time");
 static_assert(4 * (sizeof(FbRicWork) + 1024) <= 228 * 1024, "four CTAs of the backward recursion share the 228 KB of an SM");
-#ifndef IDOCP_FB_RIC_MINB
-#define IDOCP_FB_RIC_MINB 4
-#endif
-__global__ void __launch_bounds__(128, IDOCP_FB_RIC_MINB) k_fb_riccati_backward(FbArrays A) {
+constexpr int FB_RIC_MINB = 4;
+__global__ void __launch_bounds__(128, FB_RIC_MINB) k_fb_riccati_backward(FbArrays A) {
   IDOCP_DYN_SMEM(FbRicWork, wp);
   FbRicWork& w = *wp;
   const int tid = threadIdx.x, b = blockIdx.x, n = A.n_elems;
@@ -1863,7 +1792,6 @@ __global__ void __launch_bounds__(128, IDOCP_FB_RIC_MINB) k_fb_riccati_backward(
     __syncthreads();
     fb_copy(Rc.Pqq, w.Pqq, 3 * NV * NV + 2 * NV);
   }
-  FB_PHASE_BEGIN();
   for (int e = n - 2; e >= 0; --e) {
     const FbElem& el = A.elems[e];
     const bool impulse = el.kind == FB_IMPULSE;
@@ -1888,7 +1816,6 @@ __global__ void __launch_bounds__(128, IDOCP_FB_RIC_MINB) k_fb_riccati_backward(
     if (e > 0) fb_prefetch_l2(&A.kkt[(size_t)A.elems[e - 1].slot * A.B + b], (int)sizeof(FbKKT));
     if (tid == 0) w.info = 0;
     __syncthreads();
-    FB_PHASE(1, 0);
     double* Qqq = w.Qxx;
     double* Qqv = w.Qxx + NV;
     double* Qvv = w.Qxx + NV * NX + NV;
@@ -1902,7 +1829,6 @@ __global__ void __launch_bounds__(128, IDOCP_FB_RIC_MINB) k_fb_riccati_backward(
       FB_FOR(x, (NV - 6) * NV) { w.AtPvq[6 * NV + x] = dt * w.Pqq[6 * NV + x]; w.AtPvv[6 * NV + x] = dt * w.Pqv[6 * NV + x]; }
     }
     __syncthreads();
-    FB_PHASE(1, 1);
     fb_mm<FBM_ADD>(NV, NV, NV, w.Fvq, 1, NV, w.Pqv, 1, NV, w.AtPqq, NV);
     fb_mm<FBM_ADD>(NV, NV, NV, w.Fvq, 1, NV, w.Pvv, NV, 1, w.AtPqv, NV);
     if (!impulse) {
@@ -1915,7 +1841,6 @@ __global__ void __launch_bounds__(128, IDOCP_FB_RIC_MINB) k_fb_riccati_backward(
       fb_mm<FBM_SET>(NV, NV, NV, w.Fvv, 1, NV, w.Pvv, NV, 1, w.AtPvv, NV);
     }
     __syncthreads();
-    FB_PHASE(1, 2);
     // Factorize F: the three blocks are independent of each other, each gets its terms in the reference's order
     fb_mm<FBM_ADD>(NV, 6, 6, w.AtPqq, NV, 1, w.Fqq6, 6, 1, Qqq, NX);
     FB_FOR(x, NV * (NV - 6)) { const int r = x / (NV - 6), c = 6 + x - r * (NV - 6); Qqq[r * NX + c] += w.AtPqq[r * NV + c]; }
@@ -1926,7 +1851,6 @@ __global__ void __launch_bounds__(128, IDOCP_FB_RIC_MINB) k_fb_riccati_backward(
       FB_FOR(x, NV * (NV - 6)) { const int r = x / (NV - 6), c = 6 + x - r * (NV - 6); Qvv[r * NX + c] = fma(dt, w.AtPvq[r * NV + c], Qvv[r * NX + c]); }
     }
     __syncthreads();
-    FB_PHASE(1, 3);
     fb_mm<FBM_ADD>(NV, NV, NV, w.AtPqv, NV, 1, w.Fvq, NV, 1, Qqq, NX);
     fb_mm<FBM_ADD>(NV, NV, NV, w.AtPqv, NV, 1, w.Fvv, NV, 1, Qqv, NX);
     fb_mm<FBM_ADD>(NV, NV, NV, w.AtPvv, NV, 1, w.Fvv, NV, 1, Qvv, NX);
@@ -1943,7 +1867,6 @@ __global__ void __launch_bounds__(128, IDOCP_FB_RIC_MINB) k_fb_riccati_backward(
       }
     }
     __syncthreads();
-    FB_PHASE(1, 4);
     const double* Qxu = w.Qxu;   // 36 x 12, leading dimension NU
     if (!impulse) {
       // LLT(G), G = Quu (12 x 12), factor only: warp 0, lane = row, rows in registers (warp_llt.cuh).  Measured on the whole
@@ -1958,7 +1881,6 @@ __global__ void __launch_bounds__(128, IDOCP_FB_RIC_MINB) k_fb_riccati_backward(
         if (fail && tid == 0 && w.info == 0) w.info = 200 + fail;
       }
       __syncthreads();
-      FB_PHASE(1, 5);
       if (dimi == 0) {
         // K = -G^-1 Qxu^T, k = -G^-1 lu: one right-hand side per thread
         if (tid < NX) {
@@ -2016,7 +1938,6 @@ __global__ void __launch_bounds__(128, IDOCP_FB_RIC_MINB) k_fb_riccati_backward(
         __syncthreads();
       }
     }
-    FB_PHASE(1, 6);
     // ---- factorizeRiccatiFactorization ----
     FB_FOR(x, NV * NV) {
       const int r = x / NV, c = x - r * NV;
@@ -2032,7 +1953,6 @@ __global__ void __launch_bounds__(128, IDOCP_FB_RIC_MINB) k_fb_riccati_backward(
       fb_mm<FBM_SUB>(NV, NV, NU, w.K + NV, 1, NX, w.GK + NV, NX, 1, w.Pvv, NV);
       __syncthreads();
     }
-    FB_PHASE(1, 7);
     FB_FOR(x, NV * NV) {   // preserve the symmetry: one thread per unordered pair
       const int r = x / NV, c = x - r * NV;
       if (c >= r) {
@@ -2082,7 +2002,6 @@ __global__ void __launch_bounds__(128, IDOCP_FB_RIC_MINB) k_fb_riccati_backward(
       w.sv[j] = acc;
     }
     __syncthreads();
-    FB_PHASE(1, 8);
     if (dimi > 0) {
       fb_mm<FBM_SET>(NU, NX, dimi, Phiu, 1, NU, cM, NX, 1, w.DtM, NX);
       __syncthreads();
@@ -2098,11 +2017,9 @@ __global__ void __launch_bounds__(128, IDOCP_FB_RIC_MINB) k_fb_riccati_backward(
       fb_mv<FBM_SUB>(NV, dimi, Phix + NV, 1, NX, cm, w.sv);
       __syncthreads();
     }
-    FB_PHASE(1, 9);
     // store the factorisation; it stays in place as the "next" one
     fb_copy(Rc.K, w.K, (int)(offsetof(FbRic, cM) / sizeof(double)));
     if (tid < NV) { w.nsq[tid] = w.sq[tid]; w.nsv[tid] = w.sv[tid]; }
-    FB_PHASE(1, 10);
     if (tid == 0 && w.info) {
       FbDir& Dr = A.dir[(size_t)el.slot * A.B + b];
       if (Dr.info == 0.0) Dr.info = (double)w.info;
@@ -2143,13 +2060,11 @@ __global__ void __launch_bounds__(64) k_fb_riccati_forward(FbArrays A) {
     const FbKKT& Kt = A.kkt[(size_t)el.slot * A.B + b];
     const FbRic& Rc = A.ric[(size_t)el.slot * A.B + b];
     const double dt = el.dt;
-#ifndef IDOCP_FB_NO_PREFETCH
     if (e + 1 < n && A.elems[e + 1].kind != FB_TERMINAL) {   // the serial chain pays the DRAM latency of every stage otherwise
       const size_t nrec = (size_t)A.elems[e + 1].slot * A.B + b;
       fb_prefetch_l2(A.ric[nrec].K, (NU * NX + NU) * (int)sizeof(double));
       fb_prefetch_l2(A.kkt[nrec].Fqq6, (int)(offsetof(FbKKT, Phix) - offsetof(FbKKT, Fqq6)));
     }
-#endif
     if (!impulse) {
       if (tid < NU) {
         double acc = Rc.K[tid * NX] * dq[0];
@@ -2204,10 +2119,8 @@ __device__ inline double fb_fraction_to_boundary(double rate, int nn, const doub
   return mn;
 }
 
-#ifndef IDOCP_FB_EXP_MINB
-#define IDOCP_FB_EXP_MINB 0    // unspecified: 38 registers; a cap at 24 CTAs per SM (40 registers) measured 2 % slower (r2zzc)
-#endif
-__global__ void __launch_bounds__(64, IDOCP_FB_EXP_MINB) k_fb_expand(FbArrays A) {
+// no minimum CTAs per SM: 38 registers; a cap at 24 CTAs per SM (40 registers) measured 2 % slower (r2zzc)
+__global__ void __launch_bounds__(64) k_fb_expand(FbArrays A) {
   __shared__ double dx[FB_NX], du[FB_NU], daf[FB_NVF], dslack[FB_NCON], ddual[FB_NCON], steps[2 * FBC_NCOMP];
   const int tid = threadIdx.x;
   const int b = blockIdx.x / A.n_elems, e = blockIdx.x - b * A.n_elems;
@@ -2220,12 +2133,10 @@ __global__ void __launch_bounds__(64, IDOCP_FB_EXP_MINB) k_fb_expand(FbArrays A)
   FbDir& Dr = A.dir[rec];
   const FbRic& Rc = A.ric[rec];
   const FbSol& S = A.sol[rec];
-#ifndef IDOCP_FB_NO_PREFETCH
   // every thread walks its own row of P and of the expansion record below (one ascending fma chain per output): put all of the
   // CTA's DRAM requests in flight first, so that the walks find their lines in the L2
   fb_prefetch_l2(Rc.Pqq, (3 * NV * NV + 2 * NV) * (int)sizeof(double));
   if (!terminal) fb_prefetch_l2(A.exp[rec].MJtJinv, (int)offsetof(FbExp, Qafqv));
-#endif
   if (tid < NV) { dx[tid] = Dr.dq[tid]; dx[NV + tid] = Dr.dv[tid]; }
   if (tid >= 32 && tid < 32 + NU) du[tid - 32] = Dr.du[tid - 32];
   __syncthreads();
@@ -2361,10 +2272,8 @@ __global__ void k_fb_steps(FbArrays A) {
 // (ocp_linearizer.cpp:140-221, contact_dynamics.hxx:171-190, state_equation.hxx:96-108, split_solution.hxx:215-239)
 // grid = B * n_elems, 64 threads.  Reads dgmm of the NEXT stage, which no CTA of this kernel writes.
 // =====================================================================================================
-#ifndef IDOCP_FB_UPD_MINB
-#define IDOCP_FB_UPD_MINB 16   // 64 registers: 16 CTAs (32 warps) per SM; measured 1.07 -> 0.96 ms (r2zzc)
-#endif
-__global__ void __launch_bounds__(64, IDOCP_FB_UPD_MINB) k_fb_update(FbArrays A) {
+constexpr int FB_UPD_MINB = 16;   // 64 registers: 16 CTAs (32 warps) per SM; measured 1.07 -> 0.96 ms (r2zzc)
+__global__ void __launch_bounds__(64, FB_UPD_MINB) k_fb_update(FbArrays A) {
   __shared__ double dx[FB_NX], du[FB_NU], laf[FB_NVF], dbetamu[FB_NVF], dgn[FB_NV], dlmd[FB_NV], qn[FB_NQ], dqs[FB_NV], qs[FB_NQ];
   const int tid = threadIdx.x;
   const int b = blockIdx.x / A.n_elems, e = blockIdx.x - b * A.n_elems;
@@ -2377,14 +2286,12 @@ __global__ void __launch_bounds__(64, IDOCP_FB_UPD_MINB) k_fb_update(FbArrays A)
   const FbKKT& Kt = A.kkt[rec];
   const double ap = A.steps[2 * b], ad = A.steps[2 * b + 1];
   const double dt = el.dt;
-#ifndef IDOCP_FB_NO_PREFETCH
   if (!terminal) {   // the row walks below (see k_fb_expand)
     const FbExp& Ep = A.exp[rec];
     fb_prefetch_l2(Ep.MJtJinv, FB_NVF * FB_NVF * (int)sizeof(double));
     fb_prefetch_l2(Ep.Qafqv, (int)(sizeof(FbExp) - offsetof(FbExp, Qafqv)));
     if (!impulse) fb_prefetch_l2(Kt.Qxu, (FB_NX * FB_NV + FB_NPASS * FB_NV) * (int)sizeof(double));
   }
-#endif
   if (tid < NV) { dx[tid] = Dr.dq[tid]; dx[NV + tid] = Dr.dv[tid]; dlmd[tid] = Dr.dlmd[tid]; dqs[tid] = Dr.dq[tid]; }
   if (tid >= 32 && tid < 32 + NU) du[tid - 32] = Dr.du[tid - 32];
   if (tid < FB_NQ) qs[tid] = S.q[tid];
@@ -2571,10 +2478,7 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS) k_fb_init_distance(FbArra
 // s + alpha d)  ->  k_fb_ls_filter (thread per instance); finished instances drop out.
 // =====================================================================================================
 template <bool INITIAL>
-#ifndef IDOCP_FB_LS_MINB
-#define IDOCP_FB_LS_MINB 0
-#endif
-__global__ void __launch_bounds__(32 * FB_LS_WARPS, IDOCP_FB_LS_MINB) k_fb_ls_eval(FbArrays A, FbLin* lin) {
+__global__ void __launch_bounds__(32 * FB_LS_WARPS) k_fb_ls_eval(FbArrays A, FbLin* lin) {
   IDOCP_DYN_SMEM(FbLsWork, wbase);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int stage = blockIdx.x * FB_LS_WARPS + warp;

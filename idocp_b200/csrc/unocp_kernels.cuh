@@ -23,18 +23,10 @@
 
 namespace idocp_b200 {
 
-#ifndef IDOCP_LIN_MINB
-#define IDOCP_LIN_MINB 2   // min resident CTAs/SM of k_linearize (register cap = 65536 / (128 * MINB))
-#endif
-#ifndef IDOCP_UL_CTAS_PER_SM
-#define IDOCP_UL_CTAS_PER_SM 2   // persistent k_update_linearize: resident CTAs per SM (97 KB of shared memory each)
-#endif
-#ifndef IDOCP_RIC_MINB
-#define IDOCP_RIC_MINB 2
-#endif
-#ifndef IDOCP_EXP_MINB
-#define IDOCP_EXP_MINB 3   // k_expand holds its whole W record in registers (166): 3 warps per scheduler, 12 per SM
-#endif
+constexpr int LIN_MINB = 2;          // min resident CTAs/SM of k_linearize (register cap = 65536 / (128 * MINB))
+constexpr int UL_CTAS_PER_SM = 2;    // persistent k_update_linearize: resident CTAs per SM (97 KB of shared memory each)
+constexpr int RIC_MINB = 2;
+constexpr int EXP_MINB = 3;          // k_expand holds its whole W record in registers (166): 3 warps per scheduler, 12 per SM
 constexpr int WARPS_PER_CTA = 4;
 constexpr int OCTETS_PER_CTA = 4 * WARPS_PER_CTA;  // 16 octets, 128 threads
 constexpr int CTA_THREADS = 32 * WARPS_PER_CTA;
@@ -594,9 +586,9 @@ __device__ __forceinline__ void linearize_task(const DevProblem& P, const Layout
 
 // ACC = true: + the two acceleration-limit components (their own array L.XA; the six-component instantiations are untouched)
 template <bool RESIDUAL_ONLY, bool BACKWARD_EULER, bool TASK, bool ACC = false>
-__global__ void __launch_bounds__(CTA_THREADS, IDOCP_LIN_MINB) k_linearize(const DevProblem* __restrict__ Pp, Layout L,
-                                                                           const double* __restrict__ q0,
-                                                                           const double* __restrict__ v0) {
+__global__ void __launch_bounds__(CTA_THREADS, LIN_MINB) k_linearize(const DevProblem* __restrict__ Pp, Layout L,
+                                                                     const double* __restrict__ q0,
+                                                                     const double* __restrict__ v0) {
   IDOCP_DYN_SMEM(double, smem);
   double* tile = smem + (threadIdx.x >> 3) * (OCT * PAIR_TILE);
   const StageTask t = stage_task(L, ((RESIDUAL_ONLY || TASK) && !BACKWARD_EULER) ? L.N + 1 : L.N);
@@ -633,10 +625,8 @@ __global__ void k_step_min(Layout L, const double* __restrict__ primal_override)
 }
 
 constexpr int UL_D = X_NUM, UL_XN = UL_D + D_NUM, UL_DN = UL_XN + 4, UL_ST = UL_DN + 4, UL_SLOTS = UL_ST + 1;
-#ifndef IDOCP_UL_WARPS
-#define IDOCP_UL_WARPS 4   // warps per CTA of the persistent kernel (24.3 KB of shared memory each)
-#endif
-constexpr int UL_WARPS = IDOCP_UL_WARPS, UL_THREADS = 32 * UL_WARPS;
+constexpr int UL_WARPS = 4;   // warps per CTA of the persistent kernel (24.3 KB of shared memory each)
+constexpr int UL_THREADS = 32 * UL_WARPS;
 constexpr int UL_OFF_BUF = UL_WARPS * 4 * OCT * PAIR_TILE;                         // doubles, after the pair tiles
 constexpr int UL_OFF_BARS = UL_OFF_BUF + UL_WARPS * 2 * UL_SLOTS * SLOT;
 constexpr int UL_SMEM_DOUBLES = UL_OFF_BARS + 2 * UL_WARPS;
@@ -645,12 +635,7 @@ static_assert(X_LMD == 0 && X_GMM == 1 && X_Q == 2 && X_V == 3 && D_LMD == 0 && 
 static_assert((UL_OFF_BUF * 8) % 16 == 0, "TMA destinations are 16-byte aligned");
 
 template <bool TASK, bool KKT = false>
-#ifdef IDOCP_UL_MAXREG   // register cap given directly (ptxas derives the cap of minBlocks for CTAs of 128 threads)
-#define IDOCP_UL_BOUNDS __maxnreg__(IDOCP_UL_MAXREG)
-#else
-#define IDOCP_UL_BOUNDS __launch_bounds__(UL_THREADS, IDOCP_UL_CTAS_PER_SM)
-#endif
-__global__ void IDOCP_UL_BOUNDS k_update_linearize(const DevProblem* __restrict__ Pp, Layout L) {
+__global__ void __launch_bounds__(UL_THREADS, UL_CTAS_PER_SM) k_update_linearize(const DevProblem* __restrict__ Pp, Layout L) {
   IDOCP_DYN_SMEM(double, smem);
   const int warp = threadIdx.x >> 5, wl = threadIdx.x & 31;
   double* tile = smem + (threadIdx.x >> 3) * (OCT * PAIR_TILE);
@@ -717,10 +702,7 @@ constexpr int RIC_WARP_SLOTS = (RIC_RING * RIC_RING_SLOTS > RIC_BUFA_SLOTS + RIC
 // The sweep is a serial chain per warp, so its duration is (rounds of resident warps) x (one chain): 16384 instances = 4096
 // warps need 4 rounds at 8 warps / SM (3.46 waves) but 3 at 10.  Measured (profiles/r2n_variants.txt): 10 warps / SM caps the
 // kernel at 168 registers (three warps on one scheduler partition) with 600-800 B of spills: 0.423 -> 0.564 ms.  Kept at 4.
-#ifndef IDOCP_RIC_WARPS
-#define IDOCP_RIC_WARPS 4
-#endif
-constexpr int RIC_WARPS = IDOCP_RIC_WARPS;
+constexpr int RIC_WARPS = 4;
 constexpr int RIC_THREADS = 32 * RIC_WARPS;
 constexpr int RIC_OFF_STREAM = 4 * RIC_WARPS * RIC_SMEM_PER_OCT;                      // doubles
 constexpr int RIC_OFF_BARS = RIC_OFF_STREAM + RIC_WARPS * RIC_WARP_SLOTS * SLOT;
@@ -731,9 +713,9 @@ static_assert(W_KQ == 0 && W_KV == NV && W_K == 2 * NV && KQ_FV == KQ_FQ + 1, "r
 
 // TASK = true: the terminal Hessian / gradient are dense and come from record N of KQ (k_linearize<.., true>)
 template <bool TASK>
-__global__ void __launch_bounds__(RIC_THREADS, IDOCP_RIC_MINB) k_riccati(const DevProblem* __restrict__ Pp, Layout L,
-                                                         const double* __restrict__ q0,
-                                                         const double* __restrict__ v0) {
+__global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProblem* __restrict__ Pp, Layout L,
+                                                   const double* __restrict__ q0,
+                                                   const double* __restrict__ v0) {
   IDOCP_DYN_SMEM(double, smem);
   const DevProblem& P = *Pp;
   const int lane = lane_in_octet();
@@ -1018,9 +1000,6 @@ __global__ void __launch_bounds__(RIC_THREADS, IDOCP_RIC_MINB) k_riccati(const D
   if (wl == 0) {
     for (int i = 0; i < RIC_RING && i < N; ++i) issue_forward(i);
   }
-#ifdef IDOCP_RIC_SKIP_FWD   // timing experiment only: the backward sweep alone (results are wrong)
-  if (N > 0) return;
-#endif
   for (int i = 0; i < N; ++i) {
     const int e = i % RIC_RING;
     tma_bar_wait(&bars[2 + e], (i / RIC_RING) & 1);
@@ -1066,7 +1045,7 @@ __global__ void __launch_bounds__(RIC_THREADS, IDOCP_RIC_MINB) k_riccati(const D
 // TASK = true: the terminal P_N = Qqq_N is dense (record N of KQ)
 constexpr int EXP_TILE = 9;   // odd stride (doubles) of the Pqv transpose tile of k_expand
 template <bool PARNMPC, bool TASK, bool ACC = false>
-__global__ void __launch_bounds__(CTA_THREADS, IDOCP_EXP_MINB) k_expand(const DevProblem* __restrict__ Pp, Layout L, int stage_offset) {
+__global__ void __launch_bounds__(CTA_THREADS, EXP_MINB) k_expand(const DevProblem* __restrict__ Pp, Layout L, int stage_offset) {
   const DevProblem& P = *Pp;
   const int lane = lane_in_octet();
   const StageTask t = stage_task(L, PARNMPC ? L.N : L.N + 1);
@@ -1229,10 +1208,7 @@ __global__ void __launch_bounds__(CTA_THREADS, IDOCP_EXP_MINB) k_expand(const De
 // ---------------------------------------------------------------------------------------------
 // `nstages` = N + 1 with the terminal stage at index N (UnOCPSolver) or N without one (UnParNMPCSolver,
 // src/unocp/unparnmpc_solver.cpp:88-101).
-#ifndef IDOCP_UPD_MINB
-#define IDOCP_UPD_MINB 0
-#endif
-__global__ void __launch_bounds__(CTA_THREADS, IDOCP_UPD_MINB) k_update(const DevProblem* __restrict__ Pp, Layout L, int stage_offset,
+__global__ void __launch_bounds__(CTA_THREADS) k_update(const DevProblem* __restrict__ Pp, Layout L, int stage_offset,
                                                         const double* __restrict__ primal_override, int nstages) {
   const DevProblem& P = *Pp;
   const int lane = lane_in_octet();

@@ -154,29 +154,12 @@ __device__ __forceinline__ void warp_load_slots(const double* __restrict__ rec, 
   }
 }
 
-// y[r] += sum_k M[k * INV_LDX + r] x[k] for a 14 x 14 column-major M (broadcast operand), k ascending per element
-template <int K>
-__device__ __forceinline__ void inv_tl_fq(const double* M, const double (&x)[NX2], double (&y)[NX2]) {
-  if constexpr (K < NX2) {
-    inv_axpy<false, 0, NX2, K * INV_LDX, NX2>(M, x[K], y);
-    inv_tl_fq<K + 1>(M, x, y);
-  }
-}
-// col[r] -= sum_k TR[r * INV_LDX + k] st[k] for the 21 rows of this lane's column of BR
-template <int R>
-__device__ __forceinline__ void inv_br_rows(const double* TR, const double (&st)[NX2], double* col) {
-  if constexpr (R < NQ3) {
-    col[R] -= inv_dot<0, NX2, R * INV_LDX, NX2>(TR, st, 0.0);
-    inv_br_rows<R + 1>(TR, st, col);
-  }
-}
-
 // ---- the three dense products of the inversion on the FP64 tensor cores ----
 // mma.sync.aligned.m8n8k4.f64 is bit-identical to the ascending fma chain (tools/dmma_probe.cu, DESIGN.md section 5), so
 // C = A B by ONE warp in 8 x 16 strips (two tiles sharing the A fragment), accumulators chained over k from -0.0 (the first
 // fma is then the plain product), ragged edges zero-padded, equals the per-element chain of the oracle.  Operands in shared
 // memory with arbitrary strides; every element goes to `store(i, j, value)`.  Fragments: a = A[g][t], b = B[t][g],
-// c = C[g][2 t + {0, 1}], g = lane / 4, t = lane % 4.  (-DIDOCP_INV_SIMT keeps the SIMT form of the three products for A/B.)
+// c = C[g][2 t + {0, 1}], g = lane / 4, t = lane % 4.
 __device__ __forceinline__ void inv_dmma(double& d0, double& d1, double a, double b) {
 #ifndef IDOCP_B200_EMU
   asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};" : "+d"(d0), "+d"(d1) : "d"(a), "d"(b));
@@ -215,12 +198,10 @@ __device__ __forceinline__ void inv_mm_dmma(int lane, const double* __restrict__
   }
 }
 
-#ifndef IDOCP_INV_MINB
-#define IDOCP_INV_MINB 4   // 128 registers without spills (164 at three CTAs per SM), 14.3 KB of shared memory per warp
-#endif
+constexpr int INV_MINB = 4;   // 128 registers without spills (164 at three CTAs per SM), 14.3 KB of shared memory per warp
 
-__global__ void __launch_bounds__(CTA_THREADS, IDOCP_INV_MINB) k_parnmpc_invert(const DevProblem* __restrict__ Pp,
-                                                                                Layout L, ParNMPCLayout PL) {
+__global__ void __launch_bounds__(CTA_THREADS, INV_MINB) k_parnmpc_invert(const DevProblem* __restrict__ Pp,
+                                                                          Layout L, ParNMPCLayout PL) {
   IDOCP_DYN_SMEM(double, smem);
   const DevProblem& P = *Pp;
   const int wl = threadIdx.x & 31;           // lane in the warp
@@ -313,7 +294,6 @@ __global__ void __launch_bounds__(CTA_THREADS, IDOCP_INV_MINB) k_parnmpc_invert(
     }
   }
   __syncwarp();
-#ifndef IDOCP_INV_SIMT
   // ---- TR = -(TL FQinv) (14 x 21), ST = S TR (14 x 21, parked over the dead FQinv), BR = Qinv - TR^T ST (21 x 21, in place over
   //      the parked Qinv): three warp-level DMMA products, every element the oracle's ascending chain ----
   {
@@ -324,33 +304,6 @@ __global__ void __launch_bounds__(CTA_THREADS, IDOCP_INV_MINB) k_parnmpc_invert(
     __syncwarp();
     inv_mm_dmma<NQ3, NQ3, NX2>(wl, TR, INV_LDX, 1, ST, 1, INV_LDX, [=](int r, int c, double v) { A[c * INV_LDQ + r] -= v; });
   }
-#else
-  // ---- TR = -(TL FQinv) (14 x 21), lane c = column c (own column of FQinv re-read from shared memory) ----
-  {
-    double tr[NX2];
-    {
-      double fq[NX2];
-#pragma unroll
-      for (int k = 0; k < NX2; ++k) fq[k] = FQ[cq * INV_LDX + k];
-#pragma unroll
-      for (int r = 0; r < NX2; ++r) tr[r] = 0.0;
-      inv_tl_fq<0>(TL, fq, tr);          // tr[r] = sum_k TL(r, k) fq[k], ascending k
-#pragma unroll
-      for (int r = 0; r < NX2; ++r) tr[r] = -tr[r];
-    }
-    if (wl < NQ3) {
-#pragma unroll
-      for (int r = 0; r < NX2; ++r) TR[wl * INV_LDX + r] = tr[r];
-    }
-    __syncwarp();
-    // ---- BR = Qinv - TR^T (S TR) (21 x 21), in place over the parked Qinv ----
-    double st[NX2];
-#pragma unroll
-    for (int r = 0; r < NX2; ++r) st[r] = 0.0;
-    inv_tl_fq<0>(S, tr, st);             // st[r] = sum_k S(r, k) tr[k]
-    if (wl < NQ3) inv_br_rows<0>(TR, st, A + wl * INV_LDQ);
-  }
-#endif
   __syncwarp();
 
   // ---- d = KKT^-1 residual; s_new = s - d (lmd, gmm, a, q, v): lane = row, two passes (35 rows) ----
@@ -427,17 +380,15 @@ __device__ __forceinline__ void oct_matvec14(const double* __restrict__ M, doubl
 // ask the L2 for slots [first_slot, first_slot + nslots) of the (stage, group) record `rec` points into (this thread's
 // rec_ptr): the serial sweeps below would otherwise pay one DRAM round trip per stage.  No effect on results.
 __device__ __forceinline__ void warp_prefetch_slots(const double* rec, int first_slot, int nslots) {
-#if !defined(IDOCP_B200_EMU) && !defined(IDOCP_PARNMPC_NO_PREFETCH)
+#ifndef IDOCP_B200_EMU
   const int lane = threadIdx.x & 31;
   const char* c = reinterpret_cast<const char*>(rec - lane + first_slot * SLOT);
   for (int o = lane * 128; o < nslots * SLOT * static_cast<int>(sizeof(double)); o += 32 * 128)
     asm volatile("prefetch.global.L2 [%0];" ::"l"(c + o));
 #endif
 }
-#ifndef IDOCP_PARNMPC_PREFETCH_DISTANCE
-#define IDOCP_PARNMPC_PREFETCH_DISTANCE 2
-#endif
-constexpr int PARNMPC_PREFETCH_DISTANCE = IDOCP_PARNMPC_PREFETCH_DISTANCE;   // stages ahead of the one being corrected
+// stages ahead of the one being corrected; distances 4 and 8 measured slower (profiles/r2zs_variant_pf*.json)
+constexpr int PARNMPC_PREFETCH_DISTANCE = 2;
 
 // ---------------------------------------------------------------------------------------------
 // k_parnmpc_backward_serial: i = N-2 .. 0:  x_res = s_new[i+1].(lmd,gmm) - s[i+1].(lmd,gmm);

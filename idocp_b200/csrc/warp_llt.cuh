@@ -33,23 +33,6 @@ __device__ __forceinline__ void inv_axpy(const double* M, double x, double (&y)[
     }
   }
 }
-// t += sum_{k = K .. END-1} M[BASE + k] * x[k], ascending k (one chain)
-template <int K, int END, int BASE, int N>
-__device__ __forceinline__ double inv_dot(const double* M, const double (&x)[N], double t) {
-  if constexpr (K < END) {
-    if constexpr (((BASE + K) & 1) == 0 && K + 1 < END) {
-      const InvD2 v = inv_ld2(M + BASE + K);
-      t = fma(v.x, x[K], t);
-      t = fma(v.y, x[K + 1], t);
-      return inv_dot<K + 2, END, BASE, N>(M, x, t);
-    } else {
-      t = fma(M[BASE + K], x[K], t);
-      return inv_dot<K + 1, END, BASE, N>(M, x, t);
-    }
-  } else {
-    return t;
-  }
-}
 
 // Right-looking Cholesky of the lower triangle of the n x n matrix at A (column stride ld), in place; lane = row.
 // The lane keeps its row of the trailing matrix in registers.  Step k: the pivot comes from lane k by shuffle, every

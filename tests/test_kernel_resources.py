@@ -54,3 +54,31 @@ def test_kernels_documented_as_spill_free_have_no_spills():
         assert hits, frag
         for n, st, ld in hits:
             assert st == 0 and ld == 0, (n, st, ld)
+
+
+# the only macros a preprocessor conditional in idocp_b200/csrc may test, besides include guards: the SIMT-emulator build
+# and the storage class of the generated ANYmal tables
+ALLOWED_CONDITIONS = {"IDOCP_B200_EMU", "ANYMAL_TABLE"}
+
+
+def test_kernel_sources_compile_one_way():
+    """The launch bounds, prefetches and code paths the benchmarks measure are the only ones in the sources: no `-D` flag can
+    select another variant of a kernel.  Every #if / #ifdef / #ifndef / #elif tests IDOCP_B200_EMU or ANYMAL_TABLE, or is an
+    include guard (#ifndef X directly followed by a bare #define X)."""
+    import os
+    csrc = os.path.join(g.ROOT, "idocp_b200", "csrc")
+    bad = []
+    for f in sorted(os.listdir(csrc)):
+        lines = open(os.path.join(csrc, f)).read().splitlines()
+        for i, line in enumerate(lines):
+            m = re.match(r"\s*#\s*(if|ifdef|ifndef|elif)\b(.*)", line)
+            if not m:
+                continue
+            cond = re.sub(r"//.*|/\*.*?\*/", "", m.group(2))
+            names = set(re.findall(r"[A-Za-z_]\w*", cond)) - {"defined"}
+            nxt = next((l.strip() for l in lines[i + 1:] if l.strip()), "")
+            if m.group(1) == "ifndef" and len(names) == 1 and nxt == "#define " + next(iter(names)):
+                continue
+            if not names or not names <= ALLOWED_CONDITIONS:
+                bad.append("%s:%d: %s" % (f, i + 1, line.strip()))
+    assert not bad, "build switches in the kernel sources:\n" + "\n".join(bad)

@@ -31,10 +31,6 @@ fi
 if has running; then
   python bench.py --workload anymal_running --steps 10 --warmup 3 > gpurun_out/${L}_bench_anymal_running.json 2> gpurun_out/${L}_bench_anymal_running.err; cut -c 1-400 gpurun_out/${L}_bench_anymal_running.json
 fi
-if has phases; then
-  python tools/fb_phase_clocks.py > gpurun_out/${L}_fb_phase_clocks.json 2> gpurun_out/${L}_fb_phase_clocks.err; echo "phases rc=$?"
-  python tools/fb_phase_clocks.py simt > gpurun_out/${L}_fb_phase_clocks_simt.json 2> gpurun_out/${L}_fb_phase_clocks_simt.err; echo "phases simt rc=$?"
-fi
 if has dmma; then
   tools/dmma_probe > gpurun_out/${L}_dmma_probe.json 2> gpurun_out/${L}_dmma_probe.err; cat gpurun_out/${L}_dmma_probe.json
 fi
