@@ -132,6 +132,16 @@ struct DeviceHandle {
     *p = static_cast<T*>(q);
     return 0;
   }
+  // the line-search filter of n instances (line_search_filter.cuh)
+  int alloc_filter(LsFilter* F, size_t n) {
+    int rc = 0;
+    rc |= alloc(&F->alpha, n);
+    rc |= alloc(&F->state, n);
+    rc |= alloc(&F->n, n);
+    rc |= alloc(&F->cost, n * LS_FILTER_CAP);
+    rc |= alloc(&F->viol, n * LS_FILTER_CAP);
+    return rc;
+  }
 
   // device count and index checks, then the handle's non-blocking stream on `device`
   int open(int device) {
@@ -488,17 +498,25 @@ static int ensure_line_search(idocp_b200_solver* h) {
   int rc = 0;
   rc |= h->alloc(&h->LS.cost, (N + 1) * Bp);
   rc |= h->alloc(&h->LS.viol, N * Bp);
-  rc |= h->alloc(&h->LS.alpha, Bp);
-  rc |= h->alloc(&h->LS.state, Bp);
-  rc |= h->alloc(&h->LS.flt_n, Bp);
-  rc |= h->alloc(&h->LS.flt_cost, Bp * LS_FILTER_CAP);
-  rc |= h->alloc(&h->LS.flt_viol, Bp * LS_FILTER_CAP);
+  rc |= h->alloc_filter(&h->LS.f, Bp);
   if (rc != 0) return fail(IDOCP_B200_CUDA_ERROR, "line-search buffers: device memory allocation failed");
   h->ls_ready = true;
   return IDOCP_B200_OK;
 }
 
-// UnLineSearch::computeStepSize for the whole batch: lock-step rounds, no host synchronisation
+// The filter line search of both families for the whole batch, without host synchronisation: eval(mode) enqueues the
+// family's cost / violation kernel (mode 0: the current point, 1: the trial point), filter(mode) its filter round
+template <typename Eval, typename Filter>
+static void enqueue_line_search_rounds(Eval eval, Filter filter) {
+  eval(0);
+  filter(0);
+  for (int trial = 0; trial < LS_MAX_TRIALS; ++trial) {
+    eval(1);
+    filter(1);
+  }
+}
+
+// UnLineSearch::computeStepSize for the whole batch
 static int run_line_search(idocp_b200_solver* h, const double* d_q, const double* d_v) {
   const int rc = ensure_line_search(h);
   if (rc != IDOCP_B200_OK) return rc;
@@ -522,12 +540,9 @@ static int run_line_search(idocp_b200_solver* h, const double* d_q, const double
         IDOCP_LAUNCH(h, KC_LINESEARCH, (k_ls_eval<false, false>), grid, CTA_THREADS, 0, h->d_prob, h->L, h->LS, mode, off, d_q, d_v);
     }
   };
-  eval(0);
-  IDOCP_LAUNCH(h, KC_LINESEARCH, k_ls_filter, fgrid, 128, 0, h->L, h->LS, 0, ncost);
-  for (int trial = 0; trial < LS_MAX_TRIALS; ++trial) {
-    eval(1);
-    IDOCP_LAUNCH(h, KC_LINESEARCH, k_ls_filter, fgrid, 128, 0, h->L, h->LS, 1, ncost);
-  }
+  enqueue_line_search_rounds(eval, [&](int mode) {
+    IDOCP_LAUNCH(h, KC_LINESEARCH, k_ls_filter, fgrid, 128, 0, h->L, h->LS, mode, ncost);
+  });
   CUDA_OK(cudaGetLastError());
   return IDOCP_B200_OK;
 }
@@ -568,7 +583,7 @@ static int unocp_update(idocp_b200_solver* h, const double* d_q, const double* d
   if (line_search) {
     const int rc = run_line_search(h, d_q, d_v);
     if (rc != IDOCP_B200_OK) return rc;
-    override_alpha = h->LS.alpha;
+    override_alpha = h->LS.f.alpha;
   }
   if (h->pipelined) {
     // step sizes, then update + linearisation of the new iterate in one persistent launch; X (old) -> X2 (new), then the
@@ -613,7 +628,7 @@ static int parnmpc_update(idocp_b200_solver* h, double, const double* d_q, const
   if (line_search) {
     const int rc = run_line_search(h, d_q, d_v);
     if (rc != IDOCP_B200_OK) return rc;
-    override_alpha = h->LS.alpha;
+    override_alpha = h->LS.f.alpha;
   }
   IDOCP_LAUNCH(h, KC_UPDATE, k_update, stage_grid(h, N), CTA_THREADS, 0, h->d_prob, h->L, 1, override_alpha, N);
   CUDA_OK(cudaGetLastError());
@@ -916,7 +931,7 @@ extern "C" int idocp_b200_clear_line_search_filter(idocp_b200_solver* h) {
   if (!h) return fail(IDOCP_B200_INVALID_ARGUMENT, "null handle");
   if (!h->ls_ready) return IDOCP_B200_OK;  // never used: already empty
   CUDA_OK(cudaSetDevice(h->device));
-  IDOCP_LAUNCH(h, KC_LINESEARCH, k_ls_clear, (h->B + 127) / 128, 128, 0, h->LS, h->B);
+  IDOCP_LAUNCH(h, KC_LINESEARCH, k_ls_clear, (h->B + 127) / 128, 128, 0, h->LS.f.n, h->B);
   CUDA_OK(cudaGetLastError());
   return IDOCP_B200_OK;
 }

@@ -18,6 +18,7 @@
 #pragma once
 #include "fb_math.cuh"
 #include "warp_llt.cuh"
+#include "line_search_filter.cuh"
 
 namespace idocp_b200 {
 
@@ -108,15 +109,9 @@ struct FbArrays {
   const double* v0;   // [B][18]
   double* steps;      // [B][2]
   double* kkt_err;    // [B]
-  // filter line search (line_search_kernels.cuh has the fixed-base twin)
-  double* ls_alpha;   // [B] current / final primal step size
-  int* ls_state;      // [B] 0 searching, 1 finished
-  int* ls_n;          // [B] filter sizes
-  double* ls_fcost;   // [B][FB_LS_FILTER_CAP]
-  double* ls_fviol;   // [B][FB_LS_FILTER_CAP]
-  int* ls_status;     // [B] bit 2: filter capacity exceeded
+  LsFilter ls;        // filter line search of B instances (line_search_filter.cuh)
+  int* ls_status;     // [B] IDOCP_B200_STATUS_FILTER_FULL
 };
-#define FB_LS_FILTER_CAP 256
 
 #define FB_FOR(i, n) for (int i = threadIdx.x; i < (n); i += blockDim.x)
 enum { FBM_SET = 0, FBM_ADD = 1, FBM_SUB = 2 };
@@ -2472,10 +2467,9 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS) k_fb_init_distance(FbArra
 }
 
 // =====================================================================================================
-// LineSearch for OCPSolver (line_search/line_search.hpp:62-158, src/line_search/line_search.cpp:64-197,
-// line_search_filter.cpp:34-65): every instance carries its own (alpha, state, filter); the host launches lock-step
-// rounds  k_fb_ls_eval (warp per (instance, stage): stage cost and constraint violation of the trial point
-// s + alpha d)  ->  k_fb_ls_filter (thread per instance); finished instances drop out.
+// LineSearch for OCPSolver (line_search/line_search.hpp:62-158, src/line_search/line_search.cpp:64-197): the lock-step
+// rounds of line_search_filter.cuh  k_fb_ls_eval (warp per (instance, stage): stage cost and constraint violation of
+// the trial point s + alpha d)  ->  k_fb_ls_filter (thread per instance); finished instances drop out.
 // =====================================================================================================
 template <bool INITIAL>
 __global__ void __launch_bounds__(32 * FB_LS_WARPS) k_fb_ls_eval(FbArrays A, FbLin* lin) {
@@ -2485,8 +2479,8 @@ __global__ void __launch_bounds__(32 * FB_LS_WARPS) k_fb_ls_eval(FbArrays A, FbL
   if (stage >= A.B * A.n_elems) return;
   FbLsWork& w = wbase[warp];
   const int b = stage / A.n_elems, e = stage - b * A.n_elems;
-  if (INITIAL) { if (A.ls_n[b] != 0) return; } else { if (A.ls_state[b] != 0) return; }
-  const double alpha = INITIAL ? 0.0 : A.ls_alpha[b];
+  if (INITIAL) { if (A.ls.n[b] != 0) return; } else { if (A.ls.state[b] != 0) return; }
+  const double alpha = INITIAL ? 0.0 : A.ls.alpha[b];
   const FbElem& el = A.elems[e];
   const FbDevProblem& pr = *A.prob;
   const int nl = fbc_cone_bits(pr);
@@ -2733,70 +2727,15 @@ __device__ inline void fb_ls_totals(const FbArrays& A, int b, double& cost, doub
   cost = c;
   viol = v;
 }
-__device__ inline void fb_filter_augment(const FbArrays& A, int b, double cost, double viol) {
-  double* fc = A.ls_fcost + (size_t)b * FB_LS_FILTER_CAP;
-  double* fv = A.ls_fviol + (size_t)b * FB_LS_FILTER_CAP;
-  int n = A.ls_n[b], w = 0;
-  for (int i = 0; i < n; ++i) {
-    if (cost <= fc[i] && viol <= fv[i]) continue;   // dominated entry erased
-    fc[w] = fc[i]; fv[w] = fv[i]; ++w;
-  }
-  if (w < FB_LS_FILTER_CAP) {
-    fc[w] = cost - 0.005 * viol;       // line_search_filter.hpp:16-17
-    fv[w] = (1 - 0.005) * viol;
-    ++w;
-  } else {
-    A.ls_status[b] |= 4;
-  }
-  A.ls_n[b] = w;
-}
-// mode 0: augment empty filters with the current point, start the search at the fraction-to-boundary step;
-// mode 1: one backtracking decision (alpha *= 0.75 while alpha > 0.05); mode 2: publish alpha as the primal step
+// mode 0 / 1: ls_filter_round from the fraction-to-boundary step; mode 2: publish alpha as the primal step
 __global__ void k_fb_ls_filter(FbArrays A, int mode) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= A.B) return;
-  if (mode == 0) {
-    if (A.ls_n[b] == 0) {
-      double cost, viol;
-      fb_ls_totals(A, b, cost, viol);
-      fb_filter_augment(A, b, cost, viol);
-    }
-    const double amax = A.steps[2 * b];
-    const bool go = amax > 0.05;
-    A.ls_alpha[b] = go ? amax : 0.05;
-    A.ls_state[b] = go ? 0 : 1;
-    return;
-  }
   if (mode == 2) {
-    A.steps[2 * b] = A.ls_alpha[b];
+    A.steps[2 * b] = A.ls.alpha[b];
     return;
   }
-  if (A.ls_state[b] != 0) return;
-  double cost, viol;
-  fb_ls_totals(A, b, cost, viol);
-  bool accepted = true;
-  {
-    const double* fc = A.ls_fcost + (size_t)b * FB_LS_FILTER_CAP;
-    const double* fv = A.ls_fviol + (size_t)b * FB_LS_FILTER_CAP;
-    for (int i = 0; i < A.ls_n[b]; ++i)
-      if (cost >= fc[i] && viol >= fv[i]) { accepted = false; break; }
-  }
-  if (accepted) {
-    fb_filter_augment(A, b, cost, viol);
-    A.ls_state[b] = 1;
-    return;
-  }
-  const double an = A.ls_alpha[b] * 0.75;
-  if (an > 0.05) {
-    A.ls_alpha[b] = an;
-  } else {
-    A.ls_alpha[b] = 0.05;
-    A.ls_state[b] = 1;
-  }
-}
-__global__ void k_fb_ls_clear(FbArrays A) {
-  const int b = blockIdx.x * blockDim.x + threadIdx.x;
-  if (b < A.B) A.ls_n[b] = 0;
+  ls_filter_round(A.ls, b, mode, A.steps[2 * b], A.ls_status, [&](double& cost, double& viol) { fb_ls_totals(A, b, cost, viol); });
 }
 
 }  // namespace idocp_b200

@@ -1,36 +1,22 @@
 // line_search_kernels.cuh -- batched filter line search of the unconstrained solvers.
 //
-//   UnLineSearch::computeStepSize        include/idocp/line_search/unline_search.hpp:62-91
 //   UnLineSearch::computeCostAndViolation  src/line_search/unline_search.cpp:56-84
 //   SplitUnOCP::stageCost / constraintViolation  include/idocp/unocp/split_unocp.hxx:177-217
 //   TerminalOCP::terminalCost            include/idocp/ocp/terminal_ocp.hxx:89-95
-//   LineSearchFilter::isAccepted/augment  src/line_search/line_search_filter.cpp:34-65
 //
-// The reference backtracks one instance with a data-dependent trip count (alpha *= 0.75 while
-// alpha > 0.05, at most 11 trials from alpha = 1).  Here every instance of the batch carries its own
-// (alpha, state, filter); the host launches a fixed number of lock-step rounds
+// The lock-step rounds of line_search_filter.cuh:
 //   k_ls_eval (stage-parallel cost / violation of the trial step)  ->  k_ls_filter (per instance)
-// and finished instances drop out warp-uniformly.  Sums run over ascending stage index.
+// Finished instances drop out warp-uniformly.  Sums run over ascending stage index.
 #pragma once
 #include "unocp_kernels.cuh"
+#include "line_search_filter.cuh"
 
 namespace idocp_b200 {
-
-constexpr int LS_FILTER_CAP = 256;     // entries per instance (the reference's vector is unbounded)
-constexpr int LS_MAX_TRIALS = 11;      // 0.75^10 > 0.05 >= 0.75^11
-constexpr double LS_RATE = 0.75;       // unline_search.hpp:25
-constexpr double LS_MIN_STEP = 0.05;   // unline_search.hpp:26
-constexpr double LS_COST_REDUCTION = 0.005;        // line_search_filter.hpp:16
-constexpr double LS_CONSTRAINTS_REDUCTION = 0.005; // line_search_filter.hpp:17
 
 struct LineSearchLayout {
   double* cost = nullptr;      // [N+1][Bp] per-stage cost of the current trial
   double* viol = nullptr;      // [N][Bp]   per-stage constraint violation
-  double* alpha = nullptr;     // [Bp] current / final primal step size
-  int* state = nullptr;        // [Bp] 0 = searching, 1 = finished
-  int* flt_n = nullptr;        // [Bp] filter sizes
-  double* flt_cost = nullptr;  // [Bp][LS_FILTER_CAP]
-  double* flt_viol = nullptr;  // [Bp][LS_FILTER_CAP]
+  LsFilter f;                  // Bp instances
 };
 
 // min over stages of the per-stage fraction-to-boundary minima (unocp_solver.cpp:114-115);
@@ -45,38 +31,10 @@ __device__ __forceinline__ void octet_step_sizes(const Layout& L, int b, int lan
   ad = oct_min(ad);
 }
 
-// LineSearchFilter::augment (line_search_filter.cpp:48-65)
-__device__ __forceinline__ void filter_augment(const LineSearchLayout& LS, int b, double cost, double viol, int* status) {
-  double* fc = LS.flt_cost + static_cast<size_t>(b) * LS_FILTER_CAP;
-  double* fv = LS.flt_viol + static_cast<size_t>(b) * LS_FILTER_CAP;
-  int n = LS.flt_n[b], w = 0;
-  for (int i = 0; i < n; ++i) {
-    if (cost <= fc[i] && viol <= fv[i]) continue;  // dominated entry erased
-    fc[w] = fc[i]; fv[w] = fv[i]; ++w;
-  }
-  if (w < LS_FILTER_CAP) {
-    fc[w] = cost - LS_COST_REDUCTION * viol;
-    fv[w] = (1 - LS_CONSTRAINTS_REDUCTION) * viol;
-    ++w;
-  } else {
-    status[b] |= 4;  // filter capacity exceeded: entry dropped
-  }
-  LS.flt_n[b] = w;
-}
-// LineSearchFilter::isAccepted (:34-45)
-__device__ __forceinline__ bool filter_accepts(const LineSearchLayout& LS, int b, double cost, double viol) {
-  const double* fc = LS.flt_cost + static_cast<size_t>(b) * LS_FILTER_CAP;
-  const double* fv = LS.flt_viol + static_cast<size_t>(b) * LS_FILTER_CAP;
-  const int n = LS.flt_n[b];
-  for (int i = 0; i < n; ++i)
-    if (cost >= fc[i] && viol >= fv[i]) return false;
-  return true;
-}
-
 // does instance b take part in this round?  mode 0: filter initialisation (empty filters only)
 __device__ __forceinline__ bool ls_participates(const LineSearchLayout& LS, int b, int B, int mode) {
   if (b >= B) return false;
-  return mode == 0 ? (LS.flt_n[b] == 0) : (LS.state[b] == 0);
+  return mode == 0 ? (LS.f.n[b] == 0) : (LS.f.state[b] == 0);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -102,7 +60,7 @@ __global__ void __launch_bounds__(CTA_THREADS) k_ls_eval(const DevProblem* __res
   const double dt = P.dt;
   const bool act = lane < NV;
   const double z = act ? 1.0 : 0.0;
-  const double alpha = (mode == 0 || !part) ? 0.0 : LS.alpha[b];
+  const double alpha = (mode == 0 || !part) ? 0.0 : LS.f.alpha[b];
   const double* X = rec_ptr(L.X, X_NUM, L.G, i, t.g);
   const double* D = rec_ptr(L.D, D_NUM, L.G, i, t.g);
   const double q = X[X_Q * SLOT], v = X[X_V * SLOT];
@@ -228,41 +186,12 @@ __device__ __forceinline__ void ls_totals(const Layout& L, const LineSearchLayou
   cost = cs; viol = vs;
 }
 
-// ---------------------------------------------------------------------------------------------
-// k_ls_filter: one thread per instance.
-//  mode 0: augment empty filters with the current point, then start the search at alpha_max
-//  mode 1: one backtracking decision
-// ---------------------------------------------------------------------------------------------
+// k_ls_filter: one thread per instance, ls_filter_round from the fraction-to-boundary step alpha_max
 __global__ void k_ls_filter(Layout L, LineSearchLayout LS, int mode, int ncost) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= L.B) return;
-  if (mode == 0) {
-    if (LS.flt_n[b] == 0) {
-      double cost, viol;
-      ls_totals(L, LS, b, ncost, cost, viol);
-      filter_augment(LS, b, cost, viol, L.status);
-    }
-    const double amax = L.steps[2 * L.Bp + b];
-    const bool go = amax > LS_MIN_STEP;
-    LS.alpha[b] = go ? amax : LS_MIN_STEP;
-    LS.state[b] = go ? 0 : 1;
-    return;
-  }
-  if (LS.state[b] != 0) return;
-  double cost, viol;
-  ls_totals(L, LS, b, ncost, cost, viol);
-  if (filter_accepts(LS, b, cost, viol)) {
-    filter_augment(LS, b, cost, viol, L.status);
-    LS.state[b] = 1;
-    return;
-  }
-  const double an = LS.alpha[b] * LS_RATE;
-  if (an > LS_MIN_STEP) {
-    LS.alpha[b] = an;
-  } else {
-    LS.alpha[b] = LS_MIN_STEP;
-    LS.state[b] = 1;
-  }
+  ls_filter_round(LS.f, b, mode, L.steps[2 * L.Bp + b], L.status,
+                  [&](double& cost, double& viol) { ls_totals(L, LS, b, ncost, cost, viol); });
 }
 
 // max step sizes before the line search (stored for k_ls_filter mode 0): steps[2][b] = alpha_max
@@ -274,11 +203,6 @@ __global__ void __launch_bounds__(CTA_THREADS) k_ls_begin(Layout L) {
   double ap, ad;
   octet_step_sizes(L, b, lane, ap, ad);
   if (lane == 0) L.steps[2 * L.Bp + b] = ap;
-}
-
-__global__ void k_ls_clear(LineSearchLayout LS, int B) {
-  const int b = blockIdx.x * blockDim.x + threadIdx.x;
-  if (b < B) LS.flt_n[b] = 0;
 }
 
 }  // namespace idocp_b200

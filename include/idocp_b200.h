@@ -39,6 +39,7 @@ typedef enum {
  * Debug builds (split_unriccati_factorizer.hxx:38,41-42) */
 #define IDOCP_B200_STATUS_CHOL_FAIL 1  /* a Cholesky pivot was <= 0 or NaN */
 #define IDOCP_B200_STATUS_NAN       2  /* a step size / KKT error was NaN */
+#define IDOCP_B200_STATUS_FILTER_FULL 4  /* the line-search filter held its 256 entries: a new entry was dropped */
 
 typedef enum {
   IDOCP_B200_ROBOT_IIWA14 = 0
