@@ -685,11 +685,21 @@ __global__ void __launch_bounds__(UL_THREADS, UL_CTAS_PER_SM) k_update_linearize
 // one group of 4 instances); lane c owns column c.  Writes the gains / Riccati matrices to W and
 // (dq, dv, da) to D; everything else of the direction is expanded in parallel by k_expand.
 // ---------------------------------------------------------------------------------------------
+// Three [8][RIC_TILE] tiles per octet carry a stage's cross-lane traffic (tX[col * RIC_TILE + row]).  Rows 0..7 are
+// shared through __syncwarp; rows 8..14 of a lane's own column hold values only that lane reads.
+//   tA: Qaa | la (rows 0..7), shared for the Cholesky; the lane's Qaq column (rows RIC_STASH..) until the solve and s.
+//   tB: K (Kq rows 0..6, Kv rows 7..13) from the solve to the P update; then the new Pqq (rows 0..6) and Pvv (rows
+//       RIC_STASH..) for their symmetrisation.  tA is therefore free when the next stage writes Qaa.
+//   tC: the stage's Pqv (rows 0..6), read transposed as Pvq = Pqv^T through the whole next stage; the lane's Qav
+//       column (rows RIC_STASH..), as Qaq in tA.
+// Parking Qaq / Qav there keeps them out of registers across the Cholesky, which is what leaves the sweep spill-free.
 constexpr int RIC_TILE = 17;               // odd stride (doubles) -> conflict-free transposed reads
-constexpr int RIC_SMEM_PER_OCT = 2 * OCT * RIC_TILE;
+constexpr int RIC_STASH = OCT;
+constexpr int RIC_SMEM_PER_OCT = 3 * OCT * RIC_TILE;
+static_assert(RIC_STASH + NV <= RIC_TILE && 2 * NV <= RIC_TILE, "tile rows");
 // The condensed KKT record of (stage, group) is streamed into shared memory by the TMA engine one
 // stage ahead of its use, in two halves with separate barriers so that each half-buffer can be
-// re-armed as soon as its values sit in registers:
+// re-armed at the first warp sync after every lane has read it:
 //   half A = a-blocks + residual (slots AA, AQ, AV | FQ..LV: 21 + 5 slots), half X = x-blocks (QQ, QV, VV)
 // The forward recursion streams (rows of K, k | Fq, Fv) of the stages through a 3-deep ring in the
 // same per-warp region: its body is ~100 instructions per stage, i.e. pure memory latency otherwise.
@@ -708,6 +718,8 @@ constexpr int RIC_OFF_STREAM = 4 * RIC_WARPS * RIC_SMEM_PER_OCT;                
 constexpr int RIC_OFF_BARS = RIC_OFF_STREAM + RIC_WARPS * RIC_WARP_SLOTS * SLOT;
 constexpr int RIC_NBARS = 2 + RIC_RING;
 constexpr int RIC_SMEM_DOUBLES = RIC_OFF_BARS + RIC_NBARS * RIC_WARPS;
+// RIC_MINB CTAs per SM, each with its 1 KB of shared memory reserved by the system, within the SM's 228 KB
+static_assert(RIC_MINB * (RIC_SMEM_DOUBLES * 8 + 1024) <= 228 * 1024, "k_riccati shared memory");
 static_assert(KQ_AA == 0 && KQ_QQ == 3 * NV && KQ_FQ == 6 * NV && KQ_NUM == 6 * NV + 5, "record layout");
 static_assert(W_KQ == 0 && W_KV == NV && W_K == 2 * NV && KQ_FV == KQ_FQ + 1, "record layout");
 
@@ -722,6 +734,7 @@ __global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProb
   const int oct = threadIdx.x >> 3;
   double* tA = smem + oct * RIC_SMEM_PER_OCT;         // [8][RIC_TILE]
   double* tB = tA + OCT * RIC_TILE;                   // [8][RIC_TILE]
+  double* tC = tB + OCT * RIC_TILE;                   // [8][RIC_TILE]
   int g = blockIdx.x * RIC_WARPS + (threadIdx.x >> 5);
   if (g >= L.G) g = L.G - 1;     // tail warps redo the last group (identical, idempotent stores)
   const int b = g * 4 + (oct & 3);
@@ -735,21 +748,23 @@ __global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProb
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + RIC_OFF_BARS) + RIC_NBARS * warp;
   const double* kq_rec = L.KQ + static_cast<size_t>(g) * (KQ_NUM * SLOT);   // + stage * kstride
   const double* w_rec = L.W + static_cast<size_t>(g) * (W_NUM * SLOT);
+  const size_t kstride = static_cast<size_t>(L.G) * (KQ_NUM * SLOT);
   if (wl == 0) {
 #pragma unroll
     for (int k = 0; k < RIC_NBARS; ++k) tma_bar_init(&bars[k], 1);
   }
   __syncwarp();
-  auto issue_half_a = [&](int stage) {
-    const double* src = kq_rec + static_cast<size_t>(stage) * L.G * (KQ_NUM * SLOT);
-    tma_bar_expect(&bars[0], RIC_BUFA_SLOTS * SLOT * 8);
-    tma_load_1d(stream, src + KQ_AA * SLOT, 3 * NV * SLOT * 8, &bars[0]);
-    tma_load_1d(stream + 3 * NV * SLOT, src + KQ_FQ * SLOT, 5 * SLOT * 8, &bars[0]);
+  // the backward sweep re-issues into the same two buffers every stage: their shared addresses are converted once
+  const smem_t s_bufa = smem_addr(stream), s_bufx = smem_addr(stream + RIC_BUFA_SLOTS * SLOT);
+  const smem_t s_bara = smem_addr(&bars[0]), s_barx = smem_addr(&bars[1]);
+  auto issue_half_a = [&](const double* src) {   // src: the stage's KQ record
+    tma_bar_expect(s_bara, RIC_BUFA_SLOTS * SLOT * 8);
+    tma_load_1d(s_bufa, src + KQ_AA * SLOT, 3 * NV * SLOT * 8, s_bara);
+    tma_load_1d(s_bufa + 3 * NV * SLOT * 8, src + KQ_FQ * SLOT, 5 * SLOT * 8, s_bara);
   };
-  auto issue_half_x = [&](int stage) {
-    const double* src = kq_rec + static_cast<size_t>(stage) * L.G * (KQ_NUM * SLOT);
-    tma_bar_expect(&bars[1], RIC_BUFX_SLOTS * SLOT * 8);
-    tma_load_1d(stream + RIC_BUFA_SLOTS * SLOT, src + KQ_QQ * SLOT, RIC_BUFX_SLOTS * SLOT * 8, &bars[1]);
+  auto issue_half_x = [&](const double* src) {
+    tma_bar_expect(s_barx, RIC_BUFX_SLOTS * SLOT * 8);
+    tma_load_1d(s_bufx, src + KQ_QQ * SLOT, RIC_BUFX_SLOTS * SLOT * 8, s_barx);
   };
   auto issue_forward = [&](int stage) {   // ring entry stage % RIC_RING
     const int e = stage % RIC_RING;
@@ -760,9 +775,10 @@ __global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProb
     tma_load_1d(dst + (2 * NV + 1) * SLOT, kq_rec + static_cast<size_t>(stage) * L.G * (KQ_NUM * SLOT) + KQ_FQ * SLOT,
                 2 * SLOT * 8, &bars[2 + e]);
   };
+  const double* kq_stage = kq_rec + static_cast<size_t>(N - 1) * kstride;   // record of the current stage
   if (wl == 0) {
-    issue_half_a(N - 1);
-    issue_half_x(N - 1);
+    issue_half_a(kq_stage);
+    issue_half_x(kq_stage);
   }
   uint32_t phase = 0;
   const double dt = P.dt;
@@ -775,7 +791,7 @@ __global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProb
   const size_t dstride = static_cast<size_t>(L.G) * (D_NUM * SLOT);
 
   // ---- terminal stage: P_N = diag(qf, vf), s_N = -l_N (unriccati_recursion.cpp:39-47) ----
-  double Pqq[NV], Pqv[NV], Pvq[NV], Pvv[NV], sq, sv;
+  double Pqq[NV], Pqv[NV], Pvv[NV], sq, sv;   // Pvq = Pqv^T is read from tile C
   {
     const double* X = rec_ptr(L.X, X_NUM, L.G, N, g);
     const double q = X[X_Q * SLOT], v = X[X_V * SLOT], lmd = X[X_LMD * SLOT], gmm = X[X_GMM * SLOT];
@@ -791,7 +807,7 @@ __global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProb
       Pqq[r] = (r == lane) ? P.qf_weight[lane] : 0.0;
       Pvv[r] = (r == lane) ? P.vf_weight[lane] : 0.0;
       Pqv[r] = 0.0;
-      Pvq[r] = 0.0;
+      tC[lane * RIC_TILE + r] = 0.0;
     }
     if (TASK) {
       const double* KQN = rec_ptr(L.KQ, KQ_NUM, L.G, N, g);
@@ -799,43 +815,39 @@ __global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProb
       for (int r = 0; r < NV; ++r) Pqq[r] = KQN[(KQ_QQ + r) * SLOT];
       sq = -KQN[KQ_LQ * SLOT];
     }
+    __syncwarp();
   }
 
   // ---- backward recursion ----
   double* W = rec_ptr(L.W, W_NUM, L.G, N - 1, g);
-  for (int i = N - 1; i >= 0; --i, W -= wstride, phase ^= 1) {
-    double Qaa[NV], Qaq[NV], Qav[NV];
+  for (int i = N - 1; i >= 0; --i, W -= wstride, kq_stage -= kstride, phase ^= 1) {
     tma_bar_wait(&bars[0], phase);
+    // factorizeKKTMatrix, a-blocks (backward_unriccati_recursion_factorizer.hxx:44-53); the
+    // x-blocks are folded into the P update below (same operation order per entry)
+    double Qaa[NV];
 #pragma unroll
     for (int r = 0; r < NV; ++r) {
-      Qaa[r] = bufA[(KQ_AA + r) * SLOT];
-      Qaq[r] = bufA[(KQ_AQ + r) * SLOT];
-      Qav[r] = bufA[(KQ_AV + r) * SLOT];
+      const double pvq = tC[r * RIC_TILE + ln];
+      double qaq = bufA[(KQ_AQ + r) * SLOT], qav = bufA[(KQ_AV + r) * SLOT];
+      qaq = fma(dt, pvq, qaq);
+      qav = fma(dt2, pvq, qav);
+      qav = fma(dt, Pvv[r], qav);
+      Qaa[r] = fma(dt2, Pvv[r], bufA[(KQ_AA + r) * SLOT]);
+      tA[lane * RIC_TILE + RIC_STASH + r] = qaq;
+      tC[lane * RIC_TILE + RIC_STASH + r] = qav;
     }
     const double Fq = bufA[(3 * NV + 0) * SLOT], Fv = bufA[(3 * NV + 1) * SLOT];
     double la = bufA[(3 * NV + 2) * SLOT];
     const double lq = bufA[(3 * NV + 3) * SLOT], lv = bufA[(3 * NV + 4) * SLOT];
-    __syncwarp();                              // half A is in registers: stream the next stage into it
-    if (wl == 0 && i > 0) issue_half_a(i - 1);
-
-    // factorizeKKTMatrix, a-blocks (backward_unriccati_recursion_factorizer.hxx:44-53); the
-    // x-blocks are folded into the P update below (same operation order per entry)
-#pragma unroll
-    for (int r = 0; r < NV; ++r) {
-      Qaq[r] = fma(dt, Pvq[r], Qaq[r]);
-      Qav[r] = fma(dt2, Pvq[r], Qav[r]);
-      Qav[r] = fma(dt, Pvv[r], Qav[r]);
-      Qaa[r] = fma(dt2, Pvv[r], Qaa[r]);
-    }
     // products of the OLD P with Fx (used by la and by the s recursion)
     double pqqF = 0.0, pvqF = 0.0, pqvF = 0.0, pvvF = 0.0;
 #pragma unroll
     for (int k = 0; k < NV; ++k) {
       const double fq = oct_bcast(Fq, k), fv = oct_bcast(Fv, k);
-      pqqF = fma(Pqq[k], fq, pqqF);   // (Pqq Fq)_c   (row c = column c, symmetric)
-      pvqF = fma(Pvq[k], fv, pvqF);   // (Pqv Fv)_c
-      pqvF = fma(Pqv[k], fq, pqvF);   // (Pqv^T Fq)_c
-      pvvF = fma(Pvv[k], fv, pvvF);   // (Pvv Fv)_c
+      pqqF = fma(Pqq[k], fq, pqqF);                  // (Pqq Fq)_c   (row c = column c, symmetric)
+      pvqF = fma(tC[k * RIC_TILE + ln], fv, pvqF);   // (Pqv Fv)_c
+      pqvF = fma(Pqv[k], fq, pqvF);                  // (Pqv^T Fq)_c
+      pvvF = fma(Pvv[k], fv, pvvF);                  // (Pvv Fv)_c
     }
     if (TASK && i == N - 1) {
       // the dense terminal Pqq_N = Qqq_N (Gauss-Newton term of the task-space cost) is not bitwise symmetric:
@@ -848,11 +860,18 @@ __global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProb
     la = fma(dt, pqvF, la);
     la = fma(dt, pvvF, la);
     la = fma(-dt, sv, la);
+    // next s (uses the OLD P): backward_unriccati_recursion_factorizer.hxx:78-88, all but the Qa^T k terms, which
+    // are subtracted once k is known: two values instead of eight stay live across the Cholesky
+    double nsq = sq, nsv;
+    nsq -= pqqF; nsq -= pvqF;
+    nsv = fma(dt, nsq, sv); nsv -= pqvF; nsv -= pvvF;
+    nsq -= lq; nsv -= lv;
     // share Qaa (tile A: tA[col][row]) and la
 #pragma unroll
     for (int r = 0; r < NV; ++r) tA[lane * RIC_TILE + r] = Qaa[r];
     tA[lane * RIC_TILE + NV] = la;
-    __syncwarp();
+    __syncwarp();                              // tile A shared, half A consumed by every lane
+    if (wl == 0 && i > 0) issue_half_a(kq_stage - kstride);
     // Cholesky of Qaa (lower triangle), redundantly in every lane: Lm[col][row], row >= col
     double Lm[NV][NV];
     double rdiag[NV];
@@ -875,7 +894,7 @@ __global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProb
     double Kq[NV], Kv[NV], kk[NV];
 #pragma unroll
     for (int r = 0; r < NV; ++r) {
-      double y1 = Qaq[r], y2 = Qav[r], y3 = tA[r * RIC_TILE + NV];
+      double y1 = tA[lane * RIC_TILE + RIC_STASH + r], y2 = tC[lane * RIC_TILE + RIC_STASH + r], y3 = tA[r * RIC_TILE + NV];
 #pragma unroll
       for (int j = 0; j < r; ++j) {
         y1 = fma(-Lm[j][r], Kq[j], y1); y2 = fma(-Lm[j][r], Kv[j], y2); y3 = fma(-Lm[j][r], kk[j], y3);
@@ -893,7 +912,9 @@ __global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProb
     }
 #pragma unroll
     for (int r = 0; r < NV; ++r) { Kq[r] = -Kq[r]; Kv[r] = -Kv[r]; kk[r] = -kk[r]; }
-    // GK = Qaa K (full Qaa, as the reference multiplies the full matrix)
+    // GK = Qaa K (full Qaa, as the reference multiplies the full matrix).  Qaa is read from tile A again: without the
+    // compiler barrier the Cholesky's 28 loads are reused here, which keeps them live across both solves and spills
+    asm volatile("" ::: "memory");
     double GKq[NV], GKv[NV];
 #pragma unroll
     for (int r = 0; r < NV; ++r) {
@@ -909,18 +930,17 @@ __global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProb
     // share K (tile B: tB[col][0..6] = Kq[:,col], tB[col][7..13] = Kv[:,col])
 #pragma unroll
     for (int r = 0; r < NV; ++r) { tB[lane * RIC_TILE + r] = Kq[r]; tB[lane * RIC_TILE + NV + r] = Kv[r]; }
-    __syncwarp();
-    // next s (uses the OLD P): backward_unriccati_recursion_factorizer.hxx:78-88
-    double nsq, nsv;
+    // rest of the next s
     {
-      nsq = sq; nsq -= pqqF; nsq -= pvqF;
-      nsv = fma(dt, nsq, sv); nsv -= pqvF; nsv -= pvvF;
-      nsq -= lq; nsv -= lv;
       double t5 = 0.0, t6 = 0.0;
 #pragma unroll
-      for (int k = 0; k < NV; ++k) { t5 = fma(Qaq[k], kk[k], t5); t6 = fma(Qav[k], kk[k], t6); }
+      for (int k = 0; k < NV; ++k) {
+        t5 = fma(tA[lane * RIC_TILE + RIC_STASH + k], kk[k], t5);
+        t6 = fma(tC[lane * RIC_TILE + RIC_STASH + k], kk[k], t6);
+      }
       nsq -= t5; nsv -= t6;
     }
+    __syncwarp();                              // tile B shared
     // F-blocks of factorizeKKTMatrix (:34-43) + P = Qxx - K^T (Qaa K) (:64-75), row by row
     tma_bar_wait(&bars[1], phase);
 #pragma unroll
@@ -933,7 +953,7 @@ __global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProb
       Qqv += Pqv[r];
       Qvv = fma(dt2, Pqq[r], Qvv);
       Qvv = fma(dt, Pqv[r], Qvv);
-      Qvv = fma(dt, Pvq[r], Qvv);
+      Qvv = fma(dt, tC[r * RIC_TILE + ln], Qvv);
       Qvv += Pvv[r];
       double tqq = 0.0, tqv = 0.0, tvv = 0.0;
 #pragma unroll
@@ -953,25 +973,25 @@ __global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProb
       W[(W_KQ + c) * SLOT] = tB[c * RIC_TILE + ln];
       W[(W_KV + c) * SLOT] = tB[c * RIC_TILE + NV + ln];
     }
-    W[W_K * SLOT] = kk[ln];
-    __syncwarp();                              // half X consumed by every lane (and tile B read)
-    if (wl == 0 && i > 0) issue_half_x(i - 1);
-    // transposes through the tiles: Pvq = Pqv^T, symmetrise Pqq and Pvv
+    double k_own = kk[0];                      // kk[ln] by selects: a lane-dependent index would put kk in local memory
 #pragma unroll
-    for (int r = 0; r < NV; ++r) { tA[lane * RIC_TILE + r] = Pqv[r]; tB[lane * RIC_TILE + r] = Pqq[r]; }
-    __syncwarp();
+    for (int r = 1; r < NV; ++r) k_own = (ln == r) ? kk[r] : k_own;
+    W[W_K * SLOT] = k_own;
+    __syncwarp();                              // half X, K (tile B) and the old Pvq (tile C) consumed by every lane
+    if (wl == 0 && i > 0) issue_half_x(kq_stage - kstride);
+    // one round trip for the new P: Pqv stays in tile C as the next stage's Pvq; Pqq and Pvv are symmetrised
 #pragma unroll
     for (int r = 0; r < NV; ++r) {
-      Pvq[r] = tA[r * RIC_TILE + ln];                       // Pqv[lane][r]
-      Pqq[r] = 0.5 * (Pqq[r] + tB[r * RIC_TILE + ln]);      // (Pqq[r][c] + Pqq[c][r]) / 2
+      tB[lane * RIC_TILE + r] = Pqq[r];
+      tB[lane * RIC_TILE + RIC_STASH + r] = Pvv[r];
+      tC[lane * RIC_TILE + r] = Pqv[r];
     }
     __syncwarp();
 #pragma unroll
-    for (int r = 0; r < NV; ++r) tA[lane * RIC_TILE + r] = Pvv[r];
-    __syncwarp();
-#pragma unroll
-    for (int r = 0; r < NV; ++r) Pvv[r] = 0.5 * (Pvv[r] + tA[r * RIC_TILE + ln]);
-    __syncwarp();
+    for (int r = 0; r < NV; ++r) {
+      Pqq[r] = 0.5 * (Pqq[r] + tB[r * RIC_TILE + ln]);               // (Pqq[r][c] + Pqq[c][r]) / 2
+      Pvv[r] = 0.5 * (Pvv[r] + tB[r * RIC_TILE + RIC_STASH + ln]);
+    }
     sq = nsq; sv = nsv;
 #pragma unroll
     for (int r = 0; r < NV; ++r) {
