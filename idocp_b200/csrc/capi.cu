@@ -63,12 +63,17 @@ static const char* kKernelClassNames[KC_NUM] = {"linearize", "riccati", "expand"
                                                 "update_linearize", "step_min"};
 
 // What every solver handle of both families owns: its device and stream, the device allocations, the CUDA events, the
-// launch counter and the per-kernel-class event timing.  open() / release() are the one lifecycle of a handle; the
-// *_sync / *_launch_count / *_stream / *_set_profiling / *_get_profile entry points of both families forward here.
+// launch counter, the per-kernel-class event timing, the staging buffer, the initial state and the copies between the
+// caller's host arrays and the device.  open() / release() are the one lifecycle of a handle; the *_sync /
+// *_launch_count / *_stream / *_set_profiling / *_get_profile entry points of both families forward here.
 struct DeviceHandle {
   int device = 0;
   cudaStream_t stream = nullptr;
   long long launches = 0;
+  double* d_stage = nullptr;   // staging buffer of the getters / setters; each family sizes it at create time
+  size_t stage_doubles = 0;
+  double* d_q0 = nullptr;      // initial state of the batch (upload_state)
+  double* d_v0 = nullptr;
   // profiling: 0 off, 1 = CUDA events recorded around every launch on the launching stream and
   // resolved lazily in get_profile (no host synchronisation inside the timed region)
   int profiling = 0;
@@ -89,12 +94,29 @@ struct DeviceHandle {
   // The caller's q / v may be pinned host memory that it rewrites as soon as the call returns (the normal MPC loop): the
   // host waits for the H2D copies just enqueued (an event behind them), not for the kernels enqueued after them.
   cudaEvent_t copies_done = nullptr;
-  int mark_uploads() {            // right behind the copies
-    if (!copies_done && cudaEventCreate(&copies_done) != cudaSuccess) return -1;
-    return cudaEventRecord(copies_done, stream) == cudaSuccess ? 0 : -1;
+  // copies whichever of q and v is non-null to d_q0 / d_v0 and records copies_done right behind the copies
+  int upload_state(const double* q, size_t q_doubles, const double* v, size_t v_doubles) {
+    if (q) CUDA_OK(cudaMemcpyAsync(d_q0, q, q_doubles * sizeof(double), cudaMemcpyHostToDevice, stream));
+    if (v) CUDA_OK(cudaMemcpyAsync(d_v0, v, v_doubles * sizeof(double), cudaMemcpyHostToDevice, stream));
+    if (!q && !v) return IDOCP_B200_OK;
+    if ((!copies_done && cudaEventCreate(&copies_done) != cudaSuccess) || cudaEventRecord(copies_done, stream) != cudaSuccess)
+      return fail(IDOCP_B200_CUDA_ERROR, "upload of q / v failed");
+    return IDOCP_B200_OK;
   }
   int wait_for_uploads() {        // after the call's kernels have been enqueued: the wait overlaps their execution
     return (copies_done && cudaEventSynchronize(copies_done) != cudaSuccess) ? -1 : 0;
+  }
+  // Blocking copies: `src` of upload may be pageable host memory that the caller reuses as soon as the call returns, and
+  // download returns once `dst` holds the device's data (both wait for everything enqueued on the stream before them).
+  int upload(void* dst, const void* src, size_t bytes) {
+    CUDA_OK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, stream));
+    CUDA_OK(cudaStreamSynchronize(stream));
+    return IDOCP_B200_OK;
+  }
+  int download(void* dst, const void* src, size_t bytes) {
+    CUDA_OK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, stream));
+    CUDA_OK(cudaStreamSynchronize(stream));
+    return IDOCP_B200_OK;
   }
   void resolve_profile() {
     if (prof_recs.empty()) return;
@@ -215,10 +237,6 @@ struct idocp_b200_solver : DeviceHandle {
   DevProblem* d_prob = nullptr;
   DevProblem h_prob;
   Layout L;
-  double* d_q0 = nullptr;
-  double* d_v0 = nullptr;
-  double* d_stage = nullptr;   // staging buffer for getters / setters
-  size_t stage_doubles = 0;
   // UnParNMPC extras
   ParNMPCLayout PL;
   // line search (allocated on first use)
@@ -408,7 +426,7 @@ extern "C" int idocp_b200_create(const idocp_b200_problem* p, int solver_kind, i
     idocp_b200_destroy(h);
     return fail(IDOCP_B200_CUDA_ERROR, "device memory allocation failed");
   }
-  if (cudaMemcpyAsync(h->d_prob, &h->h_prob, sizeof(DevProblem), cudaMemcpyHostToDevice, h->stream) != cudaSuccess) {
+  if (h->upload(h->d_prob, &h->h_prob, sizeof(DevProblem)) != IDOCP_B200_OK) {
     idocp_b200_destroy(h);
     return fail(IDOCP_B200_CUDA_ERROR, "problem upload failed");
   }
@@ -416,9 +434,7 @@ extern "C" int idocp_b200_create(const idocp_b200_problem* p, int solver_kind, i
     // until set_task_reference is called: identity placements (only read when the task-space cost is enabled)
     std::vector<double> ident((N + 1) * 12, 0.0);
     for (size_t i = 0; i <= N; ++i) ident[i * 12] = ident[i * 12 + 4] = ident[i * 12 + 8] = 1.0;
-    if (cudaMemcpyAsync(L.task_ref, ident.data(), ident.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream) !=
-            cudaSuccess ||
-        cudaStreamSynchronize(h->stream) != cudaSuccess) {
+    if (h->upload(L.task_ref, ident.data(), ident.size() * sizeof(double)) != IDOCP_B200_OK) {
       idocp_b200_destroy(h);
       return fail(IDOCP_B200_CUDA_ERROR, "task reference upload failed");
     }
@@ -435,32 +451,46 @@ extern "C" int idocp_b200_create(const idocp_b200_problem* p, int solver_kind, i
 
 extern "C" int idocp_b200_destroy(idocp_b200_solver* h) { return destroy_handle(h); }
 
-static int field_index(const char* name) {
-  if (!name) return -1;
-  if (!std::strcmp(name, "lmd")) return X_LMD;
-  if (!std::strcmp(name, "gmm")) return X_GMM;
-  if (!std::strcmp(name, "q")) return X_Q;
-  if (!std::strcmp(name, "v")) return X_V;
-  if (!std::strcmp(name, "a")) return X_A;
-  if (!std::strcmp(name, "u")) return X_U;
-  if (!std::strcmp(name, "beta")) return X_BETA;
-  return -1;
+// The named fields of the slot-major arrays (elem_index): `nslot` slots from `slot0` of every record of `array`
+// (`ns` slots per record).  `full`: UnOCPSolver keeps the field on N + 1 stages; every other field, and every field of
+// UnParNMPCSolver, has N.
+struct Field {
+  const char* name;
+  double* Layout::*array;
+  int ns, slot0, nslot;
+  bool full;
+};
+static const Field kFields[] = {
+    {"lmd", &Layout::X, X_NUM, X_LMD, 1, true},        {"gmm", &Layout::X, X_NUM, X_GMM, 1, true},
+    {"q", &Layout::X, X_NUM, X_Q, 1, true},            {"v", &Layout::X, X_NUM, X_V, 1, true},
+    {"a", &Layout::X, X_NUM, X_A, 1, false},           {"u", &Layout::X, X_NUM, X_U, 1, false},
+    {"beta", &Layout::X, X_NUM, X_BETA, 1, false},
+    {"dlmd", &Layout::D, D_NUM, D_LMD, 1, true},       {"dgmm", &Layout::D, D_NUM, D_GMM, 1, true},
+    {"dq", &Layout::D, D_NUM, D_Q, 1, true},           {"dv", &Layout::D, D_NUM, D_V, 1, true},
+    {"da", &Layout::D, D_NUM, D_A, 1, false},          {"du", &Layout::D, D_NUM, D_U, 1, false},
+    {"dbeta", &Layout::D, D_NUM, D_BETA, 1, false},
+    {"slack", &Layout::X, X_NUM, X_SLACK, NC, false},  {"dual", &Layout::X, X_NUM, X_DUAL, NC, false},
+    {"acc_slack", &Layout::XA, XA_NUM, 0, 2, false},   {"acc_dual", &Layout::XA, XA_NUM, 2, 2, false},
+};
+static const Field* find_field(const char* name) {
+  if (name)
+    for (const Field& f : kFields)
+      if (!std::strcmp(name, f.name)) return &f;
+  return nullptr;
 }
-static int dir_index(const char* name) {
-  if (!name) return -1;
-  if (!std::strcmp(name, "dlmd")) return D_LMD;
-  if (!std::strcmp(name, "dgmm")) return D_GMM;
-  if (!std::strcmp(name, "dq")) return D_Q;
-  if (!std::strcmp(name, "dv")) return D_V;
-  if (!std::strcmp(name, "da")) return D_A;
-  if (!std::strcmp(name, "du")) return D_U;
-  if (!std::strcmp(name, "dbeta")) return D_BETA;
-  return -1;
+// the fields of getSolution / getStageSolution: one slot of X
+static const Field* solution_field(const char* name) {
+  const Field* f = find_field(name);
+  return f && f->array == &Layout::X && f->nslot == 1 ? f : nullptr;
+}
+static int field_stages(const idocp_b200_solver* h, const Field& f) {
+  return f.full && h->kind == IDOCP_B200_SOLVER_UNOCP ? h->N + 1 : h->N;
 }
 
 extern "C" int idocp_b200_set_solution(idocp_b200_solver* h, const char* name, const double* value, int broadcast) {
   if (!h || !value) return fail(IDOCP_B200_INVALID_ARGUMENT, "set_solution: null pointer");
-  const int f = field_index(name);
+  const Field* fld = solution_field(name);
+  const int f = fld ? fld->slot0 : -1;
   if (f != X_Q && f != X_V && f != X_A && f != X_U)
     return fail(IDOCP_B200_INVALID_ARGUMENT, "invalid arugment: name must be q, v, a, or u!");
   CUDA_OK(cudaSetDevice(h->device));
@@ -481,15 +511,6 @@ extern "C" int idocp_b200_init_constraints(idocp_b200_solver* h) {
   if (!h) return fail(IDOCP_B200_INVALID_ARGUMENT, "null handle");
   CUDA_OK(cudaSetDevice(h->device));
   return do_init_constraints(h);
-}
-
-static int upload_x0(idocp_b200_solver* h, const double* q, const double* v) {
-  if (!q || !v) return fail(IDOCP_B200_INVALID_ARGUMENT, "q / v: null pointer");
-  const size_t n = static_cast<size_t>(h->B) * NV * sizeof(double);
-  CUDA_OK(cudaMemcpyAsync(h->d_q0, q, n, cudaMemcpyHostToDevice, h->stream));
-  CUDA_OK(cudaMemcpyAsync(h->d_v0, v, n, cudaMemcpyHostToDevice, h->stream));
-  if (h->mark_uploads() != 0) return fail(IDOCP_B200_CUDA_ERROR, "upload of q / v failed");
-  return IDOCP_B200_OK;
 }
 
 static int ensure_line_search(idocp_b200_solver* h) {
@@ -667,7 +688,8 @@ extern "C" int idocp_b200_update_solution(idocp_b200_solver* h, double t, const 
                                           int line_search) {
   if (!h) return fail(IDOCP_B200_INVALID_ARGUMENT, "null handle");
   CUDA_OK(cudaSetDevice(h->device));
-  int rc = upload_x0(h, q, v);
+  if (!q || !v) return fail(IDOCP_B200_INVALID_ARGUMENT, "q / v: null pointer");
+  int rc = h->upload_state(q, static_cast<size_t>(h->B) * NV, v, static_cast<size_t>(h->B) * NV);
   if (rc != IDOCP_B200_OK) return rc;
   rc = idocp_b200_update_solution_device(h, t, h->d_q0, h->d_v0, line_search);
   if (h->wait_for_uploads() != 0) return fail(IDOCP_B200_CUDA_ERROR, "upload of q / v failed");
@@ -696,7 +718,8 @@ extern "C" int idocp_b200_compute_kkt_residual_device(idocp_b200_solver* h, doub
 extern "C" int idocp_b200_compute_kkt_residual(idocp_b200_solver* h, double t, const double* q, const double* v) {
   if (!h) return fail(IDOCP_B200_INVALID_ARGUMENT, "null handle");
   CUDA_OK(cudaSetDevice(h->device));
-  int rc = upload_x0(h, q, v);
+  if (!q || !v) return fail(IDOCP_B200_INVALID_ARGUMENT, "q / v: null pointer");
+  int rc = h->upload_state(q, static_cast<size_t>(h->B) * NV, v, static_cast<size_t>(h->B) * NV);
   if (rc != IDOCP_B200_OK) return rc;
   rc = idocp_b200_compute_kkt_residual_device(h, t, h->d_q0, h->d_v0);
   if (h->wait_for_uploads() != 0) return fail(IDOCP_B200_CUDA_ERROR, "upload of q / v failed");
@@ -706,149 +729,76 @@ extern "C" int idocp_b200_compute_kkt_residual(idocp_b200_solver* h, double t, c
 extern "C" int idocp_b200_kkt_error(idocp_b200_solver* h, double* out) {
   if (!h || !out) return fail(IDOCP_B200_INVALID_ARGUMENT, "kkt_error: null pointer");
   CUDA_OK(cudaSetDevice(h->device));
-  CUDA_OK(cudaMemcpyAsync(out, h->L.kkt_err, static_cast<size_t>(h->B) * sizeof(double), cudaMemcpyDeviceToHost,
-                          h->stream));
-  CUDA_OK(cudaStreamSynchronize(h->stream));
-  return IDOCP_B200_OK;
+  return h->download(out, h->L.kkt_err, static_cast<size_t>(h->B) * sizeof(double));
 }
 
-// gather one slot of `nstage` stages: out[b][stage][7]
-__global__ void k_gather(const double* __restrict__ src, int ns, int slot, int nstage, int B, int G,
+// out[b][i][c][j] = src[elem_index(ns, G, stage0 + i, b, slot0 + c, j)] for b < B, i < nstage, c < nslot, j < NV
+__global__ void k_gather(const double* __restrict__ src, int ns, int G, int B, int stage0, int nstage, int slot0, int nslot,
                          double* __restrict__ out) {
   const long idx = static_cast<long>(blockIdx.x) * blockDim.x + threadIdx.x;
-  const long total = static_cast<long>(B) * nstage * NV;
+  const long total = static_cast<long>(B) * nstage * nslot * NV;
   if (idx >= total) return;
   const int j = static_cast<int>(idx % NV);
-  const long t = idx / NV;
+  long t = idx / NV;
+  const int c = static_cast<int>(t % nslot);
+  t /= nslot;
   const int i = static_cast<int>(t % nstage);
   const int b = static_cast<int>(t / nstage);
-  out[idx] = src[elem_index(ns, G, i, b, slot, j)];
+  out[idx] = src[elem_index(ns, G, stage0 + i, b, slot0 + c, j)];
 }
 
-static int gather_to_host(idocp_b200_solver* h, const double* src, int ns, int slot, int nstage, double* out) {
-  const long total = static_cast<long>(h->B) * nstage * NV;
+// field f of stages stage0 .. stage0 + nstage - 1 of the whole batch: out[b][stage][slot][7]
+static int gather_to_host(idocp_b200_solver* h, const Field& f, int stage0, int nstage, double* out) {
+  const long total = static_cast<long>(h->B) * nstage * f.nslot * NV;
   if (static_cast<size_t>(total) > h->stage_doubles) return fail(IDOCP_B200_INVALID_ARGUMENT, "staging buffer too small");
-  IDOCP_LAUNCH(h, KC_MISC, k_gather, static_cast<int>((total + 255) / 256), 256, 0, src, ns, slot, nstage, h->B,
-               h->L.G, h->d_stage);
+  CUDA_OK(cudaSetDevice(h->device));
+  IDOCP_LAUNCH(h, KC_MISC, k_gather, static_cast<int>((total + 255) / 256), 256, 0, h->L.*f.array, f.ns, h->L.G, h->B, stage0,
+               nstage, f.slot0, f.nslot, h->d_stage);
   CUDA_OK(cudaGetLastError());
-  CUDA_OK(cudaMemcpyAsync(out, h->d_stage, total * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-  CUDA_OK(cudaStreamSynchronize(h->stream));
-  return IDOCP_B200_OK;
-}
-
-static bool full_horizon(const idocp_b200_solver* h, int f) {
-  return (f == X_LMD || f == X_GMM || f == X_Q || f == X_V) && h->kind == IDOCP_B200_SOLVER_UNOCP;
+  return h->download(out, h->d_stage, total * sizeof(double));
 }
 
 extern "C" int idocp_b200_get_solution(idocp_b200_solver* h, const char* name, double* out) {
   if (!h || !out) return fail(IDOCP_B200_INVALID_ARGUMENT, "get_solution: null pointer");
-  const int f = field_index(name);
-  if (f < 0) return fail(IDOCP_B200_INVALID_ARGUMENT, "get_solution: unknown field");
-  CUDA_OK(cudaSetDevice(h->device));
-  return gather_to_host(h, h->L.X, X_NUM, f, full_horizon(h, f) ? h->N + 1 : h->N, out);
+  const Field* f = solution_field(name);
+  if (!f) return fail(IDOCP_B200_INVALID_ARGUMENT, "get_solution: unknown field");
+  return gather_to_host(h, *f, 0, field_stages(h, *f), out);
 }
 
 // one stage of one field: out[b][7]
-__global__ void k_gather_stage(const double* __restrict__ src, int ns, int slot, int stage, int B, int G,
-                               double* __restrict__ out) {
-  const long idx = static_cast<long>(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (idx >= static_cast<long>(B) * OCT) return;
-  const int j = static_cast<int>(idx & 7);
-  const int b = static_cast<int>(idx >> 3);
-  if (j < NV) out[static_cast<size_t>(b) * NV + j] = src[elem_index(ns, G, stage, b, slot, j)];
-}
-
 extern "C" int idocp_b200_get_stage_solution(idocp_b200_solver* h, const char* name, int stage, double* out) {
   if (!h || !out) return fail(IDOCP_B200_INVALID_ARGUMENT, "get_stage_solution: null pointer");
-  const int f = field_index(name);
-  if (f < 0) return fail(IDOCP_B200_INVALID_ARGUMENT, "get_stage_solution: unknown field");
-  if (stage < 0 || stage >= (full_horizon(h, f) ? h->N + 1 : h->N))
+  const Field* f = solution_field(name);
+  if (!f) return fail(IDOCP_B200_INVALID_ARGUMENT, "get_stage_solution: unknown field");
+  if (stage < 0 || stage >= field_stages(h, *f))
     return fail(IDOCP_B200_INVALID_ARGUMENT, "get_stage_solution: stage out of range");
-  CUDA_OK(cudaSetDevice(h->device));
-  const long total = static_cast<long>(h->B) * OCT;
-  IDOCP_LAUNCH(h, KC_MISC, k_gather_stage, static_cast<int>((total + 255) / 256), 256, 0, h->L.X, X_NUM, f, stage,
-               h->B, h->L.G, h->d_stage);
-  CUDA_OK(cudaGetLastError());
-  CUDA_OK(cudaMemcpyAsync(out, h->d_stage, static_cast<size_t>(h->B) * NV * sizeof(double), cudaMemcpyDeviceToHost,
-                          h->stream));
-  CUDA_OK(cudaStreamSynchronize(h->stream));
-  return IDOCP_B200_OK;
+  return gather_to_host(h, *f, stage, 1, out);
 }
 
 extern "C" int idocp_b200_get_direction(idocp_b200_solver* h, const char* name, double* out) {
   if (!h || !out) return fail(IDOCP_B200_INVALID_ARGUMENT, "get_direction: null pointer");
-  const int f = dir_index(name);
-  if (f < 0) return fail(IDOCP_B200_INVALID_ARGUMENT, "get_direction: unknown field");
-  CUDA_OK(cudaSetDevice(h->device));
-  const bool full = (f == D_LMD || f == D_GMM || f == D_Q || f == D_V) && h->kind == IDOCP_B200_SOLVER_UNOCP;
-  return gather_to_host(h, h->L.D, D_NUM, f, full ? h->N + 1 : h->N, out);
+  const Field* f = find_field(name);
+  if (!f || f->array != &Layout::D) return fail(IDOCP_B200_INVALID_ARGUMENT, "get_direction: unknown field");
+  return gather_to_host(h, *f, 0, field_stages(h, *f), out);
 }
 
-// out[b][N][6][7]
-__global__ void k_gather_constraints(const double* __restrict__ X, int first_slot, int N, int B, int G,
-                                     double* __restrict__ out) {
-  const long idx = static_cast<long>(blockIdx.x) * blockDim.x + threadIdx.x;
-  const long total = static_cast<long>(B) * N * NC * NV;
-  if (idx >= total) return;
-  const int j = static_cast<int>(idx % NV);
-  long t = idx / NV;
-  const int c = static_cast<int>(t % NC);
-  t /= NC;
-  const int i = static_cast<int>(t % N);
-  const int b = static_cast<int>(t / N);
-  out[idx] = X[elem_index(X_NUM, G, i, b, first_slot + c, j)];
-}
-
-// out[b][N][2][7]: slots first_slot, first_slot + 1 of the acceleration-limit record
-__global__ void k_gather_acc_rows(const double* __restrict__ XA, int first_slot, int N, int B, int G, double* __restrict__ out) {
-  const long idx = static_cast<long>(blockIdx.x) * blockDim.x + threadIdx.x;
-  const long total = static_cast<long>(B) * N * 2 * NV;
-  if (idx >= total) return;
-  const int j = static_cast<int>(idx % NV);
-  long t = idx / NV;
-  const int c = static_cast<int>(t % 2);
-  t /= 2;
-  const int i = static_cast<int>(t % N);
-  const int b = static_cast<int>(t / N);
-  out[idx] = XA[elem_index(XA_NUM, G, i, b, first_slot + c, j)];
-}
-
+// out[b][N][6][7] (slack, dual: the six joint-limit components) or out[b][N][2][7] (acc_slack, acc_dual: the two
+// acceleration-limit components)
 extern "C" int idocp_b200_get_constraint_data(idocp_b200_solver* h, const char* name, double* out) {
   if (!h || !out || !name) return fail(IDOCP_B200_INVALID_ARGUMENT, "get_constraint_data: null pointer");
-  int first = -1;
-  if (!std::strcmp(name, "slack")) first = X_SLACK;
-  else if (!std::strcmp(name, "dual")) first = X_DUAL;
-  else if (!std::strcmp(name, "acc_slack") || !std::strcmp(name, "acc_dual")) {
-    // the two acceleration-limit components: out[batch][N][2][dimv]
-    if (!h->L.XA) return fail(IDOCP_B200_INVALID_ARGUMENT, "get_constraint_data: the acceleration limits are not enabled");
-    CUDA_OK(cudaSetDevice(h->device));
-    const long tot = static_cast<long>(h->B) * h->N * 2 * NV;
-    IDOCP_LAUNCH(h, KC_MISC, k_gather_acc_rows, static_cast<int>((tot + 255) / 256), 256, 0, h->L.XA, name[4] == 's' ? 0 : 2, h->N,
-                 h->B, h->L.G, h->d_stage);
-    CUDA_OK(cudaGetLastError());
-    CUDA_OK(cudaMemcpyAsync(out, h->d_stage, tot * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_OK(cudaStreamSynchronize(h->stream));
-    return IDOCP_B200_OK;
-  }
-  else return fail(IDOCP_B200_INVALID_ARGUMENT, "get_constraint_data: name must be slack, dual, acc_slack or acc_dual");
-  CUDA_OK(cudaSetDevice(h->device));
-  const long total = static_cast<long>(h->B) * h->N * NC * NV;
-  IDOCP_LAUNCH(h, KC_MISC, k_gather_constraints, static_cast<int>((total + 255) / 256), 256, 0, h->L.X, first, h->N,
-               h->B, h->L.G, h->d_stage);
-  CUDA_OK(cudaGetLastError());
-  CUDA_OK(cudaMemcpyAsync(out, h->d_stage, total * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-  CUDA_OK(cudaStreamSynchronize(h->stream));
-  return IDOCP_B200_OK;
+  const Field* f = find_field(name);
+  if (!f || f->nslot == 1)
+    return fail(IDOCP_B200_INVALID_ARGUMENT, "get_constraint_data: name must be slack, dual, acc_slack or acc_dual");
+  if (!(h->L.*f->array)) return fail(IDOCP_B200_INVALID_ARGUMENT, "get_constraint_data: the acceleration limits are not enabled");
+  return gather_to_host(h, *f, 0, h->N, out);
 }
 
 extern "C" int idocp_b200_get_step_sizes(idocp_b200_solver* h, double* primal, double* dual) {
   if (!h) return fail(IDOCP_B200_INVALID_ARGUMENT, "null handle");
   CUDA_OK(cudaSetDevice(h->device));
   const size_t n = static_cast<size_t>(h->B) * sizeof(double);
-  if (primal) CUDA_OK(cudaMemcpyAsync(primal, h->L.steps, n, cudaMemcpyDeviceToHost, h->stream));
-  if (dual) CUDA_OK(cudaMemcpyAsync(dual, h->L.steps + h->Bp, n, cudaMemcpyDeviceToHost, h->stream));
-  CUDA_OK(cudaStreamSynchronize(h->stream));
-  return IDOCP_B200_OK;
+  const int rc = primal ? h->download(primal, h->L.steps, n) : IDOCP_B200_OK;
+  return rc == IDOCP_B200_OK && dual ? h->download(dual, h->L.steps + h->Bp, n) : rc;
 }
 
 // Q[b][21*21] column-major (block order a,q,v), res[b][35]
@@ -879,19 +829,14 @@ extern "C" int idocp_b200_get_unkkt(idocp_b200_solver* h, int stage, double* Q, 
   double* dres = h->d_stage + static_cast<size_t>(h->B) * 441;
   IDOCP_LAUNCH(h, KC_MISC, k_gather_unkkt, h->B, 128, 0, h->L, stage, dQ, dres);
   CUDA_OK(cudaGetLastError());
-  CUDA_OK(cudaMemcpyAsync(Q, dQ, static_cast<size_t>(h->B) * 441 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-  CUDA_OK(cudaMemcpyAsync(res, dres, static_cast<size_t>(h->B) * 35 * sizeof(double), cudaMemcpyDeviceToHost,
-                          h->stream));
-  CUDA_OK(cudaStreamSynchronize(h->stream));
-  return IDOCP_B200_OK;
+  const int rc = h->download(Q, dQ, static_cast<size_t>(h->B) * 441 * sizeof(double));
+  return rc == IDOCP_B200_OK ? h->download(res, dres, static_cast<size_t>(h->B) * 35 * sizeof(double)) : rc;
 }
 
 extern "C" int idocp_b200_get_status(idocp_b200_solver* h, int* out) {
   if (!h || !out) return fail(IDOCP_B200_INVALID_ARGUMENT, "get_status: null pointer");
   CUDA_OK(cudaSetDevice(h->device));
-  CUDA_OK(cudaMemcpyAsync(out, h->L.status, static_cast<size_t>(h->B) * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-  CUDA_OK(cudaStreamSynchronize(h->stream));
-  return IDOCP_B200_OK;
+  return h->download(out, h->L.status, static_cast<size_t>(h->B) * sizeof(int));
 }
 
 __global__ void k_is_feasible(const DevProblem* __restrict__ Pp, Layout L, int stage_offset, int* __restrict__ out) {
@@ -922,9 +867,7 @@ extern "C" int idocp_b200_is_feasible(idocp_b200_solver* h, int* out) {
   int* d = reinterpret_cast<int*>(h->d_stage);
   IDOCP_LAUNCH(h, KC_MISC, k_is_feasible, (h->B + 127) / 128, 128, 0, h->d_prob, h->L, h->stage_offset(), d);
   CUDA_OK(cudaGetLastError());
-  CUDA_OK(cudaMemcpyAsync(out, d, static_cast<size_t>(h->B) * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-  CUDA_OK(cudaStreamSynchronize(h->stream));
-  return IDOCP_B200_OK;
+  return h->download(out, d, static_cast<size_t>(h->B) * sizeof(int));
 }
 
 extern "C" int idocp_b200_clear_line_search_filter(idocp_b200_solver* h) {
@@ -947,11 +890,8 @@ extern "C" int idocp_b200_init_backward_correction(idocp_b200_solver* h, double 
 extern "C" int idocp_b200_set_task_reference(idocp_b200_solver* h, const double* table) {
   if (!h || !table) return fail(IDOCP_B200_INVALID_ARGUMENT, "set_task_reference: null pointer");
   CUDA_OK(cudaSetDevice(h->device));
-  CUDA_OK(cudaMemcpyAsync(h->L.task_ref, table, static_cast<size_t>(h->N + 1) * 12 * sizeof(double),
-                          cudaMemcpyHostToDevice, h->stream));
-  CUDA_OK(cudaStreamSynchronize(h->stream));  // `table` may be pageable host memory reused by the caller
   h->lin_valid = false; h->kkt_valid = false;                       // the kept linearisation used the old reference
-  return IDOCP_B200_OK;
+  return h->upload(h->L.task_ref, table, static_cast<size_t>(h->N + 1) * 12 * sizeof(double));
 }
 
 // UnOCPSolver pipelining (default on): see k_linearize<.., FUSED>.  Off: linearise, solve, expand, update as four launches;

@@ -6,8 +6,9 @@
 
 Runs bench.py once per library per round, in the order A B A B ... so that clock and neighbour drift hit both sides
 alike, and reports the median and the min..max spread of ms_per_step and of every kernel's ms_per_launch for each
-library.  The GPU's name, power limit and maximum SM clock are read with nvidia-smi in the same session and stored with
-the numbers.  Arguments after `--` go to bench.py unchanged.
+library, and of e2e.ms_per_step (the same steps through the host API, with its host <-> device copies) where
+bench.py reports it.  The GPU's name, power limit and maximum SM clock are read with nvidia-smi in the same session and
+stored with the numbers.  Arguments after `--` go to bench.py unchanged.
 """
 import argparse
 import json
@@ -44,17 +45,23 @@ def main():
     smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
                          capture_output=True, text=True).stdout.strip().splitlines()
     step = {t: [] for t, _ in libs}
+    e2e = {t: [] for t, _ in libs}
     kern = {t: {} for t, _ in libs}
     for r in range(a.rounds):
         for t, path in libs:
             d = run_bench(path, bench_args)
             step[t].append(d["ms_per_step"])
+            if "ms_per_step" in (d.get("e2e") or {}):
+                e2e[t].append(d["e2e"]["ms_per_step"])
             for name, k in ((d.get("roofline") or {}).get("kernels") or {}).items():
-                kern[t].setdefault(name, []).append(k["ms_per_launch"])
-            print("round %d %-8s ms_per_step %.4f  %s" % (r, t, d["ms_per_step"],
+                # the ANYmal lines give some kernels only per-step figures
+                ms = k["ms_per_launch"] if "ms_per_launch" in k else k["ms_per_step"] / k["launches_per_step"]
+                kern[t].setdefault(name, []).append(ms)
+            print("round %d %-8s ms_per_step %.4f  e2e %s  %s" % (r, t, d["ms_per_step"], e2e[t][-1] if e2e[t] else None,
                   {n: round(v[-1], 4) for n, v in kern[t].items()}), flush=True)
     summary = {"gpu": smi, "bench_args": bench_args, "rounds": a.rounds,
-               "libraries": {t: {"ms_per_step": spread(step[t]), "kernels": {n: spread(v) for n, v in kern[t].items()}}
+               "libraries": {t: {"ms_per_step": spread(step[t]),
+                                 "e2e_ms_per_step": spread(e2e[t]) if e2e[t] else None, "kernels": {n: spread(v) for n, v in kern[t].items()}}
                              for t, _ in libs}}
     text = json.dumps(summary)
     print(text)
