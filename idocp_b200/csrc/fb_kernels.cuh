@@ -19,6 +19,7 @@
 #include "fb_math.cuh"
 #include "warp_llt.cuh"
 #include "line_search_filter.cuh"
+#include "pdipm.cuh"
 
 namespace idocp_b200 {
 
@@ -59,6 +60,29 @@ struct FbDevProblem {
 __host__ __device__ inline int fbc_cone_bits(const FbDevProblem& pr) { return (pr.cone_nonlinear[0] ? 1 : 0) | (pr.cone_nonlinear[1] ? 2 : 0); }
 __host__ __device__ inline int fbc_cone_rows(int nl, int c) { return ((nl >> (c - FBC_FRICTION)) & 1) ? 2 : 5; }
 __host__ __device__ inline int fbc_rows(int nl, int c) { return fbc_is_cone(c) ? FB_NC * fbc_cone_rows(nl, c) : (c == FBC_DISTANCE ? FB_NC : 12); }
+// contact of row j of cone component c, and the row within that contact's cone (no division by a run-time value).  The row is
+// formed from the contact rather than as j % 5: k_fb_expand would otherwise keep it live across its active-contact count and spill.
+__host__ __device__ inline void fbc_cone_row(int nl, int c, int j, int& contact, int& row) {
+  const int rpc = fbc_cone_rows(nl, c);
+  contact = rpc == 2 ? (j >> 1) : (j / 5);
+  row = j - rpc * contact;
+}
+
+// margin of row j of box component c (joint position / velocity / torque / acceleration limit): >= 0 is feasible; the residual
+// of the row is slack - margin
+__device__ __forceinline__ double fbc_box_margin(int c, int j, const FbDevProblem& pr, const double* q, const double* v, const double* a,
+                                                 const double* u) {
+  switch (c) {
+    case FBC_ACC_LO: return a[6 + j] - pr.a_min[j];
+    case FBC_ACC_UP: return pr.a_max[j] - a[6 + j];
+    case FBC_POS_LO: return q[7 + j] - pr.q_min[j];
+    case FBC_POS_UP: return pr.q_max[j] - q[7 + j];
+    case FBC_VEL_LO: return v[6 + j] - (-pr.v_max[j]);
+    case FBC_VEL_UP: return pr.v_max[j] - v[6 + j];
+    case FBC_TRQ_LO: return u[j] - (-pr.u_max[j]);
+    default:         return pr.u_max[j] - u[j];
+  }
+}
 
 // one element of the hybrid chain (shared by the whole batch)
 struct FbElem {
@@ -1028,25 +1052,16 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
       if (el.cactive[c] && j < fbc_rows(nl, c) && c != FBC_DISTANCE) {   // ContactDistance: after the kinematics, below
         const double sl = S.slack[idx];
         if (fbc_is_cone(c)) {
-          const int rpc = fbc_cone_rows(nl, c);
-          const int i = rpc == 2 ? (j >> 1) : (j / 5);   // no division by a run-time value
+          int i, ee;
+          fbc_cone_row(nl, c, j, i, ee);
           if (el.active[i]) {
             double r5[5];
-            fb_friction_residual(pr.mu, rpc == 2, w.f + 3 * i, r5);
-            res = r5[(rpc == 2 ? (j & 1) : (j % 5))] + sl;
+            fb_friction_residual(pr.mu, fbc_cone_rows(nl, c) == 2, w.f + 3 * i, r5);
+            res = r5[ee] + sl;
             dua = sl * S.dual[idx] - pr.barrier;
           }
         } else {
-          switch (c) {
-            case FBC_ACC_LO: res = pr.a_min[j] - w.a[6 + j] + sl; break;
-            case FBC_ACC_UP: res = w.a[6 + j] - pr.a_max[j] + sl; break;
-            case FBC_POS_LO: res = pr.q_min[j] - w.q[7 + j] + sl; break;
-            case FBC_POS_UP: res = w.q[7 + j] - pr.q_max[j] + sl; break;
-            case FBC_VEL_LO: res = (-pr.v_max[j]) - w.v[6 + j] + sl; break;
-            case FBC_VEL_UP: res = w.v[6 + j] - pr.v_max[j] + sl; break;
-            case FBC_TRQ_LO: res = (-pr.u_max[j]) - w.u[j] + sl; break;
-            default:         res = w.u[j] - pr.u_max[j] + sl; break;
-          }
+          res = sl - fbc_box_margin(c, j, pr, w.q, w.v, w.a, w.u);
           dua = sl * S.dual[idx] - pr.barrier;
         }
       }
@@ -1093,8 +1108,8 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
     for (int c = 0; c < 4; ++c) {
       if (!el.cactive[c]) continue;
       const double sg = (c & 1) ? 1.0 : -1.0;
-      if (c <= FBC_POS_UP) lq += sg * (dt * S.dual[12 * c + j]);
-      else lv += sg * (dt * S.dual[12 * c + j]);
+      if (c <= FBC_POS_UP) lq += sg * (dt * S.dual[fbc_offset(c) + j]);
+      else lv += sg * (dt * S.dual[fbc_offset(c) + j]);
     }
     for (int c = FBC_ACC_LO; c <= FBC_ACC_UP; ++c) {   // JointAcceleration{Lower,Upper}Limit: la.tail(12) -/+= dt dual
       if (!el.cactive[c]) continue;
@@ -1106,7 +1121,7 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
     for (int c = 4; c < 6; ++c) {
       if (!el.cactive[c]) continue;
       const double sg = (c & 1) ? 1.0 : -1.0;
-      lu += sg * (dt * S.dual[12 * c + lane]);
+      lu += sg * (dt * S.dual[fbc_offset(c) + lane]);
     }
   }
   const int cfr = impulse ? FBC_IMPULSE_FRICTION : FBC_FRICTION;
@@ -1333,10 +1348,11 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
         for (int c = FBC_ACC_LO; c <= FBC_ACC_UP; ++c) {
           if (!el.cactive[c]) continue;
           const int idx = fbc_offset(c) + j - 6;
-          const double rs = 1.0 / S.slack[idx];
-          qad += (dt * S.dual[idx]) * rs;
+          double h, g;
+          pdipm_condense(dt, S.slack[idx], S.dual[idx], Dr.residual[idx], Dr.duality[idx], h, g);
+          qad += h;
           const double sg = (c & 1) ? 1.0 : -1.0;
-          la += sg * ((dt * fma(S.dual[idx], Dr.residual[idx], -Dr.duality[idx])) * rs);
+          la += sg * g;
         }
       }
       L.Qaa[j] = qad;
@@ -1350,23 +1366,23 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
       const int j = lane - 6;
       for (int c = 0; c < 4; ++c) {
         if (!el.cactive[c]) continue;
-        const int idx = 12 * c + j;
-        const double rs = 1.0 / S.slack[idx];
-        const double h = (dt * S.dual[idx]) * rs;
+        const int idx = fbc_offset(c) + j;
+        double h, g;
+        pdipm_condense(dt, S.slack[idx], S.dual[idx], Dr.residual[idx], Dr.duality[idx], h, g);
         const double sg = (c & 1) ? 1.0 : -1.0;
-        const double g = sg * ((dt * fma(S.dual[idx], Dr.residual[idx], -Dr.duality[idx])) * rs);
-        if (c <= FBC_POS_UP) { qqd += h; lq += g; }
-        else { qvd += h; lv += g; }
+        if (c <= FBC_POS_UP) { qqd += h; lq += sg * g; }
+        else { qvd += h; lv += sg * g; }
       }
     }
     if (lane < FB_NU) {
       for (int c = 4; c < 6; ++c) {
         if (!el.cactive[c]) continue;
-        const int idx = 12 * c + lane;
-        const double rs = 1.0 / S.slack[idx];
-        qud += (dt * S.dual[idx]) * rs;
+        const int idx = fbc_offset(c) + lane;
+        double h, g;
+        pdipm_condense(dt, S.slack[idx], S.dual[idx], Dr.residual[idx], Dr.duality[idx], h, g);
+        qud += h;
         const double sg = (c & 1) ? 1.0 : -1.0;
-        lu += sg * ((dt * fma(S.dual[idx], Dr.residual[idx], -Dr.duality[idx])) * rs);
+        lu += sg * g;
       }
       L.Quu_d[lane] = qud;
     }
@@ -1391,9 +1407,8 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
       for (int i = 0; i < FB_NC; ++i) {
         double wgt = 0.0;
         if (!el.active[i]) {
-          const double rs = 1.0 / S.slack[o + i];
-          wgt = (dt * S.dual[o + i]) * rs;
-          const double g2 = (dt * fma(S.dual[o + i], Dr.residual[o + i], -Dr.duality[o + i])) * rs;
+          double g2;
+          pdipm_condense(dt, S.slack[o + i], S.dual[o + i], Dr.residual[o + i], Dr.duality[o + i], wgt, g2);
           if (lane < FB_NV) lq -= g2 * L.cdJ[i * FB_NV + lane];   // written by this very lane above
         }
         if (lane == 0) L.cdw[i] = wgt;
@@ -2105,12 +2120,7 @@ __global__ void __launch_bounds__(64) k_fb_riccati_forward(FbArrays A) {
 // =====================================================================================================
 __device__ inline double fb_fraction_to_boundary(double rate, int nn, const double* vec, const double* dvec) {
   double mn = 1.0;
-  for (int i = 0; i < nn; ++i) {
-    const double f = -rate * (vec[i] / dvec[i]);
-    if (f > 0 && f < 1) {
-      if (f < mn) mn = f;
-    }
-  }
+  for (int i = 0; i < nn; ++i) mn = pdipm_fraction_row(rate, vec[i], dvec[i], mn);
   return mn;
 }
 
@@ -2184,25 +2194,24 @@ __global__ void __launch_bounds__(64) k_fb_expand(FbArrays A) {
     double ds = 0.0, dd = 0.0;
     if (el.cactive[c] && j < fbc_rows(nl, c)) {
       if (fbc_is_cone(c)) {
-        const int rpc = fbc_cone_rows(nl, c);
-        const int i = rpc == 2 ? (j >> 1) : (j / 5);   // no division by a run-time value
+        int i, ee;
+        fbc_cone_row(nl, c, j, i, ee);
         ds = 1.0; dd = 1.0;
         if (el.active[i]) {
           int k = 0;
           for (int jj = 0; jj < i; ++jj) k += el.active[jj];
           const double* df = daf + NV + 3 * k;
           const double* fi = S.f + 3 * i;
-          const int ee = (rpc == 2 ? (j & 1) : (j % 5));
-          const bool nlc = rpc == 2;
+          const bool nlc = fbc_cone_rows(nl, c) == 2;
           const double Jdf = fma(fb_friction_jac(pr.mu, nlc, fi, ee, 2), df[2],
                                  fma(fb_friction_jac(pr.mu, nlc, fi, ee, 1), df[1], fb_friction_jac(pr.mu, nlc, fi, ee, 0) * df[0]));
           ds = -Jdf - Dr.residual[idx];
-          dd = -fma(S.dual[idx], ds, Dr.duality[idx]) / S.slack[idx];
+          dd = pdipm_dual_direction(S.slack[idx], S.dual[idx], Dr.duality[idx], ds);
         }
       } else {
         const double d = c <= FBC_POS_UP ? dx[6 + j] : (c <= FBC_VEL_UP ? dx[NV + 6 + j] : (c >= FBC_ACC_LO ? daf[6 + j] : du[j]));
         ds = ((c & 1) ? -d : d) - Dr.residual[idx];
-        dd = -fma(S.dual[idx], ds, Dr.duality[idx]) / S.slack[idx];
+        dd = pdipm_dual_direction(S.slack[idx], S.dual[idx], Dr.duality[idx], ds);
       }
     }
     dslack[idx] = ds;
@@ -2221,7 +2230,7 @@ __global__ void __launch_bounds__(64) k_fb_expand(FbArrays A) {
 #pragma unroll 1
       for (int l = 1; l < NV; ++l) acc = fma(J2[l], dx[l], acc);
       ds = acc - Dr.residual[idx];
-      dd = -fma(S.dual[idx], ds, Dr.duality[idx]) / S.slack[idx];
+      dd = pdipm_dual_direction(S.slack[idx], S.dual[idx], Dr.duality[idx], ds);
     }
     dslack[idx] = ds;
     ddual[idx] = dd;
@@ -2377,19 +2386,21 @@ __global__ void __launch_bounds__(64, FB_UPD_MINB) k_fb_update(FbArrays A) {
   }
 }
 
-// KKT error of every instance (ocp_linearizer.cpp:97-137): sum in the reference's order (grid stages and the
-// terminal stage, impulse, aux, lift), one thread per instance
+// the reference's order of sums over the chain (ocp_linearizer.cpp:97-137, line_search.hpp:174-182): pass 0 the grid
+// stages and the terminal stage, pass 1 impulse, pass 2 aux, pass 3 lift
+__host__ __device__ inline bool fb_in_pass(int kind, int pass) {
+  return (pass == 0 && (kind == FB_GRID || kind == FB_TERMINAL)) || (pass == 1 && kind == FB_IMPULSE) || (pass == 2 && kind == FB_AUX) ||
+         (pass == 3 && kind == FB_LIFT);
+}
+
+// KKT error of every instance (ocp_linearizer.cpp:97-137), one thread per instance
 __global__ void k_fb_kkt_sum(FbArrays A) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= A.B) return;
   double sum = 0.0;
   for (int pass = 0; pass < 4; ++pass)
-    for (int e = 0; e < A.n_elems; ++e) {
-      const int k = A.elems[e].kind;
-      const bool mine = (pass == 0 && (k == FB_GRID || k == FB_TERMINAL)) || (pass == 1 && k == FB_IMPULSE) ||
-                        (pass == 2 && k == FB_AUX) || (pass == 3 && k == FB_LIFT);
-      if (mine) sum += A.dir[(size_t)A.elems[e].slot * A.B + b].kkt_sq;
-    }
+    for (int e = 0; e < A.n_elems; ++e)
+      if (fb_in_pass(A.elems[e].kind, pass)) sum += A.dir[(size_t)A.elems[e].slot * A.B + b].kkt_sq;
   A.kkt_err[b] = sqrt(sum);
 }
 
@@ -2410,28 +2421,17 @@ __global__ void k_fb_init_constraints(FbArrays A, const FbInitRow* rows, int n_r
       double sl = 0.0, du = 0.0;
       if (c == FBC_DISTANCE && row.cactive[c]) continue;   // needs the forward kinematics: k_fb_init_distance
       if (row.cactive[c] && j < fbc_rows(nl, c)) {
+        double margin;
         if (fbc_is_cone(c)) {
-          const int rpc = fbc_cone_rows(nl, c);
+          int i, ee;
+          fbc_cone_row(nl, c, j, i, ee);
           double r5[5];
-          fb_friction_residual(pr.mu, rpc == 2, S.f + 3 * (rpc == 2 ? (j >> 1) : (j / 5)), r5);
-          sl = -r5[(rpc == 2 ? (j & 1) : (j % 5))];
+          fb_friction_residual(pr.mu, fbc_cone_rows(nl, c) == 2, S.f + 3 * i, r5);
+          margin = -r5[ee];
         } else {
-          switch (c) {
-            case FBC_ACC_LO: sl = S.a[6 + j] - pr.a_min[j]; break;
-            case FBC_ACC_UP: sl = pr.a_max[j] - S.a[6 + j]; break;
-            case FBC_POS_LO: sl = S.q[7 + j] - pr.q_min[j]; break;
-            case FBC_POS_UP: sl = pr.q_max[j] - S.q[7 + j]; break;
-            case FBC_VEL_LO: sl = S.v[6 + j] - (-pr.v_max[j]); break;
-            case FBC_VEL_UP: sl = pr.v_max[j] - S.v[6 + j]; break;
-            case FBC_TRQ_LO: sl = S.u[j] - (-pr.u_max[j]); break;
-            default:         sl = pr.u_max[j] - S.u[j]; break;
-          }
+          margin = fbc_box_margin(c, j, pr, S.q, S.v, S.a, S.u);
         }
-        // pdipm::SetSlackAndDualPositive (pdipm.hxx:13-23); the iteration bound keeps a margin of -inf (or a huge
-        // violation in the initial guess) from hanging the stream -- same bound as k_init_constraints and the oracle
-        int guard = 0;
-        while (sl < pr.barrier && guard < (1 << 20)) { sl += pr.barrier; ++guard; }
-        du = pr.barrier / sl;
+        pdipm_set_slack_and_dual_positive(margin, pr.barrier, sl, du);
       }
       S.slack[o + j] = sl;
       S.dual[o + j] = du;
@@ -2458,11 +2458,10 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS) k_fb_init_distance(FbArra
   if (lane < FB_NC) {
     double P[3];
     fbw_contact_point(w, lane, P);
-    double sl = P[2];
-    int guard = 0;
-    while (sl < pr.barrier && guard < (1 << 20)) { sl += pr.barrier; ++guard; }
+    double sl, du;
+    pdipm_set_slack_and_dual_positive(P[2], pr.barrier, sl, du);
     S.slack[fbc_offset(FBC_DISTANCE) + lane] = sl;
-    S.dual[fbc_offset(FBC_DISTANCE) + lane] = pr.barrier / sl;
+    S.dual[fbc_offset(FBC_DISTANCE) + lane] = du;
   }
 }
 
@@ -2547,27 +2546,15 @@ __global__ void __launch_bounds__(32 * FB_LS_WARPS) k_fb_ls_eval(FbArrays A, FbL
         if (c == FBC_DISTANCE) {
           // violation of the contact distances: after the kinematics of the trial point, below
         } else if (fbc_is_cone(c)) {
-          const int rpc = fbc_cone_rows(nl, c);
-          const int i = rpc == 2 ? (j >> 1) : (j / 5);   // no division by a run-time value
+          int i, ee;
+          fbc_cone_row(nl, c, j, i, ee);
           if (el.active[i]) {
             double r5[5];
-            fb_friction_residual(pr.mu, rpc == 2, w.f + 3 * i, r5);
-            ar = fabs(r5[(rpc == 2 ? (j & 1) : (j % 5))] + w.slack[idx]);
+            fb_friction_residual(pr.mu, fbc_cone_rows(nl, c) == 2, w.f + 3 * i, r5);
+            ar = fabs(r5[ee] + w.slack[idx]);
           }
         } else {
-          const double sl = w.slack[idx];
-          double res;
-          switch (c) {
-            case FBC_ACC_LO: res = pr.a_min[j] - w.a[6 + j] + sl; break;
-            case FBC_ACC_UP: res = w.a[6 + j] - pr.a_max[j] + sl; break;
-            case FBC_POS_LO: res = pr.q_min[j] - w.q[7 + j] + sl; break;
-            case FBC_POS_UP: res = w.q[7 + j] - pr.q_max[j] + sl; break;
-            case FBC_VEL_LO: res = (-pr.v_max[j]) - w.v[6 + j] + sl; break;
-            case FBC_VEL_UP: res = w.v[6 + j] - pr.v_max[j] + sl; break;
-            case FBC_TRQ_LO: res = (-pr.u_max[j]) - w.u[j] + sl; break;
-            default:         res = w.u[j] - pr.u_max[j] + sl; break;
-          }
-          ar = fabs(res);
+          ar = fabs(w.slack[idx] - fbc_box_margin(c, j, pr, w.q, w.v, w.a, w.u));
         }
       }
       w.duality[idx] = lg;
@@ -2707,16 +2694,13 @@ __global__ void __launch_bounds__(32 * FB_LS_WARPS) k_fb_ls_eval(FbArrays A, FbL
   }
 }
 
-// totals in the reference's order: grid stages (with the terminal stage), impulse, aux, lift (line_search.hpp:174-182)
+// totals in the reference's order (line_search.hpp:174-182): one partial sum per pass
 __device__ inline void fb_ls_totals(const FbArrays& A, int b, double& cost, double& viol) {
   double c = 0.0, v = 0.0;
   for (int pass = 0; pass < 4; ++pass) {
     double cs = 0.0, vs = 0.0;
     for (int e = 0; e < A.n_elems; ++e) {
-      const int k = A.elems[e].kind;
-      const bool mine = (pass == 0 && (k == FB_GRID || k == FB_TERMINAL)) || (pass == 1 && k == FB_IMPULSE) ||
-                        (pass == 2 && k == FB_AUX) || (pass == 3 && k == FB_LIFT);
-      if (!mine) continue;
+      if (!fb_in_pass(A.elems[e].kind, pass)) continue;
       const FbDir& Dr = A.dir[(size_t)A.elems[e].slot * A.B + b];
       cs += Dr.ls_cost;
       vs += Dr.ls_viol;

@@ -18,6 +18,7 @@
 // local) and column l of every 7x7 block.  One warp = one GROUP of 4 instances (common.cuh).
 #pragma once
 #include "chain_dynamics.cuh"
+#include "pdipm.cuh"
 #include "task_space_cost.cuh"
 #include "tma.cuh"
 
@@ -61,14 +62,17 @@ __device__ __forceinline__ double con_margin(int comp, const LaneLimits& L, doub
     default: return L.umax - u;
   }
 }
+// slack / dual direction of joint-limit row comp for the primal direction (dq, dv, du) (e.g. joint_torques_upper_limit.cpp:75-80)
+__device__ __forceinline__ void con_direction(int comp, const LaneLimits& L, double q, double v, double u, double dq, double dv,
+                                              double du, double slack, double dual, double barrier, double& dslack, double& ddual) {
+  const double r = con_residual(comp, L, q, v, u, slack);
+  const double dty = slack * dual - barrier;
+  const double dx = comp < 2 ? dq : (comp < 4 ? dv : du);
+  dslack = ((comp & 1) ? -dx : dx) - r;
+  ddual = pdipm_dual_direction(slack, dual, dty, dslack);
+}
 __device__ __forceinline__ bool comp_active(int comp, int time_stage) {
   return comp < 2 ? pos_active(time_stage) : (comp < 4 ? vel_active(time_stage) : true);
-}
-// pdipm::FractionToBoundary (pdipm.hxx:52-73) for one row
-__device__ __forceinline__ double fraction_row(double rate, double x, double dx, double cur) {
-  const double f = -rate * (x / dx);
-  if (f > 0.0 && f < 1.0 && f < cur) return f;
-  return cur;
 }
 
 __device__ __forceinline__ LaneLimits load_limits(const DevProblem& P, int lane) {
@@ -98,12 +102,12 @@ __device__ __forceinline__ AccRows acc_load(const DevProblem& P, const Layout& L
 __device__ __forceinline__ double acc_residual(const AccRows& r, int k, double a, double slack) {
   return k == 0 ? r.lim[0] - a + slack : a - r.lim[1] + slack;
 }
-// slack / dual direction of row k for the acceleration direction da (joint_acceleration_lower_limit.cpp:72-77, pdipm.hxx:76-81)
+// slack / dual direction of row k for the acceleration direction da (joint_acceleration_lower_limit.cpp:72-77)
 __device__ __forceinline__ void acc_direction(const AccRows& r, int k, double a, double da, double barrier, double& dslack, double& ddual) {
   const double res = acc_residual(r, k, a, r.sl[k]);
   const double dty = r.sl[k] * r.du[k] - barrier;
   dslack = (k ? -da : da) - res;
-  ddual = -fma(r.du[k], dslack, dty) / r.sl[k];
+  ddual = pdipm_dual_direction(r.sl[k], r.du[k], dty, dslack);
 }
 
 // warp-task decomposition of the per-stage kernels: task = (stage, group)
@@ -118,8 +122,7 @@ __device__ __forceinline__ StageTask stage_task(const Layout& L, int nstages) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// k_init_constraints: slack = margin (pushed above the barrier), dual = barrier / slack
-// (pdipm::SetSlackAndDualPositive, pdipm.hxx:13-23)
+// k_init_constraints: slack and dual of every live row from its margin
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(CTA_THREADS) k_init_constraints(const DevProblem* __restrict__ Pp, Layout L,
                                                                   int stage_offset) {
@@ -132,12 +135,8 @@ __global__ void __launch_bounds__(CTA_THREADS) k_init_constraints(const DevProbl
 #pragma unroll
   for (int c = 0; c < NC; ++c) {
     double sl = 0.0, du = 0.0;
-    if (comp_active(c, t.stage + stage_offset) && lane < NV) {
-      sl = con_margin(c, lim, q, v, u);
-      int guard = 0;
-      while (sl < P.barrier && guard < (1 << 20)) { sl += P.barrier; ++guard; }
-      du = P.barrier / sl;
-    }
+    if (comp_active(c, t.stage + stage_offset) && lane < NV)
+      pdipm_set_slack_and_dual_positive(con_margin(c, lim, q, v, u), P.barrier, sl, du);
     X[(X_SLACK + c) * SLOT] = sl;
     X[(X_DUAL + c) * SLOT] = du;
   }
@@ -147,12 +146,8 @@ __global__ void __launch_bounds__(CTA_THREADS) k_init_constraints(const DevProbl
 #pragma unroll
     for (int k = 0; k < 2; ++k) {
       double sl = 0.0, du = 0.0;
-      if (P.acc_enable[k] && lane < NV) {
-        sl = k == 0 ? a - P.a_min[lane] : P.a_max[lane] - a;
-        int guard = 0;
-        while (sl < P.barrier && guard < (1 << 20)) { sl += P.barrier; ++guard; }
-        du = P.barrier / sl;
-      }
+      if (P.acc_enable[k] && lane < NV)
+        pdipm_set_slack_and_dual_positive(k == 0 ? a - P.a_min[lane] : P.a_max[lane] - a, P.barrier, sl, du);
       XA[k * SLOT] = sl;
       XA[(2 + k) * SLOT] = du;
     }
@@ -245,11 +240,8 @@ __device__ __forceinline__ void linearize_task(const DevProblem& P, const Layout
         for (int c = 0; c < NC; ++c) {
           if (!comp_active(c, i)) continue;
           const double sl = fslack[c], dl = fdual[c];
-          const double r = con_residual(c, lim, q_old, v_old, u_old, sl);
-          const double dty = sl * dl - P.barrier;
-          const double dx = c < 2 ? dq : (c < 4 ? dv : du);
-          const double dslack = ((c & 1) ? -dx : dx) - r;
-          const double ddual = -fma(dl, dslack, dty) / sl;
+          double dslack, ddual;
+          con_direction(c, lim, q_old, v_old, u_old, dq, dv, du, sl, dl, P.barrier, dslack, ddual);
           fslack[c] = fma(ap, dslack, sl);
           fdual[c] = fma(ad, ddual, dl);
         }
@@ -483,9 +475,8 @@ __device__ __forceinline__ void linearize_task(const DevProblem& P, const Layout
       if (!comp_active(c, ts)) continue;
       const double r = con_residual(c, lim, q, v, u, slack[c]);
       const double dl = slack[c] * dual[c] - P.barrier;
-      const double rs = 1.0 / slack[c];
-      const double h = (dt * dual[c]) * rs;
-      const double g = (dt * fma(dual[c], r, -dl)) * rs;
+      double h, g;
+      pdipm_condense(dt, slack[c], dual[c], r, dl, h, g);
       const double sg = (c & 1) ? g : -g;
       if (c < 2) { Qqq_d += h; lq += sg; }
       else if (c < 4) { Qvv_d += h; lv += sg; }
@@ -497,9 +488,9 @@ __device__ __forceinline__ void linearize_task(const DevProblem& P, const Layout
         if (!acc.on[k]) continue;
         const double r = acc_residual(acc, k, a, acc.sl[k]);
         const double dl = acc.sl[k] * acc.du[k] - P.barrier;
-        const double rs = 1.0 / acc.sl[k];
-        Qaa_d += (dt * acc.du[k]) * rs;
-        const double g2 = (dt * fma(acc.du[k], r, -dl)) * rs;
+        double h2, g2;
+        pdipm_condense(dt, acc.sl[k], acc.du[k], r, dl, h2, g2);
+        Qaa_d += h2;
         la += k ? g2 : -g2;
       }
     }
@@ -1193,13 +1184,10 @@ __global__ void __launch_bounds__(CTA_THREADS, EXP_MINB) k_expand(const DevProbl
       if (!comp_active(c, i + stage_offset)) continue;
       const double sl = slk[c];
       const double dl = dul[c];
-      const double r = con_residual(c, lim, q, v, u, sl);
-      const double dty = sl * dl - P.barrier;
-      const double dx = c < 2 ? dq : (c < 4 ? dv : du);
-      const double dslack = ((c & 1) ? -dx : dx) - r;
-      const double ddual = -fma(dl, dslack, dty) / sl;
-      min_p = fraction_row(P.fraction_rate, sl, dslack, min_p);
-      min_d = fraction_row(P.fraction_rate, dl, ddual, min_d);
+      double dslack, ddual;
+      con_direction(c, lim, q, v, u, dq, dv, du, sl, dl, P.barrier, dslack, ddual);
+      min_p = pdipm_fraction_row(P.fraction_rate, sl, dslack, min_p);
+      min_d = pdipm_fraction_row(P.fraction_rate, dl, ddual, min_d);
     }
     if (ACC) {
 #pragma unroll
@@ -1207,8 +1195,8 @@ __global__ void __launch_bounds__(CTA_THREADS, EXP_MINB) k_expand(const DevProbl
         if (!acc.on[k]) continue;
         double dslack, ddual;
         acc_direction(acc, k, xa, da, P.barrier, dslack, ddual);
-        min_p = fraction_row(P.fraction_rate, acc.sl[k], dslack, min_p);
-        min_d = fraction_row(P.fraction_rate, acc.du[k], ddual, min_d);
+        min_p = pdipm_fraction_row(P.fraction_rate, acc.sl[k], dslack, min_p);
+        min_d = pdipm_fraction_row(P.fraction_rate, acc.du[k], ddual, min_d);
       }
     }
   }
@@ -1285,11 +1273,8 @@ __global__ void __launch_bounds__(CTA_THREADS) k_update(const DevProblem* __rest
   for (int c = 0; c < NC; ++c) {
     if (!comp_active(c, i + stage_offset)) continue;
     const double sl = slk[c], dl = dul[c];
-    const double r = con_residual(c, lim, q, v, u, sl);
-    const double dty = sl * dl - P.barrier;
-    const double dx = c < 2 ? dq : (c < 4 ? dv : du);
-    const double dslack = ((c & 1) ? -dx : dx) - r;
-    const double ddual = -fma(dl, dslack, dty) / sl;
+    double dslack, ddual;
+    con_direction(c, lim, q, v, u, dq, dv, du, sl, dl, P.barrier, dslack, ddual);
     X[(X_SLACK + c) * SLOT] = fma(ap, dslack, sl);
     X[(X_DUAL + c) * SLOT] = fma(ad, ddual, dl);
   }
