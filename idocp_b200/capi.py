@@ -103,7 +103,8 @@ EXPORTS = [
     "idocp_b200_get_direction", "idocp_b200_get_constraint_data", "idocp_b200_get_step_sizes",
     "idocp_b200_get_unkkt", "idocp_b200_check_cost_derivatives", "idocp_b200_get_status", "idocp_b200_is_feasible",
     "idocp_b200_clear_line_search_filter", "idocp_b200_sync", "idocp_b200_launch_count", "idocp_b200_stream",
-    "idocp_b200_set_task_reference", "idocp_b200_set_profiling", "idocp_b200_get_profile", "idocp_b200_set_pipelining",
+    "idocp_b200_set_task_reference", "idocp_b200_set_instance_reference", "idocp_b200_set_instance_task_reference",
+    "idocp_b200_clear_instance_references", "idocp_b200_set_profiling", "idocp_b200_get_profile", "idocp_b200_set_pipelining",
     "idocp_b200_contact_sequence_create", "idocp_b200_contact_sequence_destroy",
     "idocp_b200_contact_sequence_set_uniform", "idocp_b200_contact_sequence_push_back",
     "idocp_b200_contact_sequence_pop_back", "idocp_b200_contact_sequence_pop_front",
@@ -126,7 +127,8 @@ EXPORTS = [
     "idocp_b200_fb_sharded_sync", "idocp_b200_fb_sharded_launch_count",
     "idocp_b200_create_sharded", "idocp_b200_sharded_destroy", "idocp_b200_sharded_num_shards", "idocp_b200_sharded_shard",
     "idocp_b200_sharded_set_solution", "idocp_b200_sharded_init_constraints", "idocp_b200_sharded_init_backward_correction",
-    "idocp_b200_sharded_set_task_reference", "idocp_b200_sharded_update_solution", "idocp_b200_sharded_compute_kkt_residual",
+    "idocp_b200_sharded_set_task_reference", "idocp_b200_sharded_set_instance_reference",
+    "idocp_b200_sharded_set_instance_task_reference", "idocp_b200_sharded_clear_instance_references", "idocp_b200_sharded_update_solution", "idocp_b200_sharded_compute_kkt_residual",
     "idocp_b200_sharded_kkt_error", "idocp_b200_sharded_get_solution", "idocp_b200_sharded_get_stage_solution",
     "idocp_b200_sharded_get_step_sizes", "idocp_b200_sharded_get_status", "idocp_b200_sharded_clear_line_search_filter",
     "idocp_b200_sharded_sync",
@@ -169,6 +171,9 @@ class Library:
         L.idocp_b200_clear_line_search_filter.argtypes = [C.c_void_p]
         L.idocp_b200_sync.argtypes = [C.c_void_p]
         L.idocp_b200_set_task_reference.argtypes = [C.c_void_p, _dp]
+        L.idocp_b200_set_instance_reference.argtypes = [C.c_void_p, C.c_char_p, _dp]
+        L.idocp_b200_set_instance_task_reference.argtypes = [C.c_void_p, _dp]
+        L.idocp_b200_clear_instance_references.argtypes = [C.c_void_p]
         L.idocp_b200_contact_sequence_create.argtypes = [C.c_int, C.c_int, C.POINTER(C.c_void_p)]
         L.idocp_b200_contact_sequence_destroy.argtypes = [C.c_void_p]
         L.idocp_b200_contact_sequence_set_uniform.argtypes = [C.c_void_p, _ip, _dp]
@@ -217,8 +222,8 @@ class Library:
         L.idocp_b200_fb_total_weight.restype = C.c_double
         L.idocp_b200_fb_contact_frame_positions.argtypes = [_dp, _dp]
         L.idocp_b200_create_sharded.argtypes = [C.POINTER(Problem), C.c_int, C.c_int, _ip, C.c_int, C.POINTER(C.c_void_p)]
-        for name in ("set_solution", "init_constraints", "init_backward_correction", "set_task_reference", "update_solution",
-                     "compute_kkt_residual", "kkt_error", "get_solution", "get_stage_solution", "get_step_sizes", "get_status",
+        for name in ("set_solution", "init_constraints", "init_backward_correction", "set_task_reference", "set_instance_reference",
+                     "set_instance_task_reference", "clear_instance_references", "update_solution", "compute_kkt_residual", "kkt_error", "get_solution", "get_stage_solution", "get_step_sizes", "get_status",
                      "clear_line_search_filter", "sync"):
             getattr(L, "idocp_b200_sharded_" + name).argtypes = getattr(L, "idocp_b200_" + name).argtypes
         for family in ("", "fb_"):

@@ -14,6 +14,7 @@
 #include <cstdio>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/idocp_b200.h"
@@ -53,6 +54,13 @@ static int fail(int code, const std::string& msg) {
     if (e_ != cudaSuccess)                                                                   \
       return fail(IDOCP_B200_CUDA_ERROR, std::string(#expr) + ": " + cudaGetErrorString(e_)); \
   } while (0)
+
+// f(std::true_type) if `flag` else f(std::false_type): turns a run-time problem flag into a kernel template argument
+template <typename F>
+static void with_flag(bool flag, F f) {
+  if (flag) f(std::true_type());
+  else f(std::false_type());
+}
 
 enum KernelClass { KC_LINEARIZE = 0, KC_RICCATI, KC_EXPAND, KC_UPDATE, KC_KKT, KC_MISC, KC_PARNMPC_COARSE,
                    KC_PARNMPC_CORR, KC_LINESEARCH, KC_FB_LINEARIZE, KC_FB_CONDENSE, KC_FB_RICCATI, KC_FB_FORWARD, KC_FB_EXPAND, KC_FB_UPDATE,
@@ -251,8 +259,14 @@ struct idocp_b200_solver : DeviceHandle {
   bool kkt_tracking = false;
   bool kkt_valid = false;
   int sm_count = 1;            // persistent kernels launch one CTA pair per SM
+  // per-instance cost references (idocp_b200_set_instance_reference / _task_reference): L.iref / L.itask point at these
+  // allocations while the mode is on (nullptr in shared mode); the allocations outlive a clear for the next set
+  double* d_iref = nullptr;
+  double* d_itask = nullptr;
+  std::vector<double> iref_host;   // [B][IREF_NUM][7]: the configuration references of every instance in the caller's layout
 
   int stage_offset() const { return kind == IDOCP_B200_SOLVER_UNPARNMPC ? 1 : 0; }
+  bool iref() const { return L.iref || L.itask; }   // kernels: the IREF instantiations
 };
 
 extern "C" const char* idocp_b200_last_error(void) { return g_last_error.c_str(); }
@@ -407,10 +421,14 @@ extern "C" int idocp_b200_create(const idocp_b200_problem* p, int solver_kind, i
   rc |= h->alloc(&h->d_stage, h->stage_doubles);
   if (cudaFuncSetAttribute(k_riccati<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kRicSmem) != cudaSuccess) rc |= -1;
   if (cudaFuncSetAttribute(k_riccati<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kRicSmem) != cudaSuccess) rc |= -1;
-  if (cudaFuncSetAttribute(k_update_linearize<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kUlSmem) != cudaSuccess) rc |= -1;
-  if (cudaFuncSetAttribute(k_update_linearize<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kUlSmem) != cudaSuccess) rc |= -1;
-  if (cudaFuncSetAttribute(k_update_linearize<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kUlSmem) != cudaSuccess) rc |= -1;
-  if (cudaFuncSetAttribute(k_update_linearize<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kUlSmem) != cudaSuccess) rc |= -1;
+  for (int task = 0; task < 2; ++task)
+    for (int kkt = 0; kkt < 2; ++kkt)
+      for (int iref = 0; iref < 2; ++iref)
+        with_flag(task, [&](auto T) { with_flag(kkt, [&](auto K) { with_flag(iref, [&](auto IR) {
+          if (cudaFuncSetAttribute(k_update_linearize<decltype(T)::value, decltype(K)::value, decltype(IR)::value>,
+                                   cudaFuncAttributeMaxDynamicSharedMemorySize, kUlSmem) != cudaSuccess)
+            rc |= -1;
+        }); }); });
   {
     int dev = 0, sms = 0;
     if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && sms > 0)
@@ -549,17 +567,10 @@ static int run_line_search(idocp_b200_solver* h, const double* d_q, const double
   IDOCP_LAUNCH(h, KC_LINESEARCH, k_ls_begin, group_grid(h), CTA_THREADS, 0, h->L);
   auto eval = [&](int mode) {
     const int grid = stage_grid(h, ncost);
-    if (par) {
-      if (task)
-        IDOCP_LAUNCH(h, KC_LINESEARCH, (k_ls_eval<true, true>), grid, CTA_THREADS, 0, h->d_prob, h->L, h->LS, mode, off, d_q, d_v);
-      else
-        IDOCP_LAUNCH(h, KC_LINESEARCH, (k_ls_eval<false, true>), grid, CTA_THREADS, 0, h->d_prob, h->L, h->LS, mode, off, d_q, d_v);
-    } else {
-      if (task)
-        IDOCP_LAUNCH(h, KC_LINESEARCH, (k_ls_eval<true, false>), grid, CTA_THREADS, 0, h->d_prob, h->L, h->LS, mode, off, d_q, d_v);
-      else
-        IDOCP_LAUNCH(h, KC_LINESEARCH, (k_ls_eval<false, false>), grid, CTA_THREADS, 0, h->d_prob, h->L, h->LS, mode, off, d_q, d_v);
-    }
+    with_flag(task, [&](auto T) { with_flag(par, [&](auto PAR) { with_flag(h->iref(), [&](auto IR) {
+      IDOCP_LAUNCH(h, KC_LINESEARCH, (k_ls_eval<decltype(T)::value, decltype(PAR)::value, decltype(IR)::value>), grid, CTA_THREADS, 0,
+                   h->d_prob, h->L, h->LS, mode, off, d_q, d_v);
+    }); }); });
   };
   enqueue_line_search_rounds(eval, [&](int mode) {
     IDOCP_LAUNCH(h, KC_LINESEARCH, k_ls_filter, fgrid, 128, 0, h->L, h->LS, mode, ncost);
@@ -568,28 +579,38 @@ static int run_line_search(idocp_b200_solver* h, const double* d_q, const double
   return IDOCP_B200_OK;
 }
 
-// k_linearize / k_expand instantiation by the run-time problem flags (task-space cost, acceleration limits)
+// k_linearize / k_expand instantiation by the run-time problem flags (task-space cost, acceleration limits, per-instance references)
 template <bool RES, bool BE>
 static void launch_linearize(idocp_b200_solver* h, int cls, int nstages, const double* d_q, const double* d_v) {
-  const bool task = h->prob.task_enabled != 0, acc = h->L.XA != nullptr;
   const int grid = stage_grid(h, nstages);
-  if (task && acc) IDOCP_LAUNCH(h, cls, (k_linearize<RES, BE, true, true>), grid, CTA_THREADS, kLinSmem, h->d_prob, h->L, d_q, d_v);
-  else if (task) IDOCP_LAUNCH(h, cls, (k_linearize<RES, BE, true, false>), grid, CTA_THREADS, kLinSmem, h->d_prob, h->L, d_q, d_v);
-  else if (acc) IDOCP_LAUNCH(h, cls, (k_linearize<RES, BE, false, true>), grid, CTA_THREADS, kLinSmem, h->d_prob, h->L, d_q, d_v);
-  else IDOCP_LAUNCH(h, cls, (k_linearize<RES, BE, false, false>), grid, CTA_THREADS, kLinSmem, h->d_prob, h->L, d_q, d_v);
+  with_flag(h->prob.task_enabled != 0, [&](auto task) { with_flag(h->L.XA != nullptr, [&](auto acc) { with_flag(h->iref(), [&](auto iref) {
+    IDOCP_LAUNCH(h, cls, (k_linearize<RES, BE, decltype(task)::value, decltype(acc)::value, decltype(iref)::value>), grid, CTA_THREADS,
+                 kLinSmem, h->d_prob, h->L, d_q, d_v);
+  }); }); });
 }
 template <bool PARNMPC>
 static void launch_expand(idocp_b200_solver* h, int nstages, int stage_offset) {
-  const bool task = !PARNMPC && h->prob.task_enabled != 0, acc = h->L.XA != nullptr;
+  // UnParNMPCSolver has no terminal stage, the only place k_expand reads a reference
   const int grid = stage_grid(h, nstages);
-  if (task && acc) IDOCP_LAUNCH(h, KC_EXPAND, (k_expand<PARNMPC, !PARNMPC, true>), grid, CTA_THREADS, 0, h->d_prob, h->L, stage_offset);
-  else if (task) IDOCP_LAUNCH(h, KC_EXPAND, (k_expand<PARNMPC, !PARNMPC, false>), grid, CTA_THREADS, 0, h->d_prob, h->L, stage_offset);
-  else if (acc) IDOCP_LAUNCH(h, KC_EXPAND, (k_expand<PARNMPC, false, true>), grid, CTA_THREADS, 0, h->d_prob, h->L, stage_offset);
-  else IDOCP_LAUNCH(h, KC_EXPAND, (k_expand<PARNMPC, false, false>), grid, CTA_THREADS, 0, h->d_prob, h->L, stage_offset);
+  with_flag(!PARNMPC && h->prob.task_enabled != 0, [&](auto task) { with_flag(h->L.XA != nullptr, [&](auto acc) {
+    with_flag(!PARNMPC && h->iref(), [&](auto iref) {
+      IDOCP_LAUNCH(h, KC_EXPAND, (k_expand<PARNMPC, decltype(task)::value, decltype(acc)::value, decltype(iref)::value>), grid,
+                   CTA_THREADS, 0, h->d_prob, h->L, stage_offset);
+    });
+  }); });
+}
+
+// the persistent update + linearisation (k_update_linearize) of the run-time flags
+static void launch_update_linearize(idocp_b200_solver* h, int grid) {
+  with_flag(h->prob.task_enabled != 0, [&](auto task) { with_flag(h->kkt_tracking, [&](auto kkt) { with_flag(h->iref(), [&](auto iref) {
+    IDOCP_LAUNCH(h, KC_UPDATE_LINEARIZE, (k_update_linearize<decltype(task)::value, decltype(kkt)::value, decltype(iref)::value>), grid,
+                 UL_THREADS, kUlSmem, h->d_prob, h->L);
+  }); }); });
 }
 
 static int unocp_update(idocp_b200_solver* h, const double* d_q, const double* d_v, int line_search) {
-  const bool task = h->prob.task_enabled != 0;
+  // the terminal blocks come from record N of KQ with a task-space cost or per-instance references (k_riccati<true>)
+  const bool task = h->prob.task_enabled != 0 || h->iref();
   if (!(h->pipelined && h->lin_valid)) {
     launch_linearize<false, false>(h, KC_LINEARIZE, task ? h->N + 1 : h->N, d_q, d_v);
   }
@@ -612,14 +633,7 @@ static int unocp_update(idocp_b200_solver* h, const double* d_q, const double* d
     IDOCP_LAUNCH(h, KC_STEP_MIN, k_step_min, (h->Bp + 127) / 128, 128, 0, h->L, override_alpha);
     const long ul_tasks = static_cast<long>(h->N + 1) * h->L.G;
     const int ul_grid = static_cast<int>(std::min<long>((ul_tasks + UL_WARPS - 1) / UL_WARPS, static_cast<long>(UL_CTAS_PER_SM) * h->sm_count));
-    if (task && h->kkt_tracking)
-      IDOCP_LAUNCH(h, KC_UPDATE_LINEARIZE, (k_update_linearize<true, true>), ul_grid, UL_THREADS, kUlSmem, h->d_prob, h->L);
-    else if (task)
-      IDOCP_LAUNCH(h, KC_UPDATE_LINEARIZE, (k_update_linearize<true, false>), ul_grid, UL_THREADS, kUlSmem, h->d_prob, h->L);
-    else if (h->kkt_tracking)
-      IDOCP_LAUNCH(h, KC_UPDATE_LINEARIZE, (k_update_linearize<false, true>), ul_grid, UL_THREADS, kUlSmem, h->d_prob, h->L);
-    else
-      IDOCP_LAUNCH(h, KC_UPDATE_LINEARIZE, (k_update_linearize<false, false>), ul_grid, UL_THREADS, kUlSmem, h->d_prob, h->L);
+    launch_update_linearize(h, ul_grid);
     std::swap(h->L.X, h->L.X2);
     h->lin_valid = true;
     h->kkt_valid = h->kkt_tracking;
@@ -666,7 +680,9 @@ static int parnmpc_kkt_residual(idocp_b200_solver* h, double, const double* d_q,
 
 // UnParNMPCSolver::initBackwardCorrection (src/unocp/unparnmpc_solver.cpp:69-71)
 static int parnmpc_init_backward_correction(idocp_b200_solver* h, double) {
-  if (h->prob.task_enabled)
+  if (h->prob.task_enabled && h->L.itask)
+    IDOCP_LAUNCH(h, KC_MISC, (k_parnmpc_init_aux<true, true>), stage_grid(h, h->N), CTA_THREADS, kLinSmem, h->d_prob, h->L, h->PL);
+  else if (h->prob.task_enabled)
     IDOCP_LAUNCH(h, KC_MISC, k_parnmpc_init_aux<true>, stage_grid(h, h->N), CTA_THREADS, kLinSmem, h->d_prob, h->L, h->PL);
   else
     IDOCP_LAUNCH(h, KC_MISC, k_parnmpc_init_aux<false>, stage_grid(h, h->N), CTA_THREADS, kLinSmem, h->d_prob, h->L,
@@ -892,6 +908,69 @@ extern "C" int idocp_b200_set_task_reference(idocp_b200_solver* h, const double*
   CUDA_OK(cudaSetDevice(h->device));
   h->lin_valid = false; h->kkt_valid = false;                       // the kept linearisation used the old reference
   return h->upload(h->L.task_ref, table, static_cast<size_t>(h->N + 1) * 12 * sizeof(double));
+}
+
+// Per-instance cost references.  Every set / clear invalidates the kept linearisation (it was made with the old references);
+// the line-search filter is left as it is, as on a change of the shared references.  Padded instances (B <= b < Bp) repeat
+// the last instance: they are computed but never reported.
+extern "C" int idocp_b200_set_instance_reference(idocp_b200_solver* h, const char* name, const double* value) {
+  if (!h || !name || !value) return fail(IDOCP_B200_INVALID_ARGUMENT, "set_instance_reference: null pointer");
+  const int field = !std::strcmp(name, "q_ref") ? IREF_Q : !std::strcmp(name, "v_ref") ? IREF_V : !std::strcmp(name, "u_ref") ? IREF_U : -1;
+  if (field < 0) return fail(IDOCP_B200_INVALID_ARGUMENT, "invalid argument: name must be q_ref, v_ref, or u_ref!");
+  CUDA_OK(cudaSetDevice(h->device));
+  const size_t B = h->B, Bp = h->Bp, G = h->L.G;
+  if (!h->d_iref && h->alloc(&h->d_iref, G * IREF_NUM * SLOT) != 0)
+    return fail(IDOCP_B200_CUDA_ERROR, "set_instance_reference: device memory allocation failed");
+  if (!h->L.iref) {   // entering per-instance mode: the fields not set yet start as copies of the problem's
+    h->iref_host.assign(B * IREF_NUM * NV, 0.0);
+    for (size_t b = 0; b < B; ++b)
+      for (int j = 0; j < NV; ++j) {
+        h->iref_host[(b * IREF_NUM + IREF_Q) * NV + j] = h->prob.q_ref[j];
+        h->iref_host[(b * IREF_NUM + IREF_V) * NV + j] = h->prob.v_ref[j];
+        h->iref_host[(b * IREF_NUM + IREF_U) * NV + j] = h->prob.u_ref[j];
+      }
+  }
+  for (size_t b = 0; b < B; ++b)
+    for (int j = 0; j < NV; ++j) h->iref_host[(b * IREF_NUM + field) * NV + j] = value[b * NV + j];
+  // [b][field][j] -> [group][field][b & 3][lane], padding lane 7 zero as DevProblem's
+  std::vector<double> dev(G * IREF_NUM * SLOT, 0.0);
+  for (size_t b = 0; b < Bp; ++b)
+    for (int f = 0; f < IREF_NUM; ++f)
+      for (int j = 0; j < NV; ++j)
+        dev[elem_index(IREF_NUM, static_cast<int>(G), 0, static_cast<int>(b), f, j)] = h->iref_host[((b < B ? b : B - 1) * IREF_NUM + f) * NV + j];
+  const int rc = h->upload(h->d_iref, dev.data(), dev.size() * sizeof(double));
+  if (rc != IDOCP_B200_OK) return rc;
+  h->L.iref = h->d_iref;
+  h->lin_valid = false; h->kkt_valid = false;
+  return IDOCP_B200_OK;
+}
+
+extern "C" int idocp_b200_set_instance_task_reference(idocp_b200_solver* h, const double* table) {
+  if (!h || !table) return fail(IDOCP_B200_INVALID_ARGUMENT, "set_instance_task_reference: null pointer");
+  if (!h->prob.task_enabled)
+    return fail(IDOCP_B200_INVALID_ARGUMENT, "invalid argument: set_instance_task_reference needs a task-space cost (task_enabled == 0)!");
+  CUDA_OK(cudaSetDevice(h->device));
+  const size_t B = h->B, Bp = h->Bp, rows = static_cast<size_t>(h->N) + 1;
+  if (!h->d_itask && h->alloc(&h->d_itask, rows * Bp * 12) != 0)
+    return fail(IDOCP_B200_CUDA_ERROR, "set_instance_task_reference: device memory allocation failed");
+  // [b][row][12] -> [row][b][12]: the four instances of a (stage, group) task are 48 contiguous doubles
+  std::vector<double> dev(rows * Bp * 12);
+  for (size_t i = 0; i < rows; ++i)
+    for (size_t b = 0; b < Bp; ++b)
+      std::memcpy(&dev[(i * Bp + b) * 12], table + ((b < B ? b : B - 1) * rows + i) * 12, 12 * sizeof(double));
+  const int rc = h->upload(h->d_itask, dev.data(), dev.size() * sizeof(double));
+  if (rc != IDOCP_B200_OK) return rc;
+  h->L.itask = h->d_itask;
+  h->lin_valid = false; h->kkt_valid = false;
+  return IDOCP_B200_OK;
+}
+
+extern "C" int idocp_b200_clear_instance_references(idocp_b200_solver* h) {
+  if (!h) return fail(IDOCP_B200_INVALID_ARGUMENT, "null handle");
+  h->L.iref = nullptr;
+  h->L.itask = nullptr;
+  h->lin_valid = false; h->kkt_valid = false;
+  return IDOCP_B200_OK;
 }
 
 // UnOCPSolver pipelining (default on): see k_linearize<.., FUSED>.  Off: linearise, solve, expand, update as four launches;

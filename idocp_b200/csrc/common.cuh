@@ -80,8 +80,27 @@ struct Layout {
   double* task_ref;   // [N+1][12] host-sampled SE3 reference per stage index (R row-major, p); see capi.cu
   double* XA;         // [N][G][XA_NUM slots]: slack (lower, upper), dual (lower, upper) of the two acceleration-limit components;
                       // nullptr unless one of them is enabled (the X record and the hot kernels stay as they are otherwise)
+  // per-instance cost references (idocp_b200_set_instance_reference / _task_reference); nullptr in shared mode, where the
+  // kernels read DevProblem::q_ref / v_ref / u_ref and task_ref.  Read only by the IREF kernel instantiations.
+  double* iref;       // [G][IREF_NUM slots]: q_ref, v_ref, u_ref of every instance in the slot layout of X
+  double* itask;      // [N+1][Bp][12]: task-space reference of every (stage row, instance), rows as task_ref
 };
 constexpr int XA_NUM = 4;
+enum IrefSlot { IREF_Q = 0, IREF_V, IREF_U, IREF_NUM };
+
+// The ConfigurationSpaceCost reference (slot IREF_Q / _V / _U) of this lane's joint in instance group g: the instance's own
+// in per-instance mode (IREF and L.iref set), the problem's otherwise
+template <bool IREF, int FIELD>
+__device__ __forceinline__ double cfg_ref(const DevProblem& P, const Layout& L, int g, int lane) {
+  if (IREF && L.iref) return L.iref[(static_cast<size_t>(g) * IREF_NUM + FIELD) * SLOT + (threadIdx.x & 31)];
+  return FIELD == IREF_Q ? P.q_ref[lane] : (FIELD == IREF_V ? P.v_ref[lane] : P.u_ref[lane]);
+}
+// row `row` of the task-space reference table of instance b: its own table (IREF and L.itask set) or the shared one
+template <bool IREF>
+__device__ __forceinline__ const double* task_ref_row(const Layout& L, int row, int b) {
+  if (IREF && L.itask) return L.itask + (static_cast<size_t>(row) * L.Bp + b) * 12;
+  return L.task_ref + static_cast<size_t>(row) * 12;
+}
 
 // element index of (stage, instance b, slot, joint j) in an array with `ns` slots per record
 __host__ __device__ __forceinline__ size_t elem_index(int ns, int G, int stage, int b, int slot, int j) {

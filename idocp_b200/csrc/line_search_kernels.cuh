@@ -45,7 +45,8 @@ __device__ __forceinline__ bool ls_participates(const LineSearchLayout& LS, int 
 // BACKWARD_EULER = true: UnParNMPCSolver (src/line_search/unline_search.cpp:87-122; split_unparnmpc.hxx:177-224,
 // terminal_unparnmpc.hxx:196-227): N stages, the last one adds the terminal cost, the state-equation defect
 // uses the TRIAL previous stage (x0 for index 0), the last stage's reference time is t + N dt (table row N)
-template <bool TASK, bool BACKWARD_EULER>
+// IREF = true: the instance's cost references (common.cuh: cfg_ref, task_ref_row)
+template <bool TASK, bool BACKWARD_EULER, bool IREF = false>
 __global__ void __launch_bounds__(CTA_THREADS) k_ls_eval(const DevProblem* __restrict__ Pp, Layout L,
                                                          LineSearchLayout LS, int mode, int stage_offset,
                                                          const double* __restrict__ q0, const double* __restrict__ v0) {
@@ -70,15 +71,15 @@ __global__ void __launch_bounds__(CTA_THREADS) k_ls_eval(const DevProblem* __res
   if (!BACKWARD_EULER && i == N) {
     // TerminalOCP::terminalCost -> ConfigurationSpaceCost::computeTerminalCost (configuration_space_cost.cpp:259-273)
     double l = 0.0;
-    l += oct_sum_ordered(z * (P.qf_weight[lane] * (qt - P.q_ref[lane]) * (qt - P.q_ref[lane])));
-    l += oct_sum_ordered(z * (P.vf_weight[lane] * (vt - P.v_ref[lane]) * (vt - P.v_ref[lane])));
+    l += oct_sum_ordered(z * (P.qf_weight[lane] * (qt - cfg_ref<IREF, IREF_Q>(P, L, t.g, lane)) * (qt - cfg_ref<IREF, IREF_Q>(P, L, t.g, lane))));
+    l += oct_sum_ordered(z * (P.vf_weight[lane] * (vt - cfg_ref<IREF, IREF_V>(P, L, t.g, lane)) * (vt - cfg_ref<IREF, IREF_V>(P, L, t.g, lane))));
     double tc = 0.5 * l;
     if (TASK) {
       double R[9];
       V3 p;
       chain_fk(lane, act ? qt : 0.0, P.model + lane * MODEL_STRIDE, R, p);
       TaskEval te;
-      task_evaluate<false>(R, p, P.ee, L.task_ref + static_cast<size_t>(N) * 12, te, P.task_enabled);
+      task_evaluate<false>(R, p, P.ee, task_ref_row<IREF>(L, N, b), te, P.task_enabled);
       tc += 0.5 * task_weighted_sqnorm(te, P.task_wf6);
     }
     if (lane == 0 && part) LS.cost[static_cast<size_t>(N) * L.Bp + b] = tc;
@@ -105,23 +106,23 @@ __global__ void __launch_bounds__(CTA_THREADS) k_ls_eval(const DevProblem* __res
   }
   // ---- SplitUnOCP::stageCost (split_unocp.hxx:177-196) ----
   double l = 0.0;
-  l += oct_sum_ordered(z * (P.q_weight[lane] * (qt - P.q_ref[lane]) * (qt - P.q_ref[lane])));
-  l += oct_sum_ordered(z * (P.v_weight[lane] * (vt - P.v_ref[lane]) * (vt - P.v_ref[lane])));
+  l += oct_sum_ordered(z * (P.q_weight[lane] * (qt - cfg_ref<IREF, IREF_Q>(P, L, t.g, lane)) * (qt - cfg_ref<IREF, IREF_Q>(P, L, t.g, lane))));
+  l += oct_sum_ordered(z * (P.v_weight[lane] * (vt - cfg_ref<IREF, IREF_V>(P, L, t.g, lane)) * (vt - cfg_ref<IREF, IREF_V>(P, L, t.g, lane))));
   l += oct_sum_ordered(z * (P.a_weight[lane] * at * at));
-  l += oct_sum_ordered(z * (P.u_weight[lane] * (ut - P.u_ref[lane]) * (ut - P.u_ref[lane])));
+  l += oct_sum_ordered(z * (P.u_weight[lane] * (ut - cfg_ref<IREF, IREF_U>(P, L, t.g, lane)) * (ut - cfg_ref<IREF, IREF_U>(P, L, t.g, lane))));
   double cost = 0.5 * dt * l;
   double R[9];
   V3 p;
   chain_fk(lane, act ? qt : 0.0, P.model + lane * MODEL_STRIDE, R, p);
   TaskEval te;
   if (TASK) {
-    task_evaluate<false>(R, p, P.ee, L.task_ref + static_cast<size_t>(last ? N : i) * 12, te, P.task_enabled);
+    task_evaluate<false>(R, p, P.ee, task_ref_row<IREF>(L, last ? N : i, b), te, P.task_enabled);
     cost += 0.5 * dt * task_weighted_sqnorm(te, P.task_w6);
   }
   if (last) {   // TerminalUnParNMPC::stageCost: + computeTerminalCost
     double lf = 0.0;
-    lf += oct_sum_ordered(z * (P.qf_weight[lane] * (qt - P.q_ref[lane]) * (qt - P.q_ref[lane])));
-    lf += oct_sum_ordered(z * (P.vf_weight[lane] * (vt - P.v_ref[lane]) * (vt - P.v_ref[lane])));
+    lf += oct_sum_ordered(z * (P.qf_weight[lane] * (qt - cfg_ref<IREF, IREF_Q>(P, L, t.g, lane)) * (qt - cfg_ref<IREF, IREF_Q>(P, L, t.g, lane))));
+    lf += oct_sum_ordered(z * (P.vf_weight[lane] * (vt - cfg_ref<IREF, IREF_V>(P, L, t.g, lane)) * (vt - cfg_ref<IREF, IREF_V>(P, L, t.g, lane))));
     double tc = 0.5 * lf;
     if (TASK) tc += 0.5 * task_weighted_sqnorm(te, P.task_wf6);
     cost += tc;

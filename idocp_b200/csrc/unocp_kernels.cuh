@@ -192,7 +192,10 @@ __global__ void k_set_solution(Layout L, int field, const double* __restrict__ v
 // KKT (with FUSED): also leave the squared KKT norm of the NEW iterate's stage in L.kkt_stage -- the very numbers
 // k_linearize<RESIDUAL_ONLY> would compute from it (same operations on the same values), so that a computeKKTResidual that
 // follows the pipelined updateSolution (ocpbenchmarker::Convergence, an MPC loop that watches the KKT error) only has to sum them
-template <bool RESIDUAL_ONLY, bool BACKWARD_EULER, bool TASK, bool FUSED, bool ACC = false, bool KKT = false>
+// IREF: the cost references of the instance (common.cuh: cfg_ref, task_ref_row) instead of the problem's; the forward-Euler
+// solver then also covers the terminal stage N and leaves diag(qf_weight), lq_N, lv_N in record N of KQ as TASK does, since
+// the per-instance Riccati sweep (k_riccati<true>) takes the terminal blocks from there
+template <bool RESIDUAL_ONLY, bool BACKWARD_EULER, bool TASK, bool FUSED, bool ACC = false, bool KKT = false, bool IREF = false>
 __device__ __forceinline__ void linearize_task(const DevProblem& P, const Layout& L, const double* __restrict__ q0,
                                                const double* __restrict__ v0, double* tile, const int i, const int g,
                                                const double* X, const double* D, const double* Xnf, const double* Dn,
@@ -252,23 +255,23 @@ __device__ __forceinline__ void linearize_task(const DevProblem& P, const Layout
         Xw[(X_SLACK + c) * SLOT] = fslack[c];
         Xw[(X_DUAL + c) * SLOT] = fdual[c];
       }
-    } else if (!TASK && !KKT) {
+    } else if (!TASK && !KKT && !IREF) {
       return;   // terminal stage: the update is all there is to do
     }
   }
 
-  if ((RESIDUAL_ONLY || TASK || KKT) && !BACKWARD_EULER && i == L.N) {
+  if ((RESIDUAL_ONLY || TASK || KKT || IREF) && !BACKWARD_EULER && i == L.N) {
     // TerminalOCP::linearizeOCP / computeKKTResidual + squaredNormKKTResidual (ocp/terminal_ocp.hxx:50-66,120-144)
     double lq = 0.0, lv = 0.0;
-    lq += P.qf_weight[lane] * (q - P.q_ref[lane]);
-    lv += P.vf_weight[lane] * (v - P.v_ref[lane]);
+    lq += P.qf_weight[lane] * (q - cfg_ref<IREF, IREF_Q>(P, L, g, lane));
+    lv += P.vf_weight[lane] * (v - cfg_ref<IREF, IREF_V>(P, L, g, lane));
     double hf[NV];
     if (TASK) {
       double R[9];
       V3 p;
       chain_fk(lane, act ? q : 0.0, P.model + lane * MODEL_STRIDE, R, p);
       TaskEval te;
-      task_evaluate<true>(R, p, P.ee, L.task_ref + static_cast<size_t>(i) * 12, te, P.task_enabled);
+      task_evaluate<true>(R, p, P.ee, task_ref_row<IREF>(L, i, b), te, P.task_enabled);
       task_share_columns(lane, te, tile);
       double gf;
       task_gradient_hessian(te, P.task_wf6, tile, gf, hf);
@@ -281,13 +284,13 @@ __device__ __forceinline__ void linearize_task(const DevProblem& P, const Layout
       const double e = oct_sum_ordered(lq * lq) + oct_sum_ordered(lv * lv);
       if (lane == 0) L.kkt_stage[static_cast<size_t>(i) * L.Bp + b] = e;
     }
-    if (RESIDUAL_ONLY || !TASK) {
+    if (RESIDUAL_ONLY || (!TASK && !IREF)) {
       // (nothing else to do: residual only, or the fused update of a problem without a task-space cost)
     } else {
       // terminal record: rows of Qqq_N (slot = row, lane = column), lq_N, lv_N
       double* KQ = rec_ptr(L.KQ, KQ_NUM, L.G, i, g);
 #pragma unroll
-      for (int r = 0; r < NV; ++r) KQ[(KQ_QQ + r) * SLOT] = (r == lane ? P.qf_weight[lane] : 0.0) + (act ? hf[r] : 0.0);
+      for (int r = 0; r < NV; ++r) KQ[(KQ_QQ + r) * SLOT] = (r == lane ? P.qf_weight[lane] : 0.0) + (TASK && act ? hf[r] : 0.0);
       KQ[KQ_LQ * SLOT] = lq;
       KQ[KQ_LV * SLOT] = lv;
     }
@@ -335,7 +338,7 @@ __device__ __forceinline__ void linearize_task(const DevProblem& P, const Layout
     chain_fk(lane, q, P.model + lane * MODEL_STRIDE, R, p);
     if (TASK) {
       TaskEval te;
-      task_evaluate<true>(R, p, P.ee, L.task_ref + static_cast<size_t>(i) * 12, te, P.task_enabled);
+      task_evaluate<true>(R, p, P.ee, task_ref_row<IREF>(L, i, b), te, P.task_enabled);
       task_share_columns(lane, te, tile);
       task_gradient_hessian(te, P.task_w6, tile, task_g, task_h);
       if (last) task_gradient_hessian(te, P.task_wf6, tile, task_gf, task_hf);
@@ -349,14 +352,14 @@ __device__ __forceinline__ void linearize_task(const DevProblem& P, const Layout
 
   // ---- gradient of the Lagrangian (SURVEY A.2 steps 1-4) ----
   double lq = 0.0, lv = 0.0, la = 0.0, lu = 0.0;
-  lq += dt * P.q_weight[lane] * (q - P.q_ref[lane]);
-  lv += dt * P.v_weight[lane] * (v - P.v_ref[lane]);
+  lq += dt * P.q_weight[lane] * (q - cfg_ref<IREF, IREF_Q>(P, L, g, lane));
+  lv += dt * P.v_weight[lane] * (v - cfg_ref<IREF, IREF_V>(P, L, g, lane));
   la += dt * P.a_weight[lane] * a;
-  lu += dt * P.u_weight[lane] * (u - P.u_ref[lane]);
+  lu += dt * P.u_weight[lane] * (u - cfg_ref<IREF, IREF_U>(P, L, g, lane));
   if (TASK) lq += dt * task_g;
   if (last) {   // + computeTerminalCostDerivatives (terminal_unparnmpc.hxx:84)
-    lq += P.qf_weight[lane] * (q - P.q_ref[lane]);
-    lv += P.vf_weight[lane] * (v - P.v_ref[lane]);
+    lq += P.qf_weight[lane] * (q - cfg_ref<IREF, IREF_Q>(P, L, g, lane));
+    lv += P.vf_weight[lane] * (v - cfg_ref<IREF, IREF_V>(P, L, g, lane));
     if (TASK) lq += task_gf;
   }
 #pragma unroll
@@ -576,14 +579,14 @@ __device__ __forceinline__ void linearize_task(const DevProblem& P, const Layout
 
 
 // ACC = true: + the two acceleration-limit components (their own array L.XA; the six-component instantiations are untouched)
-template <bool RESIDUAL_ONLY, bool BACKWARD_EULER, bool TASK, bool ACC = false>
+template <bool RESIDUAL_ONLY, bool BACKWARD_EULER, bool TASK, bool ACC = false, bool IREF = false>
 __global__ void __launch_bounds__(CTA_THREADS, LIN_MINB) k_linearize(const DevProblem* __restrict__ Pp, Layout L,
                                                                      const double* __restrict__ q0,
                                                                      const double* __restrict__ v0) {
   IDOCP_DYN_SMEM(double, smem);
   double* tile = smem + (threadIdx.x >> 3) * (OCT * PAIR_TILE);
-  const StageTask t = stage_task(L, ((RESIDUAL_ONLY || TASK) && !BACKWARD_EULER) ? L.N + 1 : L.N);
-  linearize_task<RESIDUAL_ONLY, BACKWARD_EULER, TASK, false, ACC>(*Pp, L, q0, v0, tile, t.stage, t.g,
+  const StageTask t = stage_task(L, ((RESIDUAL_ONLY || TASK || IREF) && !BACKWARD_EULER) ? L.N + 1 : L.N);
+  linearize_task<RESIDUAL_ONLY, BACKWARD_EULER, TASK, false, ACC, false, IREF>(*Pp, L, q0, v0, tile, t.stage, t.g,
                                                              rec_ptr(L.X, X_NUM, L.G, t.stage, t.g), nullptr, nullptr, nullptr, 1.0, 1.0);
 }
 
@@ -625,7 +628,7 @@ static_assert(X_LMD == 0 && X_GMM == 1 && X_Q == 2 && X_V == 3 && D_LMD == 0 && 
               "the next stage's (lmd, gmm, q, v) and their directions are the first four slots of a record");
 static_assert((UL_OFF_BUF * 8) % 16 == 0, "TMA destinations are 16-byte aligned");
 
-template <bool TASK, bool KKT = false>
+template <bool TASK, bool KKT = false, bool IREF = false>
 __global__ void __launch_bounds__(UL_THREADS, UL_CTAS_PER_SM) k_update_linearize(const DevProblem* __restrict__ Pp, Layout L) {
   IDOCP_DYN_SMEM(double, smem);
   const int warp = threadIdx.x >> 5, wl = threadIdx.x & 31;
@@ -665,7 +668,7 @@ __global__ void __launch_bounds__(UL_THREADS, UL_CTAS_PER_SM) k_update_linearize
     tma_bar_wait(&bars[buf], (k >> 1) & 1);
     const double* rec = bufs + buf * (UL_SLOTS * SLOT);
     const int o4 = (threadIdx.x >> 3) & 3;
-    linearize_task<false, false, TASK, true, false, KKT>(*Pp, L, nullptr, nullptr, tile, static_cast<int>(wt / L.G), static_cast<int>(wt % L.G),
+    linearize_task<false, false, TASK, true, false, KKT, IREF>(*Pp, L, nullptr, nullptr, tile, static_cast<int>(wt / L.G), static_cast<int>(wt % L.G),
                                              rec + wl, rec + UL_D * SLOT + wl, rec + UL_XN * SLOT + wl, rec + UL_DN * SLOT + wl,
                                              rec[UL_ST * SLOT + o4], rec[UL_ST * SLOT + 4 + o4]);
   }
@@ -714,7 +717,8 @@ static_assert(RIC_MINB * (RIC_SMEM_DOUBLES * 8 + 1024) <= 228 * 1024, "k_riccati
 static_assert(KQ_AA == 0 && KQ_QQ == 3 * NV && KQ_FQ == 6 * NV && KQ_NUM == 6 * NV + 5, "record layout");
 static_assert(W_KQ == 0 && W_KV == NV && W_K == 2 * NV && KQ_FV == KQ_FQ + 1, "record layout");
 
-// TASK = true: the terminal Hessian / gradient are dense and come from record N of KQ (k_linearize<.., true>)
+// TASK = true: the terminal Hessian / gradient come from record N of KQ (k_linearize<.., true> and the per-instance reference
+// instantiations, which write the cost's reference there: this sweep itself reads no reference)
 template <bool TASK>
 __global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProblem* __restrict__ Pp, Layout L,
                                                    const double* __restrict__ q0,
@@ -805,6 +809,7 @@ __global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProb
 #pragma unroll
       for (int r = 0; r < NV; ++r) Pqq[r] = KQN[(KQ_QQ + r) * SLOT];
       sq = -KQN[KQ_LQ * SLOT];
+      sv = -KQN[KQ_LV * SLOT];
     }
     __syncwarp();
   }
@@ -1054,8 +1059,9 @@ __global__ void __launch_bounds__(RIC_THREADS, RIC_MINB) k_riccati(const DevProb
 // PARNMPC = true (UnParNMPCSolver): N stages, none terminal, the costate direction is already in D
 // (k_parnmpc_forward_parallel); only the condensed direction and the step sizes are computed.
 // TASK = true: the terminal P_N = Qqq_N is dense (record N of KQ)
+// IREF = true: the terminal gradient from the instance's cost reference (common.cuh: cfg_ref)
 constexpr int EXP_TILE = 9;   // odd stride (doubles) of the Pqv transpose tile of k_expand
-template <bool PARNMPC, bool TASK, bool ACC = false>
+template <bool PARNMPC, bool TASK, bool ACC = false, bool IREF = false>
 __global__ void __launch_bounds__(CTA_THREADS, EXP_MINB) k_expand(const DevProblem* __restrict__ Pp, Layout L, int stage_offset) {
   const DevProblem& P = *Pp;
   const int lane = lane_in_octet();
@@ -1070,8 +1076,8 @@ __global__ void __launch_bounds__(CTA_THREADS, EXP_MINB) k_expand(const DevProbl
   if (!PARNMPC && i == N) {
     const double q = X[X_Q * SLOT], v = X[X_V * SLOT], lmd = X[X_LMD * SLOT], gmm = X[X_GMM * SLOT];
     double lq = 0.0, lv = 0.0;
-    lq += P.qf_weight[lane] * (q - P.q_ref[lane]);
-    lv += P.vf_weight[lane] * (v - P.v_ref[lane]);
+    lq += P.qf_weight[lane] * (q - cfg_ref<IREF, IREF_Q>(P, L, t.g, lane));
+    lv += P.vf_weight[lane] * (v - cfg_ref<IREF, IREF_V>(P, L, t.g, lane));
     lq -= lmd;
     lv -= gmm;
     double dlmd = P.qf_weight[lane] * dq; dlmd -= -lq;

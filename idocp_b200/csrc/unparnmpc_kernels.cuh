@@ -61,8 +61,8 @@ inline int parnmpc_alloc(ParNMPCLayout& PL, int N, int Bp, Alloc alloc) {
 // k_parnmpc_init_aux: every aux_mat = Hessian of the terminal cost = diag(qf_weight, vf_weight)
 // ---------------------------------------------------------------------------------------------
 // TASK = true: + the (dense) Gauss-Newton Hessian of the terminal task-space cost at s[N-1]
-// (TerminalUnParNMPC::computeTerminalCostHessian, terminal_unparnmpc.hxx:230-241)
-template <bool TASK>
+// (TerminalUnParNMPC::computeTerminalCostHessian, terminal_unparnmpc.hxx:230-241); IREF = true: the instance's task table
+template <bool TASK, bool IREF = false>
 __global__ void __launch_bounds__(CTA_THREADS) k_parnmpc_init_aux(const DevProblem* __restrict__ Pp, Layout L,
                                                                   ParNMPCLayout PL) {
   IDOCP_DYN_SMEM(double, smem);
@@ -81,7 +81,7 @@ __global__ void __launch_bounds__(CTA_THREADS) k_parnmpc_init_aux(const DevProbl
     V3 p;
     chain_fk(lane, act ? X[X_Q * SLOT] : 0.0, P.model + lane * MODEL_STRIDE, R, p);
     TaskEval te;
-    task_evaluate<true>(R, p, P.ee, L.task_ref + static_cast<size_t>(L.N - 1) * 12, te, P.task_enabled);
+    task_evaluate<true>(R, p, P.ee, task_ref_row<IREF>(L, L.N - 1, t.g * 4 + ((threadIdx.x >> 3) & 3)), te, P.task_enabled);
     task_share_columns(lane, te, tile);
     double gf, hf[NV];
     task_gradient_hessian(te, P.task_wf6, tile, gf, hf);

@@ -164,12 +164,30 @@ class _BatchSolver:
 
     def setTaskReference(self, ref, t=0.0):
         """TimeVaryingTaskSpace6DCost reference: `ref` is the user's compute_q_6d_ref(t) -> 12 doubles
-        (R row-major, p), sampled here on the host at every stage time, or an (N+1, 12) table."""
+        (R row-major, p), sampled here on the host at every stage time, or an (N+1, 12) table shared by the batch.
+        A (batch, N+1, 12) table gives every instance its own reference (idocp_b200_set_instance_task_reference; rows as
+        stageTimes(t)) until clearInstanceReferences()."""
         table = np.array([ref(x) for x in self.stageTimes(t)]) if callable(ref) else np.asarray(ref, dtype=np.float64)
         table = np.ascontiguousarray(table, dtype=np.float64)
+        if table.shape == (self.batch, self.N + 1, 12):
+            self.lib.check(self._f("set_instance_task_reference")(self._h, dptr(table)))
+            return
         if table.shape != (self.N + 1, 12):
-            raise ValueError("task reference table must have shape (%d, 12)" % (self.N + 1))
+            raise ValueError("task reference table must have shape (%d, 12) or (%d, %d, 12)" % (self.N + 1, self.batch, self.N + 1))
         self.lib.check(self._f("set_task_reference")(self._h, dptr(table)))
+
+    def setCostReference(self, name, value):
+        """ConfigurationSpaceCost::set_q_ref / set_v_ref / set_u_ref of every instance: name in ("q_ref", "v_ref", "u_ref"),
+        value (batch, dimv).  The first call switches the batch to per-instance references; the two other fields start as
+        the problem's.  Invalidates the kept linearisation; the line-search filter is left as it is."""
+        value = np.ascontiguousarray(np.asarray(value, dtype=np.float64))
+        if value.shape != (self.batch, DIMV):
+            raise ValueError("setCostReference: expected shape (%d, %d), got %s" % (self.batch, DIMV, value.shape))
+        self.lib.check(self._f("set_instance_reference")(self._h, name.encode(), dptr(value)))
+
+    def clearInstanceReferences(self):
+        """Back to the problem's q_ref / v_ref / u_ref and the last shared task table for every instance."""
+        self.lib.check(self._f("clear_instance_references")(self._h))
 
     def updateSolution(self, t, q, v, line_search=False):
         q, v = self._x(q), self._x(v)

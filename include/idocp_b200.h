@@ -157,6 +157,23 @@ int idocp_b200_clear_line_search_filter(idocp_b200_solver* h);
  * Call it before updateSolution / computeKKTResidual / initBackwardCorrection whenever t changes. */
 int idocp_b200_set_task_reference(idocp_b200_solver* h, const double* table);
 
+/* Per-instance cost references: the counterpart of one reference solver object per instance, each with its own
+ * ConfigurationSpaceCost::set_q_ref / set_v_ref / set_u_ref and its own task-space reference.  A handle starts in shared mode
+ * (the problem's q_ref / v_ref / u_ref, the table of idocp_b200_set_task_reference for every instance).
+ *   set_instance_reference: name in {"q_ref", "v_ref", "u_ref"}, value[batch][7].  The first call switches the
+ *     configuration-space cost to per-instance references; the two other fields start as copies of the problem's.
+ *   set_instance_task_reference: table[batch][N+1][12] = [R row-major (9), p (3)], rows as idocp_b200_set_task_reference
+ *     (a constant target: every row the same).  Switches the task-space cost to per-instance tables; the shared table that
+ *     idocp_b200_set_task_reference keeps writing is stored but not read until the clear.  Needs task_enabled != 0.
+ *   clear_instance_references: back to the problem's references and the last shared table.
+ * Every call invalidates the linearisation a pipelined UnOCPSolver keeps for its next updateSolution.  The line-search
+ * filter is NOT cleared, as on a change of the shared references; call idocp_b200_clear_line_search_filter for a fresh
+ * start.  Instance b gives the bits of a shared-mode handle whose problem / table hold instance b's references.  The
+ * DerivativeChecker (idocp_b200_check_cost_derivatives) always uses the shared references. */
+int idocp_b200_set_instance_reference(idocp_b200_solver* h, const char* name, const double* value);
+int idocp_b200_set_instance_task_reference(idocp_b200_solver* h, const double* table);
+int idocp_b200_clear_instance_references(idocp_b200_solver* h);
+
 /* Device-side analogue of idocp::DerivativeChecker (include/idocp/utils/derivative_checker.hpp:14-66,
  * src/utils/derivative_checker.cpp:47-312) for the cost of this handle's problem: for n samples of a split solution
  * (q, v, a, u rows [n][7], host pointers) the kernel evaluates the cost with the device functions of the line search and its
@@ -210,6 +227,9 @@ int idocp_b200_sharded_set_solution(idocp_b200_sharded* s, const char* name, con
 int idocp_b200_sharded_init_constraints(idocp_b200_sharded* s);
 int idocp_b200_sharded_init_backward_correction(idocp_b200_sharded* s, double t);
 int idocp_b200_sharded_set_task_reference(idocp_b200_sharded* s, const double* table);
+int idocp_b200_sharded_set_instance_reference(idocp_b200_sharded* s, const char* name, const double* value /* [batch][7] */);
+int idocp_b200_sharded_set_instance_task_reference(idocp_b200_sharded* s, const double* table /* [batch][N+1][12] */);
+int idocp_b200_sharded_clear_instance_references(idocp_b200_sharded* s);
 int idocp_b200_sharded_update_solution(idocp_b200_sharded* s, double t, const double* q, const double* v, int line_search);
 int idocp_b200_sharded_compute_kkt_residual(idocp_b200_sharded* s, double t, const double* q, const double* v);
 int idocp_b200_sharded_kkt_error(idocp_b200_sharded* s, double* out /* [batch] */);

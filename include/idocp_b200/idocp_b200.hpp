@@ -644,6 +644,24 @@ class SolverBase {
     }
   }
   void clearLineSearchFilter() { check(idocp_b200_sharded_clear_line_search_filter(hs_.get())); }
+  // Per-instance cost references (idocp_b200_set_instance_reference): the batch counterpart of one solver object per instance,
+  // each with its own ConfigurationSpaceCost::set_q_ref / set_v_ref / set_u_ref.  name in {"q_ref", "v_ref", "u_ref"},
+  // per_instance row-major [batch][dimv]; the fields not set start as the cost's.  The line-search filter is kept.
+  void setCostReference(const std::string& name, const double* per_instance) {
+    check(idocp_b200_sharded_set_instance_reference(hs_.get(), name.c_str(), per_instance));
+  }
+  // per-instance task-space reference table_per_instance[batch][N+1][12] = [R row-major (9), p (3)] per stage index, rows as
+  // the cost's reference is sampled (sampleTaskReference); while it is set, the cost's reference object is not sampled
+  void setTaskReference(const double* table_per_instance) {
+    check(idocp_b200_sharded_set_instance_task_reference(hs_.get(), table_per_instance));
+    instance_tables_ = true;
+  }
+  // back to the cost's references for every instance (the reference object is sampled again at the next call)
+  void clearInstanceReferences() {
+    check(idocp_b200_sharded_clear_instance_references(hs_.get()));
+    instance_tables_ = false;
+    task_sampled_ = false;
+  }
   // fuse the update with the linearisation of the new iterate (UnOCPSolver, default on; results are bit-identical)
   void setPipelining(bool enabled) { for (idocp_b200_solver* h : shards_) check(idocp_b200_set_pipelining(h, enabled ? 1 : 0)); }
   bool isCurrentSolutionFeasible() {
@@ -669,7 +687,7 @@ class SolverBase {
   // the user's compute_q_6d_ref at the time of every stage index (unocp_solver.cpp:80-93: t + i dt, terminal
   // t + T; unbackward_correction.cpp:73-95: t + (i+1) dt, last stage t + T), re-sampled only when t changes
   void sampleTaskReference(double t) {
-    if (!task_ || !task_->ref()) return;
+    if (!task_ || !task_->ref() || instance_tables_) return;
     if (task_sampled_ && t == task_t_) return;
     const double dt = T_ / N_;
     std::vector<double> table(static_cast<size_t>(N_ + 1) * 12);
@@ -705,6 +723,7 @@ class SolverBase {
   double T_;
   std::shared_ptr<TimeVaryingTaskSpace6DCost> task_;
   bool task_sampled_ = false;
+  bool instance_tables_ = false;   // setTaskReference(table_per_instance) is in force: the cost's reference is not sampled
   double task_t_ = 0.0;
   std::vector<double> qb_, vb_;
 };
