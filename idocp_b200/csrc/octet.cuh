@@ -49,7 +49,7 @@ __device__ __forceinline__ V3 mul(const S3& A, V3 b) {
             fma(A.zz, b.z, fma(A.yz, b.y, A.xz * b.x))};
 }
 
-// sin / cos for |x| up to a few pi: Cody-Waite reduction by pi/2 + the classic degree-13/14
+// sin / cos: Cody-Waite reduction by pi/2 + the classic degree-13/14
 // minimax kernels, written with explicit fma so that the oracle can repeat it bit for bit.
 __device__ __forceinline__ void canon_sincos(double x, double* sn, double* cs) {
   const double k = rint(x * 6.36619772367581382433e-01);            // x * 2/pi
@@ -68,7 +68,7 @@ __device__ __forceinline__ void canon_sincos(double x, double* sn, double* cs) {
   pc = fma(z, pc, -1.38888888888741095749e-03);
   pc = fma(z, pc, 4.16666666666666019037e-02);
   const double c = fma(z * z, pc, fma(-0.5, z, 1.0));
-  const int q = static_cast<int>(k) & 3;
+  const int q = static_cast<int>(static_cast<long long>(k) & 3);   // exact for every |k| < 2^53 (an int overflows past 2^31)
   *sn = (q == 0) ? s : (q == 1) ? c : (q == 2) ? -s : -c;
   *cs = (q == 0) ? c : (q == 1) ? -s : (q == 2) ? -c : s;
 }
@@ -98,11 +98,19 @@ __device__ __forceinline__ double canon_rsqrt(double x) {
   return y;
 }
 
-// natural logarithm of a positive normal double (barrier cost of the line search): the classic
-// k*ln2 + log(1+f) reduction with the degree-14 minimax polynomial in s = f/(2+f), one code path,
-// written with plain IEEE operations so that the oracle repeats it bit for bit (<= 2 ulp).
+// natural logarithm (barrier cost of the line search): the classic fdlibm k*ln2 + log(1+f) reduction with the
+// degree-14 minimax polynomial in s = f/(2+f), written with plain IEEE operations so that the oracle repeats it bit for
+// bit.  Subnormals are scaled by 2^54 first; 0, negatives, NaN and +inf give std::log's results.
 __device__ __forceinline__ double canon_log(double x) {
-  if (!(x > 0.0)) return (x == 0.0) ? -1.0 / 0.0 : 0.0 / 0.0;  // log(0) = -inf, log(<0) = NaN as std::log
+  int k = 0;
+  if (!(x >= 2.2250738585072014e-308)) {   // not a positive normal: 0, subnormal, negative or NaN
+    if (x == 0.0) return -1.0 / 0.0;
+    if (!(x > 0.0)) return (x != x) ? x : 0.0 / 0.0;
+    x *= 18014398509481984.0;              // 2^54
+    k = -54;
+  } else if (!(x < 1.0 / 0.0)) {
+    return x;                              // log(+inf) = +inf
+  }
   long long bits;
 #ifdef IDOCP_B200_EMU
   memcpy(&bits, &x, sizeof(bits));
@@ -110,7 +118,7 @@ __device__ __forceinline__ double canon_log(double x) {
   bits = __double_as_longlong(x);
 #endif
   int hx = static_cast<int>(bits >> 32);
-  int k = (hx >> 20) - 1023;
+  k += (hx >> 20) - 1023;
   hx &= 0x000fffff;
   const int i = (hx + 0x95f64) & 0x100000;       // mantissa >= sqrt(2): use x/2, k+1
   k += (i >> 20);
@@ -135,7 +143,8 @@ __device__ __forceinline__ double canon_log(double x) {
 }
 
 // acos on [-1, 1]: the fdlibm e_acos.c algorithm with plain IEEE operations (task-space cost: log3 of
-// the end-effector rotation error); the oracle repeats it bit for bit.
+// the end-effector rotation error); the oracle repeats it bit for bit.  Arguments below -1 give pi, above 1 give 0,
+// NaN gives NaN.
 __device__ __forceinline__ double canon_acos_poly(double z) {
   const double pS0 = 1.66666666666666657415e-01, pS1 = -3.25565818622400915405e-01, pS2 = 2.01212532134862925881e-01,
                pS3 = -4.00555345006794114027e-02, pS4 = 7.91534994289814532176e-04, pS5 = 3.47933107596021167570e-05;
@@ -148,7 +157,7 @@ __device__ __forceinline__ double canon_acos_poly(double z) {
 __device__ __forceinline__ double canon_acos(double x) {
   const double pio2_hi = 1.57079632679489655800e+00, pio2_lo = 6.12323399573676603587e-17;
   const double pi = 3.14159265358979311600e+00;
-  if (!(x > -1.0)) return pi;
+  if (!(x > -1.0)) return (x != x) ? x : pi;
   if (!(x < 1.0)) return 0.0;
   if (fabs(x) < 0.5) {
     const double r = canon_acos_poly(x * x);

@@ -63,18 +63,27 @@ static inline void canon_sincos(double x, double* sn, double* cs) {
   pc = fma(z, pc, -1.38888888888741095749e-03);
   pc = fma(z, pc, 4.16666666666666019037e-02);
   const double c = fma(z * z, pc, fma(-0.5, z, 1.0));
-  const int q = ((int)k) & 3;
+  const int q = (int)((long long)k & 3);   /* exact for every |k| < 2^53 (an int overflows past 2^31) */
   *sn = (q == 0) ? s : (q == 1) ? c : (q == 2) ? -s : -c;
   *cs = (q == 0) ? c : (q == 1) ? -s : (q == 2) ? -c : s;
 }
 void oracle_canon_sincos(double x, double* sn, double* cs) { canon_sincos(x, sn, cs); }
-/* natural logarithm of a positive normal double (twin of canon_log in octet.cuh) */
+/* natural logarithm (twin of canon_log in octet.cuh): subnormals scaled by 2^54 first; 0, negatives, NaN and +inf
+ * as std::log */
 static inline double canon_log(double x) {
-  if (!(x > 0.0)) return (x == 0.0) ? -INFINITY : NAN;  /* as std::log */
+  int k = 0;
+  if (!(x >= 2.2250738585072014e-308)) {   /* not a positive normal: 0, subnormal, negative or NaN */
+    if (x == 0.0) return -INFINITY;
+    if (!(x > 0.0)) return (x != x) ? x : NAN;
+    x *= 18014398509481984.0;              /* 2^54 */
+    k = -54;
+  } else if (!(x < INFINITY)) {
+    return x;                              /* log(+inf) = +inf */
+  }
   long long bits;
   memcpy(&bits, &x, sizeof(bits));
   int hx = (int)(bits >> 32);
-  int k = (hx >> 20) - 1023;
+  k += (hx >> 20) - 1023;
   hx &= 0x000fffff;
   const int i = (hx + 0x95f64) & 0x100000;
   k += (i >> 20);
@@ -442,7 +451,7 @@ static inline double canon_acos(double x) {
                pS3 = -4.00555345006794114027e-02, pS4 = 7.91534994289814532176e-04, pS5 = 3.47933107596021167570e-05;
   const double qS1 = -2.40339491173441421878e+00, qS2 = 2.02094576023350569471e+00, qS3 = -6.88283971605453293030e-01,
                qS4 = 7.70381505559019352791e-02;
-  if (!(x > -1.0)) return pi;      /* x <= -1 (and NaN -> pi, never reached with a clamped argument) */
+  if (!(x > -1.0)) return (x != x) ? x : pi;   /* x <= -1 gives pi, NaN gives NaN */
   if (!(x < 1.0)) return 0.0;
   const double ax = fabs(x);
   if (ax < 0.5) {
