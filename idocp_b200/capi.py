@@ -118,13 +118,15 @@ EXPORTS = [
     "idocp_b200_fb_sync", "idocp_b200_fb_launch_count", "idocp_b200_fb_stream", "idocp_b200_fb_set_profiling",
     "idocp_b200_fb_get_profile", "idocp_b200_fb_record_bytes", "idocp_b200_fb_problem_default",
     "idocp_b200_fb_total_weight", "idocp_b200_fb_contact_frame_positions", "idocp_b200_fb_clear_line_search_filter",
-    "idocp_b200_fb_set_strict_discretization",
+    "idocp_b200_fb_set_strict_discretization", "idocp_b200_fb_set_instance_cost_reference",
+    "idocp_b200_fb_clear_instance_cost_references",
     "idocp_b200_fb_create_sharded", "idocp_b200_fb_sharded_destroy", "idocp_b200_fb_sharded_num_shards", "idocp_b200_fb_sharded_shard",
     "idocp_b200_fb_sharded_set_solution", "idocp_b200_fb_sharded_set_cost_reference", "idocp_b200_fb_sharded_discretize",
     "idocp_b200_fb_sharded_init_constraints", "idocp_b200_fb_sharded_set_strict_discretization",
     "idocp_b200_fb_sharded_update_solution", "idocp_b200_fb_sharded_compute_kkt_residual", "idocp_b200_fb_sharded_kkt_error",
     "idocp_b200_fb_sharded_clear_line_search_filter", "idocp_b200_fb_sharded_get_step_sizes", "idocp_b200_fb_sharded_get",
-    "idocp_b200_fb_sharded_sync", "idocp_b200_fb_sharded_launch_count",
+    "idocp_b200_fb_sharded_sync", "idocp_b200_fb_sharded_launch_count", "idocp_b200_fb_sharded_set_instance_cost_reference",
+    "idocp_b200_fb_sharded_clear_instance_cost_references",
     "idocp_b200_create_sharded", "idocp_b200_sharded_destroy", "idocp_b200_sharded_num_shards", "idocp_b200_sharded_shard",
     "idocp_b200_sharded_set_solution", "idocp_b200_sharded_init_constraints", "idocp_b200_sharded_init_backward_correction",
     "idocp_b200_sharded_set_task_reference", "idocp_b200_sharded_set_instance_reference",
@@ -198,6 +200,8 @@ class Library:
         L.idocp_b200_fb_destroy.argtypes = [C.c_void_p]
         L.idocp_b200_fb_set_solution.argtypes = [C.c_void_p, C.c_char_p, _dp, C.c_int]
         L.idocp_b200_fb_set_cost_reference.argtypes = [C.c_void_p, C.c_int, C.c_int, _dp, _dp]
+        L.idocp_b200_fb_set_instance_cost_reference.argtypes = [C.c_void_p, C.c_int, C.c_int, _dp, _dp]
+        L.idocp_b200_fb_clear_instance_cost_references.argtypes = [C.c_void_p]
         L.idocp_b200_fb_discretize.argtypes = [C.c_void_p, C.c_double, C.c_int, _ip, _ip, _dp, _dp, _ip, _ip, _ip]
         L.idocp_b200_fb_init_constraints.argtypes = [C.c_void_p, C.c_double]
         L.idocp_b200_fb_update_solution.argtypes = [C.c_void_p, C.c_double, _dp, _dp, C.c_int]
@@ -215,7 +219,7 @@ class Library:
         # the sharded twins take the same arguments behind the handle
         for name in ("set_solution", "set_cost_reference", "discretize", "init_constraints", "update_solution", "compute_kkt_residual",
                      "kkt_error", "get_step_sizes", "get", "sync", "clear_line_search_filter", "set_strict_discretization",
-                     "launch_count"):
+                     "launch_count", "set_instance_cost_reference", "clear_instance_cost_references"):
             getattr(L, "idocp_b200_fb_sharded_" + name).argtypes = getattr(L, "idocp_b200_fb_" + name).argtypes
         L.idocp_b200_fb_create_sharded.argtypes = [C.POINTER(FbProblem), C.c_void_p, C.c_int, _ip, C.c_int, C.POINTER(C.c_void_p)]
         L.idocp_b200_fb_problem_default.argtypes = [C.POINTER(FbProblem)]

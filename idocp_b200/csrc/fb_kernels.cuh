@@ -135,7 +135,18 @@ struct FbArrays {
   double* kkt_err;    // [B]
   LsFilter ls;        // filter line search of B instances (line_search_filter.cuh)
   int* ls_status;     // [B] IDOCP_B200_STATUS_FILTER_FULL
+  const double* iref; // [slot][B][FB_IREF] per-instance (q_ref, v_ref) (the IREF instantiations); nullptr in shared mode
 };
+constexpr int FB_IREF = FB_NQ + FB_NV;
+// the cost reference (q_ref, then v_ref) of record `rec` = (slot, instance): per instance (IREF) or shared by the batch
+template <bool IREF>
+__device__ __forceinline__ const double* fb_ref_q(const FbArrays& A, const FbElem& el, size_t rec) {
+  return IREF ? A.iref + rec * FB_IREF : el.ref_q;
+}
+template <bool IREF>
+__device__ __forceinline__ const double* fb_ref_v(const FbArrays& A, const FbElem& el, size_t rec) {
+  return IREF ? A.iref + rec * FB_IREF + FB_NQ : el.ref_v;
+}
 
 #define FB_FOR(i, n) for (int i = threadIdx.x; i < (n); i += blockDim.x)
 enum { FBM_SET = 0, FBM_ADD = 1, FBM_SUB = 2 };
@@ -934,7 +945,8 @@ constexpr int FB_ROBOT_WARPS = 6;   // x 2 CTAs per SM: 12 warps (18.6 KB of sha
 constexpr int FB_ROBOT_MINB = 2;
 constexpr int FB_LS_WARPS = 5;      // k_fb_ls_eval (FbLsWork, 23 KB per warp)
 
-template <bool RESIDUAL_ONLY>
+// IREF: the cost reference of (slot, instance) comes from A.iref instead of the chain element shared by the batch
+template <bool RESIDUAL_ONLY, bool IREF>
 __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot(FbArrays A, FbLin* lin) {
   IDOCP_DYN_SMEM(FbRobotWork, wbase);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -992,7 +1004,7 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
   // ---- SE(3): lanes 0..2 in lock-step on (q, q_ref), (q, q_next), (q_prev, q) ----
   if (lane < 3 && !(terminal && lane == 1)) {
     const double* qp = lane == 2 ? w.qprev : w.q;
-    const double* qm = lane == 0 ? el.ref_q : (lane == 1 ? w.nq : w.q);
+    const double* qm = lane == 0 ? fb_ref_q<IREF>(A, el, rec) : (lane == 1 ? w.nq : w.q);
     fbw_se3_pair(qp, qm, w.relR[lane], w.relp[lane], w.rellog[lane], w.relJ[lane]);
   }
   __syncwarp();
@@ -1026,7 +1038,7 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
   }
   if (lane < FB_NV) {
     const int j = lane;
-    const double qd = j < 6 ? w.rellog[0][j] : (w.q[1 + j] - el.ref_q[1 + j]);
+    const double qd = j < 6 ? w.rellog[0][j] : (w.q[1 + j] - fb_ref_q<IREF>(A, el, rec)[1 + j]);
     if (j < 6) {
       double acc = J6c[j] * (wq[0] * w.rellog[0][0]);
       for (int k = 1; k < 6; ++k) acc = fma(J6c[6 * k + j], wq[k] * w.rellog[0][k], acc);
@@ -1034,7 +1046,7 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS, FB_ROBOT_MINB) k_fb_robot
     } else {
       lq += sc * (wq[j] * qd);
     }
-    lv += sc * (wv[j] * (w.v[j] - el.ref_v[j]));
+    lv += sc * (wv[j] * (w.v[j] - fb_ref_v<IREF>(A, el, rec)[j]));
     if (!terminal) la += sc * (wa[j] * w.a[j]);
   }
   if (ci >= 0) {   // ContactForceCost gradient (contact_force_cost.cpp:161-187)
@@ -2470,7 +2482,7 @@ __global__ void __launch_bounds__(32 * FB_ROBOT_WARPS) k_fb_init_distance(FbArra
 // rounds of line_search_filter.cuh  k_fb_ls_eval (warp per (instance, stage): stage cost and constraint violation of
 // the trial point s + alpha d)  ->  k_fb_ls_filter (thread per instance); finished instances drop out.
 // =====================================================================================================
-template <bool INITIAL>
+template <bool INITIAL, bool IREF>
 __global__ void __launch_bounds__(32 * FB_LS_WARPS) k_fb_ls_eval(FbArrays A, FbLin* lin) {
   IDOCP_DYN_SMEM(FbLsWork, wbase);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -2527,7 +2539,7 @@ __global__ void __launch_bounds__(32 * FB_LS_WARPS) k_fb_ls_eval(FbArrays A, FbL
   // q - q_ref and (not terminal) q - q_next, base blocks by lanes 0 and 1 in lock-step
   if (lane < 2 && !(terminal && lane == 1)) {
     double R[9], p3[3];
-    fb_relative(lane == 0 ? el.ref_q : w.nq, w.q, R, p3);
+    fb_relative(lane == 0 ? fb_ref_q<IREF>(A, el, rec) : w.nq, w.q, R, p3);
     fb_log6(R, p3, w.rellog[lane]);
   }
   __syncwarp();
@@ -2565,8 +2577,8 @@ __global__ void __launch_bounds__(32 * FB_LS_WARPS) k_fb_ls_eval(FbArrays A, FbL
   if (lane == 0) {
     const double half = (terminal || impulse) ? 0.5 : 0.5 * dt;
     double l = 0.0;
-    for (int j = 0; j < FB_NV; ++j) { const double d = j < 6 ? w.rellog[0][j] : (w.q[1 + j] - el.ref_q[1 + j]); l = fma(wq[j] * d, d, l); }
-    for (int j = 0; j < FB_NV; ++j) { const double d = w.v[j] - el.ref_v[j]; l = fma(wv[j] * d, d, l); }
+    for (int j = 0; j < FB_NV; ++j) { const double d = j < 6 ? w.rellog[0][j] : (w.q[1 + j] - fb_ref_q<IREF>(A, el, rec)[1 + j]); l = fma(wq[j] * d, d, l); }
+    for (int j = 0; j < FB_NV; ++j) { const double d = w.v[j] - fb_ref_v<IREF>(A, el, rec)[j]; l = fma(wv[j] * d, d, l); }
     if (!terminal)
       for (int j = 0; j < FB_NV; ++j) l = fma(wa[j] * w.a[j], w.a[j], l);
     double cost = half * l;

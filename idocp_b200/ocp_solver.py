@@ -44,6 +44,7 @@ class OCPSolver:
             self.lib.check(self.lib.L.idocp_b200_fb_create(C.byref(problem), self.contact_sequence._h, self.B, int(device),
                                                            C.byref(self._h)))
         self._chain = []
+        self.instance_reference = None
 
     def _f(self, name):
         """The C-ABI entry point `name` of this solver: idocp_b200_fb_<name> or its sharded twin (same arguments)."""
@@ -91,17 +92,35 @@ class OCPSolver:
                             dimi=int(dimi[e])) for e in range(n)]
         return self._chain
 
+    def setInstanceCostReference(self, fn):
+        """Per-instance configuration references: fn(t) returns (q_ref (B, 19), v_ref (B, 18)), row b the reference of
+        instance b at time t.  From now on every call samples fn at the time of every stage instead of the shared q_ref."""
+        self.instance_reference = fn
+
+    def clearInstanceCostReferences(self):
+        """Back to the shared reference q_ref(t) for every instance.  The shared reference is not sampled while per-instance
+        references are set, so a following updateSolutionResident (which samples nothing) runs on the shared values of the
+        last sampled call until the next updateSolution / computeKKTResidual / initConstraints samples q_ref(t) again."""
+        self.instance_reference = None
+        self.lib.check(self._f("clear_instance_cost_references")(self._h))
+
     def _sample_reference(self, t):
         chain = self.discretize(t)
-        if self.q_ref is None:
+        fn = self.instance_reference or self.q_ref
+        if fn is None:
             return chain
+        per = self.instance_reference is not None
+        shape_q, shape_v = (self.B, NQ), (self.B, NV)
+        setter = self._f("set_instance_cost_reference" if per else "set_cost_reference")
         for el in chain:
-            q_ref, v_ref = self.q_ref(el["t"])
+            q_ref, v_ref = fn(el["t"])
             q_ref = np.ascontiguousarray(q_ref, dtype=np.float64)
             v_ref = np.ascontiguousarray(v_ref, dtype=np.float64)
+            if per and (q_ref.shape != shape_q or v_ref.shape != shape_v):
+                raise ValueError("per-instance references must be q_ref %s and v_ref %s, got %s and %s"
+                                 % (shape_q, shape_v, q_ref.shape, v_ref.shape))
             kind = KIND_GRID if el["kind"] == KIND_TERMINAL else el["kind"]
-            self.lib.check(self._f("set_cost_reference")(self._h, kind, el["index"], capi.dptr(q_ref),
-                                                                       capi.dptr(v_ref)))
+            self.lib.check(setter(self._h, kind, el["index"], capi.dptr(q_ref), capi.dptr(v_ref)))
         return chain
 
     def initConstraints(self, t):

@@ -304,8 +304,8 @@ int idocp_b200_discretize_ocp(const idocp_b200_contact_sequence* cs, double T, i
 
 /* ------------------------------------------------------------------------------------------------------------
  * OCPSolver for the floating-base robot (ANYmal: free-flyer + 12 joints, 4 point contacts), SURVEY.md section 8 row a12.
- * One handle = a batch of independent OCP instances that share the problem, the contact schedule and the cost
- * reference and differ in the initial state and in their iterates.  Mirrors
+ * One handle = a batch of independent OCP instances that share the problem and the contact schedule and differ in the
+ * initial state, in their iterates and, optionally, in the cost reference.  Mirrors
  *   OCPSolver(robot, cost, constraints, T, N, max_num_impulse, nthreads)   src/ocp/ocp_solver.cpp:10-48
  *   setSolution / initConstraints / updateSolution / computeKKTResidual / KKTError / getSolution
  *                                                                          src/ocp/ocp_solver.cpp:60-92,96-213,244-280
@@ -359,6 +359,19 @@ int idocp_b200_fb_destroy(idocp_b200_fb_solver* h);
 int idocp_b200_fb_set_solution(idocp_b200_fb_solver* h, const char* name, const double* value, int per_instance);
 /* cost reference of one slot: kind 0 grid stage (index = time stage, N = terminal), 1 impulse, 2 aux, 3 lift */
 int idocp_b200_fb_set_cost_reference(idocp_b200_fb_solver* h, int kind, int index, const double* q_ref, const double* v_ref);
+/* Per-instance cost references: the counterpart of one reference OCPSolver per instance, each with its own q_ref(t) / v_ref.
+ * A handle starts in shared mode (the references of idocp_b200_fb_set_cost_reference for every instance).
+ *   set_instance_cost_reference: q_ref[batch][19], v_ref[batch][18] of the slot (kind, index), same kind / index rules as
+ *     idocp_b200_fb_set_cost_reference.  The first call after creation or a clear switches to per-instance references and
+ *     starts every slot of every instance from the shared references, so the slots never set keep the shared values.
+ *     idocp_b200_fb_set_cost_reference keeps writing the shared references, which are not read until the clear.
+ *   clear_instance_cost_references: back to the shared references.
+ * The host keeps the table and copies the slots that changed at the next initConstraints / updateSolution /
+ * computeKKTResidual, so a reference that does not change between calls is copied once.  Neither call clears the
+ * line-search filter, as on a change of the shared references.  Instance b gives the bits of a shared-mode handle whose
+ * references are instance b's. */
+int idocp_b200_fb_set_instance_cost_reference(idocp_b200_fb_solver* h, int kind, int index, const double* q_ref, const double* v_ref);
+int idocp_b200_fb_clear_instance_cost_references(idocp_b200_fb_solver* h);
 /* the chain of stages at time t in the order of the Riccati recursion; arrays of capacity cap (may be NULL;
  * active is [cap][4], the contact / impulse status of the stage); returns the number of stages.
  * dimi > 0: the switching constraint of the coming impulse is imposed on that stage */
@@ -403,6 +416,9 @@ int idocp_b200_fb_sharded_num_shards(const idocp_b200_fb_sharded* s, int* n, int
 int idocp_b200_fb_sharded_shard(idocp_b200_fb_sharded* s, int index, idocp_b200_fb_solver** out);
 int idocp_b200_fb_sharded_set_solution(idocp_b200_fb_sharded* s, const char* name, const double* value, int per_instance);
 int idocp_b200_fb_sharded_set_cost_reference(idocp_b200_fb_sharded* s, int kind, int index, const double* q_ref, const double* v_ref);
+int idocp_b200_fb_sharded_set_instance_cost_reference(idocp_b200_fb_sharded* s, int kind, int index, const double* q_ref /* [batch][19] */,
+                                                      const double* v_ref /* [batch][18] */);
+int idocp_b200_fb_sharded_clear_instance_cost_references(idocp_b200_fb_sharded* s);
 int idocp_b200_fb_sharded_discretize(idocp_b200_fb_sharded* s, double t, int cap, int* kind, int* index, double* stage_t, double* dt,
                                      int* dimf, int* dimi, int* active);
 int idocp_b200_fb_sharded_init_constraints(idocp_b200_fb_sharded* s, double t);

@@ -19,6 +19,7 @@
 #include <array>
 #include <cmath>
 #include <cstring>
+#include <functional>
 
 #include "idocp_b200.hpp"
 
@@ -392,6 +393,22 @@ class OCPSolver {
     if (un_) { un_->clearLineSearchFilter(); return; }
     detail::check(idocp_b200_fb_sharded_clear_line_search_filter(sh_.get()));
   }
+  // Per-instance configuration references: ref(t, q_ref, v_ref) writes q_ref [batch][19] and v_ref [batch][18], row b the
+  // reference of instance b at time t.  While it is set, every call samples it at the time of every stage instead of the
+  // cost's reference; the line-search filter is kept, as on a change of the shared reference.
+  using InstanceCostReference = std::function<void(double t, double* q_ref, double* v_ref)>;
+  void setInstanceCostReference(InstanceCostReference ref) {
+    if (un_) detail::die("idocp_b200: per-instance references of a fixed-base robot: use UnOCPSolver::setCostReference");
+    if (!ref) detail::die("invalid argument: the per-instance reference must not be empty");
+    instance_ref_ = std::move(ref);
+  }
+  // back to the cost's reference for every instance (it is not sampled while per-instance references are set: the next
+  // initConstraints / updateSolution / computeKKTResidual samples it again)
+  void clearInstanceCostReferences() {
+    if (un_) return;
+    instance_ref_ = nullptr;
+    detail::check(idocp_b200_fb_sharded_clear_instance_cost_references(sh_.get()));
+  }
   // assert(isWellDefined()) of OCPDiscretizer::discretizeOCP as a run-time error (default) or ignored like a Release build
   void setStrictDiscretization(bool strict) { detail::check(idocp_b200_fb_sharded_set_strict_discretization(sh_.get(), strict ? 1 : 0)); }
   double KKTError() { return KKTErrors()[0]; }
@@ -498,6 +515,15 @@ class OCPSolver {
   void sampleReference(const double t) {
     t_last_ = t;
     const int n = discretize();
+    if (instance_ref_) {
+      std::vector<double> q_ref(static_cast<size_t>(batch_) * 19), v_ref(static_cast<size_t>(batch_) * 18);
+      for (int e = 0; e < n; ++e) {
+        instance_ref_(t_[e], q_ref.data(), v_ref.data());
+        const int kind = kind_[e] == 4 ? 0 : kind_[e];
+        detail::check(idocp_b200_fb_sharded_set_instance_cost_reference(sh_.get(), kind, index_[e], q_ref.data(), v_ref.data()));
+      }
+      return;
+    }
     if (!cost_->fbConfig()) return;
     VectorXd q_ref(19);
     for (int e = 0; e < n; ++e) {
@@ -527,6 +553,7 @@ class OCPSolver {
   std::vector<int> kind_, index_, dimf_;
   std::vector<double> t_, q_, v_;
   std::vector<std::array<int, 4>> active_;
+  InstanceCostReference instance_ref_;
 };
 
 // hybrid/collision_checker.hxx:22-53: which contact frames are at or below the ground (z <= 0) at configuration q.  Host
